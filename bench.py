@@ -5,6 +5,7 @@
     python bench.py --workload din | retrieval                    # configs[1] (DIN, MovieLens-shaped) / configs[4] (YouTubeDNN, 10 M items)
     python bench.py --impl reference --steps K --warmup W         # the reference restated on CPU (oracle), same workload
     python -m torch.distributed.run ... bench.py --gpus N --verify   # N>1: correctness of the sharded step against a 1-GPU engine
+    python bench.py --steps K --warmup W --dump-outputs DIR       # also write the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one full training step on one batch of synthetic samples.  Prints ONE JSON line (contract in the task statement):
 `value` = device-resident throughput (CUDA events), `e2e` = through the reference-shaped API -- `handyrec_b200.models.<Model>(...)
@@ -207,6 +208,23 @@ def build_deepfm_model(vocabs):
     return model, KL
 
 
+def deepfm_outputs(eng, ids):
+    """What a caller of `train_step_on_device(ids, ...)` holds after the step: the mean loss and the click probabilities of the
+    batch, the DNN and FM weights after the update, and, per field, the table rows of a fixed sample of the batch's ids after the
+    update (the tables hold 6.5 GB)."""
+    import torch
+
+    import bench_models
+
+    B = ids.shape[0]
+    pos = torch.from_numpy(bench_models.sample_rows(B)).to(ids.device)
+    out = {"loss": eng.loss_sum.double().cpu() / B, "prob": eng.prob[:B].cpu(), "fm_w": eng.fm_w.cpu(), "fm_w0": eng.fm_w0.cpu()}
+    for i in range(len(eng.units)):
+        out[f"dnn_W{i}"], out[f"dnn_b{i}"] = eng.get_dense_weights(i)
+    out["table_rows"] = torch.stack([eng.tables[t][ids[pos, col].long()] for t, _, _, col, _ in eng.plan_fields]).cpu()
+    return {k: v.numpy() for k, v in out.items()}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -228,7 +246,14 @@ def main():
                     help="embedding backward: auto = the engine times both implementations in its first steps and keeps the faster one; "
                          "units / sort pin one (profiling under ncu distorts the trial timings)")
     ap.add_argument("--verify", action="store_true", help="N>1: 3 sharded steps at a small batch compared with a single-GPU engine on the concatenated batch")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="one GPU: after the timed steps, write what the last of them computed as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB; large embedding tables as a fixed sample of rows), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.verify or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the outputs of the CUDA path's timed steps on one GPU (--impl ours, no --verify, one process)")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload != "deepfm":
@@ -335,6 +360,10 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     launches = launch_count() - l0
+    if args.dump_outputs:
+        import bench_models
+
+        bench_models.write_outputs(args.dump_outputs, deepfm_outputs(eng, ids_pool[(args.steps - 1) % NB]))
 
     # ---- end-to-end through the reference-shaped API ----------------------------------------------
     if True:

@@ -1,5 +1,5 @@
 """bench.py workloads besides DeepFM: DIN (BASELINE.json configs[1]), YouTubeMatchDNN retrieval (configs[4]), their CPU arms
-(oracle/), and the multi-GPU --verify mode.  Imported by bench.py only."""
+(oracle/), the multi-GPU --verify mode, and the writer of --dump-outputs.  Imported by bench.py only."""
 from __future__ import annotations
 
 import json
@@ -15,6 +15,41 @@ ML = {"user_id": (6041, 32), "gender": (3, 4), "occupation": (22, 16), "zip": (3
 DIN_B, DIN_T, GENRES_L = 4096, 50, 6
 RET_B, RET_ITEMS, RET_SAMPLED, RET_EMBD = 4096, 10_000_000, 100, 64
 RET_CPU_ITEMS = 1_000_000  # catalogue rows on the CPU arm (the reference recomputes EVERY catalogue row every step)
+DUMP_ROWS = 4096  # --dump-outputs: rows kept of a table too large to write whole
+DUMP_MAX_BYTES = 64 << 20
+
+
+def sample_rows(n, seed=0):
+    """--dump-outputs: a fixed, seeded, sorted choice of min(n, DUMP_ROWS) distinct indices below n."""
+    return np.sort(np.random.RandomState(seed).choice(n, min(n, DUMP_ROWS), replace=False))
+
+
+def write_outputs(directory, arrays):
+    """--dump-outputs: DIR/<name>.npy for every array, float32 kept as it is and anything else as float64."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs, more than {DUMP_MAX_BYTES}")
+    os.makedirs(directory, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, f"{k}.npy"), v)
+
+
+def model_outputs(model, loss):
+    """What a caller of `Model.train_on_batch` holds after the step: the loss it returned and the model's weights, tables of
+    more than 2^20 entries as a fixed sample of their rows."""
+    import torch
+
+    from handyrec_b200.checkpoint import _named_weights
+
+    out = {"loss": np.array([loss], dtype=np.float64)}
+    for name, _, p in _named_weights(model):
+        w = p.detach()
+        if w.numel() > (1 << 20):
+            w = w[torch.from_numpy(sample_rows(w.shape[0])).to(w.device)]
+        out[name] = w.cpu().numpy()
+    return out
 
 
 def _hist(rng, n, T, vocab):
@@ -202,11 +237,13 @@ def run(args, load_peaks, ClockSampler, WORKLOADS, METRICS):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for s in range(args.steps):
-        model.train_on_batch(*pool_dev[s % NB])
+        loss = model.train_on_batch(*pool_dev[s % NB])
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
     launches = launch_count() - l0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, model_outputs(model, loss))
     # end to end: Model.fit on host dict-of-arrays (numpy), one epoch of `steps` batches
     reps = (args.steps + NB - 1) // NB
     xh = {k: np.concatenate([v] * reps)[: args.steps * B] for k, v in x.items()}

@@ -1,23 +1,40 @@
 """CPU: the reference's OWN model files, imported unchanged through handyrec_b200.compat, build the same graphs as this package's
-constructors -- layer for layer -- and DeepFM-shaped graphs are recognised by the lowering.  Needs the reference checkout
-(/root/reference), which exists in the build container only: skipped on the GPU box."""
+constructors -- layer for layer -- and DeepFM-shaped graphs are recognised by the lowering.
+
+The graphs the reference's files build (input names, then layer kind, configuration, input and output shapes per node) are stored in
+tests/golden/compat_graphs.json, so the comparison runs without a checkout of the reference.  With a checkout
+(REFERENCE_ROOT=/path/to/HandyRec) the reference's files are also built through the compat shim and held to the stored graphs, and
+`python -m tests.test_compat_cpu /path/to/HandyRec` rewrites the file from them.  The stored file was recorded from
+`handyrec_b200.models` at a commit whose graphs this test had found equal to those of the reference's files."""
+import importlib
+import json
 import os
 import sys
 
 import numpy as np
 import pytest
 
-REF = os.environ.get("REFERENCE_ROOT", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "handyrec", "models")), reason="no reference checkout")
+REF = os.environ.get("REFERENCE_ROOT")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "compat_graphs.json")
+
+
+def _is_checkout(root):
+    return root is not None and os.path.isdir(os.path.join(root, "handyrec", "models"))
 
 
 @pytest.fixture(scope="module")
 def ref_models():
+    """The reference's `handyrec.models` over the compat shim; None without a checkout, or when a real TensorFlow is importable
+    (the shim is not needed then)."""
+    if not _is_checkout(REF):
+        yield None
+        return
     try:
         import tensorflow  # noqa: F401
 
         if not getattr(tensorflow, "__handyrec_b200_shim__", False):
-            pytest.skip("a real TensorFlow is importable: the shim is not needed")
+            yield None
+            return
     except ImportError:
         pass
     from handyrec_b200 import compat
@@ -54,6 +71,16 @@ def _signature(model):
     return sig
 
 
+def _graph(model, family):
+    """What the comparison covers, in the form the golden file stores it (JSON: tuples read back as lists)."""
+    g = {"inputs": [t.name for t in model.inputs], "nodes": _signature(model)}
+    if family == "retrieval":
+        for attr in ("user_input", "user_embedding", "item_input", "item_embedding"):
+            assert hasattr(model, attr)
+        g["item_embedding_shape"] = tuple(model.item_embedding.shape)
+    return json.loads(json.dumps(g))
+
+
 def _groups(kind):
     from handyrec_b200.features import EmbdFeatureGroup, FeatureGroup, FeaturePool
 
@@ -84,37 +111,41 @@ CASES = [
 ]
 
 
+def _key(name, kw):
+    return name + json.dumps(kw, sort_keys=True)
+
+
+def _reference_graph(family, name, kw, kind):
+    ref_ctor = getattr(importlib.import_module("handyrec.models." + family), name)  # the reference's package __init__ imports nothing
+    assert ref_ctor.__code__.co_filename.startswith(REF)  # really the reference's file
+    return _graph(ref_ctor(*_groups(kind), **kw), family)
+
+
 @pytest.mark.parametrize("kind,family,name,kw,ours_kw", CASES)
 def test_reference_model_files_build_the_same_graph(ref_models, kind, family, name, kw, ours_kw):
     import handyrec_b200.models as ours
 
-    import importlib
-
-    ref_ctor = getattr(importlib.import_module("handyrec.models." + family), name)  # the reference's package __init__ imports nothing
-    assert ref_ctor.__code__.co_filename.startswith(REF)  # really the reference's file
-    m_ref = ref_ctor(*_groups(kind), **kw)
-    m_ours = getattr(ours, name)(*_groups(kind), **kw, **ours_kw)
-    assert [t.name for t in m_ref.inputs] == [t.name for t in m_ours.inputs]
-    assert _signature(m_ref) == _signature(m_ours)
-    if family == "retrieval":
-        for attr in ("user_input", "user_embedding", "item_input", "item_embedding"):
-            assert hasattr(m_ref, attr) and hasattr(m_ours, attr)
-        assert tuple(m_ref.item_embedding.shape) == tuple(m_ours.item_embedding.shape)
+    with open(GOLDEN) as f:
+        want = json.load(f)[_key(name, kw)]
+    if ref_models is not None:
+        assert _reference_graph(family, name, kw, kind) == want
+    assert _graph(getattr(ours, name)(*_groups(kind), **kw, **ours_kw), family) == want
 
 
 def test_reference_deepfm_is_lowered_onto_the_fused_engine(ref_models):
     """`compile()` recognises the graph the reference's DeepFM.py builds (shared FM / DNN features) and binds the fused engine;
-    a DNN with BatchNorm keeps the layer-by-layer path."""
+    a DNN with BatchNorm keeps the layer-by-layer path.  Without a checkout the graph comes from this package's DeepFM, which the
+    test above holds to the reference's."""
     from handyrec_b200.features import FeatureGroup, FeaturePool
     from handyrec_b200.lowering import match_deepfm
+    from handyrec_b200.models import DeepFM
 
     user, item = _features()
     feats = [f for f in user if type(f).__name__ != "DenseFeature"] + item[:1]
     pool = FeaturePool()
     fm, dnn = FeatureGroup("fm", feats, pool), FeatureGroup("dnn", user + item[:1], pool)
-    import importlib
-
-    DeepFM = importlib.import_module("handyrec.models.ranking").DeepFM
+    if ref_models is not None:
+        DeepFM = importlib.import_module("handyrec.models.ranking").DeepFM
     m = DeepFM(fm, dnn, dnn_hidden_units=(16, 1))
     spec = match_deepfm(m)
     assert spec is not None and len(spec.fields) == len(feats) and [t.name for t in spec.dense_inputs] == ["age"]
@@ -125,3 +156,16 @@ def test_reference_deepfm_is_lowered_onto_the_fused_engine(ref_models):
     pool3 = FeaturePool()  # different feature lists in the two groups: two lookups are needed, no fusion
     m_diff = DeepFM(FeatureGroup("fm", feats[:2], pool3), FeatureGroup("dnn", user + item[:1], pool3), dnn_hidden_units=(16, 1))
     assert match_deepfm(m_diff) is None
+
+
+if __name__ == "__main__":
+    REF = sys.argv[1] if len(sys.argv) > 1 else REF
+    if not _is_checkout(REF):
+        raise SystemExit("usage: python -m tests.test_compat_cpu /path/to/HandyRec  (a checkout of the reference)")
+    from handyrec_b200 import compat
+
+    compat.install(REF)
+    graphs = {_key(name, kw): _reference_graph(family, name, kw, kind) for kind, family, name, kw, _ in CASES}
+    with open(GOLDEN, "w") as f:  # one graph per line
+        f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(g)}" for k, g in graphs.items()) + "\n}\n")
+    print(f"wrote {GOLDEN}: {len(graphs)} graphs from {REF}")
