@@ -20,7 +20,7 @@ HRB_OK, HRB_BAD_ARG, HRB_UNSUPPORTED, HRB_CUDA_ERROR, HRB_WORKSPACE = 0, 1, 2, 3
 # enums
 POOL = {"none": 0, None: 0, "mean": 1, "sum": 2, "max": 3}
 ACT = {None: 0, "linear": 0, "relu": 1, "sigmoid": 2, "tanh": 3, "dice": 4}
-OPT_SGD, OPT_ADAM_LAZY = 0, 1
+OPT_SGD, OPT_ADAM_LAZY, OPT_ADAGRAD = 0, 1, 2
 GEMM_AUTO, GEMM_FP32, GEMM_3XTF32 = 0, 1, 2
 BWD_AUTO, BWD_UNITS, BWD_SORT = 0, 1, 2
 

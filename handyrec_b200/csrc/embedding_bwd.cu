@@ -991,10 +991,12 @@ int run_unit_update(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, in
     a.debug = dbg;
   }
 #endif
-  const bool adam = opt.opt == HRB_OPT_ADAM_LAZY;
+  const int mode = upd_mode(opt.opt);
   for (int gi = 0; gi < us.n_g; ++gi) {
-#define HRB_UNITS(GG)                                                   \
-  rc = adam ? launch_units<1, GG>(a, us, gi, st) : launch_units<0, GG>(a, us, gi, st); \
+#define HRB_UNITS(GG)                                                                      \
+  rc = mode == UPD_ADAM      ? launch_units<UPD_ADAM, GG>(a, us, gi, st)                   \
+       : mode == UPD_ADAGRAD ? launch_units<UPD_ADAGRAD, GG>(a, us, gi, st)                \
+                             : launch_units<UPD_SGD, GG>(a, us, gi, st);                   \
   break;
     switch (us.g_values[gi]) {
       case 1: HRB_UNITS(1)

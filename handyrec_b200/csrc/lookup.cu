@@ -556,9 +556,9 @@ __device__ __forceinline__ int find_table(const TableDev* __restrict__ t, int n,
   return lo;
 }
 
-template <int MODE>  // 0 sgd, 1 adam lazy, 2 dense gradient add
+template <int MODE>  // UpdMode: sgd, adam lazy, adagrad, or dense gradient add
 __device__ __forceinline__ void apply_row(const ApplyCtx& c, uint32_t key, int q, float4 g) {
-  if (MODE == 2) {
+  if (MODE == UPD_DENSE_ADD) {
     float4* p = reinterpret_cast<float4*>(c.dense_out + (int64_t)key * c.tables[0].dim) + q;
     float4 o = *p;
     o.x += g.x; o.y += g.y; o.z += g.z; o.w += g.w;
@@ -967,12 +967,14 @@ static int run_sorted_update(int mode, const BwdWorkspace& w, int64_t n, uint32_
   }                                                                                                            \
   bwd_merge_kernel<M><<<grid2, launch_threads, 0, st>>>(n_chunks, G, ctx, w.partial, w.pkey, w.pflag);         \
   HRB_LAUNCH_CHECK();
-  if (mode == 0) {
-    HRB_RUN_MODE(0)
-  } else if (mode == 1) {
-    HRB_RUN_MODE(1)
+  if (mode == UPD_SGD) {
+    HRB_RUN_MODE(UPD_SGD)
+  } else if (mode == UPD_ADAM) {
+    HRB_RUN_MODE(UPD_ADAM)
+  } else if (mode == UPD_ADAGRAD) {
+    HRB_RUN_MODE(UPD_ADAGRAD)
   } else {
-    HRB_RUN_MODE(2)
+    HRB_RUN_MODE(UPD_DENSE_ADD)
   }
 #undef HRB_RUN_MODE
   return HRB_OK;
@@ -1304,10 +1306,14 @@ HRB_API int hrb_lookup_bwd_update(const hrb_plan* plan, const int32_t* ids, int6
   HRB_REQUIRE(aligned16(dout) && dout_ld % 4 == 0, "hrb_lookup_bwd_update: dout must be 16-byte aligned, dout_ld %% 4 == 0");
   if (plan->has_max)
     return fail(HRB_UNSUPPORTED, "hrb_lookup_bwd_update: max-pooled fields go through hrb_seq_pool_bwd + hrb_embedding_bwd_dense");
-  HRB_REQUIRE(opt_host->opt == HRB_OPT_SGD || opt_host->opt == HRB_OPT_ADAM_LAZY, "hrb_lookup_bwd_update: unknown optimiser %d", opt_host->opt);
+  HRB_REQUIRE(opt_host->opt == HRB_OPT_SGD || opt_host->opt == HRB_OPT_ADAM_LAZY || opt_host->opt == HRB_OPT_ADAGRAD,
+              "hrb_lookup_bwd_update: unknown optimiser %d", opt_host->opt);
   if (opt_host->opt == HRB_OPT_ADAM_LAZY)
     for (const auto& t : plan->tdev_host)
       HRB_REQUIRE(t.grad || (t.m && t.v), "hrb_lookup_bwd_update: lazy Adam needs adam_m/adam_v for every table");
+  if (opt_host->opt == HRB_OPT_ADAGRAD)
+    for (const auto& t : plan->tdev_host)
+      HRB_REQUIRE(t.grad || t.m, "hrb_lookup_bwd_update: Adagrad needs an accumulator (adam_m) for every row-updated table");
   const int G = plan->max_dim / 4;
   if (G > 256) return fail(HRB_UNSUPPORTED, "hrb_lookup_bwd_update: dim %d too large", plan->max_dim);
   if (batch == 0) return HRB_OK;
@@ -1330,7 +1336,7 @@ HRB_API int hrb_lookup_bwd_update(const hrb_plan* plan, const int32_t* ids, int6
   ApplyCtx ctx{plan->d_tables, plan->n_tables, *opt_host, nullptr, 0.f};
   if (opt_host->opt == HRB_OPT_ADAM_LAZY)
     ctx.lr_t = opt_host->lr * sqrtf(opt_host->bias_corr2) / opt_host->bias_corr1;
-  return run_sorted_update(opt_host->opt == HRB_OPT_SGD ? 0 : 1, w, n, sentinel, plan->key_bits, G, src, ctx, hot_from_plan(plan), st);
+  return run_sorted_update(upd_mode(opt_host->opt), w, n, sentinel, plan->key_bits, G, src, ctx, hot_from_plan(plan), st);
 }
 
 HRB_API int hrb_embedding_bwd_dense_workspace(int64_t n_ids, int32_t dim, size_t* bytes) {
@@ -1378,7 +1384,7 @@ HRB_API int hrb_embedding_bwd_dense(const int32_t* ids, int64_t n_ids, const flo
     hot.keys = nullptr;
     hot.n_keys = (int32_t)vocab;
   }
-  return run_sorted_update(2, w, n_ids, sentinel, key_bits, dim / 4, src, ctx, hot, st);
+  return run_sorted_update(UPD_DENSE_ADD, w, n_ids, sentinel, key_bits, dim / 4, src, ctx, hot, st);
 }
 
 // =============================================================================================
@@ -1736,9 +1742,12 @@ HRB_API int hrb_keyed_bwd_update(const hrb_plan* plan, const uint32_t* keys, con
   if (n == 0) return HRB_OK;
   HRB_REQUIRE(keys && grads && aligned16(grads), "hrb_keyed_bwd_update: null/misaligned pointer");
   if (!plan->uniform_dim) return fail(HRB_UNSUPPORTED, "hrb_keyed_bwd_update: needs one embedding dim");
-  HRB_REQUIRE(opt_host->opt == HRB_OPT_SGD || opt_host->opt == HRB_OPT_ADAM_LAZY, "hrb_keyed_bwd_update: unknown optimiser %d", opt_host->opt);
+  HRB_REQUIRE(opt_host->opt == HRB_OPT_SGD || opt_host->opt == HRB_OPT_ADAM_LAZY || opt_host->opt == HRB_OPT_ADAGRAD,
+              "hrb_keyed_bwd_update: unknown optimiser %d", opt_host->opt);
   if (opt_host->opt == HRB_OPT_ADAM_LAZY)
     for (const auto& t : plan->tdev_host) HRB_REQUIRE(t.m && t.v, "hrb_keyed_bwd_update: lazy Adam needs adam_m/adam_v for every table");
+  if (opt_host->opt == HRB_OPT_ADAGRAD)
+    for (const auto& t : plan->tdev_host) HRB_REQUIRE(t.m, "hrb_keyed_bwd_update: Adagrad needs an accumulator (adam_m) for every table");
   BwdWorkspace w;
   int rc = carve_bwd_ws(n, 1, plan->max_dim, plan->key_bits, workspace, w);
   if (rc != HRB_OK) return rc;
@@ -1752,7 +1761,7 @@ HRB_API int hrb_keyed_bwd_update(const hrb_plan* plan, const uint32_t* keys, con
   FlatGrad src{grads, plan->max_dim};
   ApplyCtx ctx{plan->d_tables, plan->n_tables, *opt_host, nullptr, 0.f};
   if (opt_host->opt == HRB_OPT_ADAM_LAZY) ctx.lr_t = opt_host->lr * sqrtf(opt_host->bias_corr2) / opt_host->bias_corr1;
-  return run_sorted_update(opt_host->opt == HRB_OPT_SGD ? 0 : 1, w, n, (uint32_t)plan->total_rows, plan->key_bits, plan->max_dim / 4, src, ctx,
+  return run_sorted_update(upd_mode(opt_host->opt), w, n, (uint32_t)plan->total_rows, plan->key_bits, plan->max_dim / 4, src, ctx,
                            hot_from_plan(plan), st);
 }
 

@@ -78,8 +78,25 @@ __global__ void __launch_bounds__(256) sgd_kernel(float* __restrict__ p, const f
   }
 }
 
+// Keras Adagrad (ResourceApplyAdagradV2): eps outside the square root, no step counter
+__device__ __forceinline__ float adagrad_update(float w, float& acc, float g, float lr, float eps) {
+  acc = fmaf(g, g, acc);
+  return w - lr * g / (sqrtf(acc) + eps);
+}
+
+__global__ void __launch_bounds__(256) adagrad_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ acc, int64_t n,
+                                                     float lr, float eps, float l2_scale) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const float w = p[i];
+    float a = acc[i];
+    p[i] = adagrad_update(w, a, fmaf(l2_scale, w, g[i]), lr, eps);
+    acc[i] = a;
+  }
+}
+
 // Many small parameter tensors in ONE launch (the layer-by-layer models step 12-27 tensors: one launch each was 0.4 ms of
-// host time per step).  Block b works on the tensor whose block range contains it; same arithmetic as adam_kernel / sgd_kernel.
+// host time per step).  Block b works on the tensor whose block range contains it; same arithmetic as adam_kernel / sgd_kernel /
+// adagrad_kernel.  m holds the Adagrad accumulator.
 struct MultiArgs {
   float* p[HRB_MULTI_MAX];
   const float* g[HRB_MULTI_MAX];
@@ -90,7 +107,8 @@ struct MultiArgs {
   int32_t first_block[HRB_MULTI_MAX + 1];
   int32_t count;
 };
-template <bool ADAM>
+enum MultiOpt { MULTI_SGD, MULTI_ADAM, MULTI_ADAGRAD };
+template <int OPT>
 __global__ void __launch_bounds__(256) multi_step_kernel(const MultiArgs a, float lr_t, float b1, float b2, float eps) {
   int t = 0;
   while (t + 1 < a.count && (int)blockIdx.x >= a.first_block[t + 1]) ++t;
@@ -102,12 +120,16 @@ __global__ void __launch_bounds__(256) multi_step_kernel(const MultiArgs a, floa
   for (int64_t i = b * blockDim.x + threadIdx.x; i < a.n[t]; i += nb * blockDim.x) {
     const float w = p[i];
     const float gi = fmaf(l2, w, g[i]);
-    if (ADAM) {
+    if (OPT == MULTI_ADAM) {
       const float mi = b1 * a.m[t][i] + (1.f - b1) * gi;
       const float vi = b2 * a.v[t][i] + (1.f - b2) * gi * gi;
       a.m[t][i] = mi;
       a.v[t][i] = vi;
       p[i] = w - lr_t * mi / (sqrtf(vi) + eps);
+    } else if (OPT == MULTI_ADAGRAD) {
+      float acc = a.m[t][i];
+      p[i] = adagrad_update(w, acc, gi, lr_t, eps);
+      a.m[t][i] = acc;
     } else {
       p[i] = w - lr_t * gi;
     }
@@ -279,6 +301,14 @@ HRB_API int hrb_adam_step(float* param, const float* grad, float* m, float* v, i
   return HRB_OK;
 }
 
+HRB_API int hrb_adagrad_step(float* param, const float* grad, float* acc, int64_t n, float lr, float eps, float l2_scale, void* stream) {
+  HRB_REQUIRE(param && grad && acc && n >= 0, "hrb_adagrad_step: bad argument");
+  if (n == 0) return HRB_OK;
+  adagrad_kernel<<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(param, grad, acc, n, lr, eps, l2_scale);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
 HRB_API int hrb_sgd_step(float* param, const float* grad, int64_t n, float lr, float l2_scale, void* stream) {
   HRB_REQUIRE(param && grad && n >= 0, "hrb_sgd_step: bad argument");
   if (n == 0) return HRB_OK;
@@ -287,19 +317,20 @@ HRB_API int hrb_sgd_step(float* param, const float* grad, int64_t n, float lr, f
   return HRB_OK;
 }
 
-static int multi_step(bool adam, int32_t count, float* const* param, const float* const* grad, float* const* m, float* const* v,
+static int multi_step(int opt, int32_t count, float* const* param, const float* const* grad, float* const* m, float* const* v,
                       const int64_t* n, const float* l2_scale, float lr_t, float b1, float b2, float eps, cudaStream_t st) {
   for (int32_t c0 = 0; c0 < count; c0 += HRB_MULTI_MAX) {
     MultiArgs a{};
     int blocks = 0;
     for (int32_t i = c0; i < count && i < c0 + HRB_MULTI_MAX; ++i) {
-      HRB_REQUIRE(n[i] >= 0 && (n[i] == 0 || (param[i] && grad[i] && (!adam || (m[i] && v[i])))), "multi-tensor step: null tensor %d", i);
+      HRB_REQUIRE(n[i] >= 0 && (n[i] == 0 || (param[i] && grad[i] && (opt == MULTI_SGD || m[i]) && (opt != MULTI_ADAM || v[i]))),
+                  "multi-tensor step: null tensor %d", i);
       if (n[i] == 0) continue;
       const int k = a.count++;
       a.p[k] = param[i];
       a.g[k] = grad[i];
-      a.m[k] = adam ? m[i] : nullptr;
-      a.v[k] = adam ? v[i] : nullptr;
+      a.m[k] = opt != MULTI_SGD ? m[i] : nullptr;
+      a.v[k] = opt == MULTI_ADAM ? v[i] : nullptr;
       a.n[k] = n[i];
       a.l2[k] = l2_scale ? l2_scale[i] : 0.f;
       a.first_block[k] = blocks;
@@ -307,8 +338,9 @@ static int multi_step(bool adam, int32_t count, float* const* param, const float
     }
     if (a.count == 0) continue;
     a.first_block[a.count] = blocks;
-    if (adam) multi_step_kernel<true><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
-    else multi_step_kernel<false><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
+    if (opt == MULTI_ADAM) multi_step_kernel<MULTI_ADAM><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
+    else if (opt == MULTI_ADAGRAD) multi_step_kernel<MULTI_ADAGRAD><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
+    else multi_step_kernel<MULTI_SGD><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
     HRB_LAUNCH_CHECK();
   }
   return HRB_OK;
@@ -319,14 +351,21 @@ HRB_API int hrb_adam_step_multi(int32_t count, float* const* param_host, const f
                                 float beta2, float eps, float bias_corr1, float bias_corr2, void* stream) {
   HRB_REQUIRE(count >= 0 && (count == 0 || (param_host && grad_host && m_host && v_host && n_host)) && bias_corr1 > 0.f,
               "hrb_adam_step_multi: bad argument");
-  return multi_step(true, count, param_host, grad_host, m_host, v_host, n_host, l2_scale_host, lr * sqrtf(bias_corr2) / bias_corr1, beta1, beta2,
+  return multi_step(MULTI_ADAM, count, param_host, grad_host, m_host, v_host, n_host, l2_scale_host, lr * sqrtf(bias_corr2) / bias_corr1, beta1, beta2,
                     eps, (cudaStream_t)stream);
 }
 
 HRB_API int hrb_sgd_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, const int64_t* n_host,
                                const float* l2_scale_host, float lr, void* stream) {
   HRB_REQUIRE(count >= 0 && (count == 0 || (param_host && grad_host && n_host)), "hrb_sgd_step_multi: bad argument");
-  return multi_step(false, count, param_host, grad_host, nullptr, nullptr, n_host, l2_scale_host, lr, 0.f, 0.f, 0.f, (cudaStream_t)stream);
+  return multi_step(MULTI_SGD, count, param_host, grad_host, nullptr, nullptr, n_host, l2_scale_host, lr, 0.f, 0.f, 0.f, (cudaStream_t)stream);
+}
+
+HRB_API int hrb_adagrad_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, float* const* acc_host,
+                                   const int64_t* n_host, const float* l2_scale_host, float lr, float eps, void* stream) {
+  HRB_REQUIRE(count >= 0 && (count == 0 || (param_host && grad_host && acc_host && n_host)), "hrb_adagrad_step_multi: bad argument");
+  return multi_step(MULTI_ADAGRAD, count, param_host, grad_host, acc_host, nullptr, n_host, l2_scale_host, lr, 0.f, 0.f, eps,
+                    (cudaStream_t)stream);
 }
 
 HRB_API int hrb_dice_fwd(const float* x, int64_t rows, int32_t units, const float* alpha, float* mean, float* var,

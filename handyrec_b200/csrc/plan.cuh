@@ -23,16 +23,32 @@ struct FieldDev {
 
 struct TableDev {
   float* w;
-  float* m;
-  float* v;
+  float* m;     // optimiser state: Adam first moment / Adagrad accumulator
+  float* v;     // Adam second moment
   int64_t rows;
   uint32_t key_base;
   int32_t dim;
   float* grad;  // non-null: a13 adds the row's gradient sum here instead of updating the row (hrb_plan_set_dense_grads)
 };
 
-// One touched row of one table takes its update (a13).  MODE 0: SGD, 1: lazy Adam.  A table with a dense-gradient buffer
-// (hrb_plan_set_dense_grads) receives the gradient sum instead and is stepped by the caller's dense optimiser.
+// Row-update modes of apply_table_row(s) and of every kernel that dispatches on them.  UPD_DENSE_ADD is lookup.cu's
+// dense-gradient face (hrb_embedding_bwd_dense), which never reaches apply_table_row(s).
+enum UpdMode : int { UPD_SGD = 0, UPD_ADAM = 1, UPD_DENSE_ADD = 2, UPD_ADAGRAD = 3 };
+
+// hrb_opt -> UpdMode of the row update
+inline int upd_mode(int32_t opt) {
+  return opt == HRB_OPT_ADAM_LAZY ? UPD_ADAM : opt == HRB_OPT_ADAGRAD ? UPD_ADAGRAD : UPD_SGD;
+}
+
+// Keras Adagrad (ResourceSparseApplyAdagradV2, eps outside the square root) on one float of a row; acc is the table's
+// accumulator (TableDev::m)
+__device__ __forceinline__ void adagrad_elem(float& w, float& acc, float g, float lr, float eps) {
+  acc = fmaf(g, g, acc);
+  w -= lr * g / (sqrtf(acc) + eps);
+}
+
+// One touched row of one table takes its update (a13).  MODE: UpdMode (SGD, lazy Adam, Adagrad).  A table with a dense-gradient
+// buffer (hrb_plan_set_dense_grads) receives the gradient sum instead and is stepped by the caller's dense optimiser.
 template <int MODE>
 __device__ __forceinline__ void apply_table_row(const TableDev& t, const hrb_opt_params& opt, float lr_t, int64_t row, int q, float4 g) {
   if (q * 4 >= t.dim) return;
@@ -48,9 +64,16 @@ __device__ __forceinline__ void apply_table_row(const TableDev& t, const hrb_opt
   float4 w = *wp;
   const float l2 = opt.l2_scale;
   g.x = fmaf(l2, w.x, g.x); g.y = fmaf(l2, w.y, g.y); g.z = fmaf(l2, w.z, g.z); g.w = fmaf(l2, w.w, g.w);
-  if (MODE == 0) {
+  if (MODE == UPD_SGD) {
     const float lr = opt.lr;
     w.x -= lr * g.x; w.y -= lr * g.y; w.z -= lr * g.z; w.w -= lr * g.w;
+  } else if (MODE == UPD_ADAGRAD) {
+    float4* ap = reinterpret_cast<float4*>(t.m) + off;
+    float4 a = *ap;
+    const float lr = opt.lr, e = opt.eps;
+    adagrad_elem(w.x, a.x, g.x, lr, e); adagrad_elem(w.y, a.y, g.y, lr, e);
+    adagrad_elem(w.z, a.z, g.z, lr, e); adagrad_elem(w.w, a.w, g.w, lr, e);
+    *ap = a;
   } else {
     float4* mp = reinterpret_cast<float4*>(t.m) + off;
     float4* vp = reinterpret_cast<float4*>(t.v) + off;
@@ -99,10 +122,8 @@ __device__ __forceinline__ void apply_table_rows(const TableDev& t, const hrb_op
   for (int i = 0; i < N; ++i) {
     if (ok[i]) {
       w[i] = reinterpret_cast<float4*>(t.w)[off[i]];
-      if (MODE == 1) {
-        m[i] = reinterpret_cast<float4*>(t.m)[off[i]];
-        v[i] = reinterpret_cast<float4*>(t.v)[off[i]];
-      }
+      if (MODE != UPD_SGD) m[i] = reinterpret_cast<float4*>(t.m)[off[i]];
+      if (MODE == UPD_ADAM) v[i] = reinterpret_cast<float4*>(t.v)[off[i]];
     }
   }
   const float l2 = opt.l2_scale;
@@ -111,9 +132,15 @@ __device__ __forceinline__ void apply_table_rows(const TableDev& t, const hrb_op
     if (!ok[i]) continue;
     float4 gi = g[i], wi = w[i];
     gi.x = fmaf(l2, wi.x, gi.x); gi.y = fmaf(l2, wi.y, gi.y); gi.z = fmaf(l2, wi.z, gi.z); gi.w = fmaf(l2, wi.w, gi.w);
-    if (MODE == 0) {
+    if (MODE == UPD_SGD) {
       const float lr = opt.lr;
       wi.x -= lr * gi.x; wi.y -= lr * gi.y; wi.z -= lr * gi.z; wi.w -= lr * gi.w;
+    } else if (MODE == UPD_ADAGRAD) {
+      float4 ai = m[i];
+      const float lr = opt.lr, e = opt.eps;
+      adagrad_elem(wi.x, ai.x, gi.x, lr, e); adagrad_elem(wi.y, ai.y, gi.y, lr, e);
+      adagrad_elem(wi.z, ai.z, gi.z, lr, e); adagrad_elem(wi.w, ai.w, gi.w, lr, e);
+      reinterpret_cast<float4*>(t.m)[off[i]] = ai;
     } else {
       float4 mi = m[i], vi = v[i];
       const float b1 = opt.beta1, b2 = opt.beta2, e = opt.eps, lr = lr_t;

@@ -12,7 +12,7 @@ Data layout of one batch in HBM (all fp32, row-major):
   A_i  (B, ld_i)  activations of Dense layer i (ld_i = round-up-4(units_i))
   params          ONE flat buffer: W_0 | b_0 | ... | W_n | b_n | fm_w (D) | fm_w0 (1), every block padded
                   to 4 floats; W_i is (K_i_padded, ld_i) with zero rows/columns at the padding
-  grads / adam m,v  same layout as params
+  grads / adam m,v  same layout as params (Adagrad: its accumulator in the place of m, no v)
 Reference order of the DNN input is kept (dense first, layers/utils.py:70-84); the padding rows of
 W_0 multiply zero columns of X0 and receive zero gradients, so they stay zero.
 """
@@ -51,6 +51,9 @@ class DeepFMEngine:
     buffer (`engine.tables[t]` is the live table), their row gradients are reduced into the flat gradient buffer and
     they take the same optimiser step as the dense parameters -- exactly Keras' treatment of an IndexedSlices
     gradient (dense moment decay and dense l2_embd).  Every other table gets the touched-rows-only update.
+
+    optimizer: "adam", "sgd" or "adagrad" (Keras Adagrad; accumulators start at `initial_accumulator_value`).  Under
+    Adagrad the touched-rows-only update is exactly Keras' step whenever l2_embd = 0 (DESIGN.md 3).
     """
 
     def __init__(
@@ -71,6 +74,7 @@ class DeepFMEngine:
         task: str = "binary",
         dense_table_max_rows: int = 0,
         dense_update_tables: Optional[Sequence[int]] = None,
+        initial_accumulator_value: float = 0.1,
     ):
         if dnn_hidden_units[-1] != 1:  # DeepFM.py:59-60
             raise ValueError("Output size of dnn should be 1")
@@ -78,6 +82,8 @@ class DeepFMEngine:
             raise ValueError(f"fused engine supports relu/sigmoid/tanh/linear DNN activations, got {dnn_activation!r}")
         if task != "binary":
             raise ValueError("fused engine implements task='binary'")
+        if initial_accumulator_value < 0:
+            raise ValueError(f"initial_accumulator_value must be non-negative, got {initial_accumulator_value}")
         self.dev = tables[0].device
         self.tables = list(tables)
         self.D = int(tables[0].shape[1])
@@ -89,9 +95,10 @@ class DeepFMEngine:
         self.B = int(batch_size)
         self.act = dnn_activation or "linear"
         self.optimizer = optimizer
-        self.emb_opt = embedding_optimizer or ("adam_lazy" if optimizer == "adam" else "sgd")
+        self.emb_opt = embedding_optimizer or {"adam": "adam_lazy", "adagrad": "adagrad"}.get(optimizer, "sgd")
         self.lr, self.l2_embd, self.l2_dnn = float(lr), float(l2_embd), float(l2_dnn)
-        self.beta1, self.beta2, self.eps = 0.9, 0.999, 1e-7  # Keras Adam defaults
+        self.beta1, self.beta2, self.eps = 0.9, 0.999, 1e-7  # Keras Adam defaults (eps: also Keras Adagrad's)
+        self.initial_accumulator_value = float(initial_accumulator_value)
         self.gemm_mode = gemm_mode
         self.step_count = 0
 
@@ -137,6 +144,8 @@ class DeepFMEngine:
         self.grads = torch.zeros(off, device=self.dev, dtype=torch.float32)
         self.opt_m = torch.zeros(off, device=self.dev, dtype=torch.float32) if optimizer == "adam" else None
         self.opt_v = torch.zeros(off, device=self.dev, dtype=torch.float32) if optimizer == "adam" else None
+        if optimizer == "adagrad":  # opt_m is the accumulator
+            self.opt_m = torch.full((off,), self.initial_accumulator_value, device=self.dev, dtype=torch.float32)
         self.W, self.b, self.dW, self.db = [], [], [], []
         for (wo, bo), Kp, ld in zip(offs, self.layer_K, self.layer_ld):
             self.W.append(self.params[wo : wo + Kp * ld].view(Kp, ld))
@@ -155,11 +164,13 @@ class DeepFMEngine:
             self.tables[t] = live
             table_grads[t] = self.grads[o : o + n].view_as(live)
         self.table_grads = table_grads
-        self.adam_m = self.adam_v = None
+        self.adam_m = self.adam_v = self.accum = None
         if self.emb_opt == "adam_lazy":
             self.adam_m = [None if t in self._table_off else torch.zeros_like(w) for t, w in enumerate(self.tables)]
             self.adam_v = [None if t in self._table_off else torch.zeros_like(w) for t, w in enumerate(self.tables)]
-        self.plan = K.LookupPlan(self.tables, plan_fields, self.adam_m, self.adam_v)
+        elif self.emb_opt == "adagrad":
+            self.accum = [None if t in self._table_off else torch.full_like(w, self.initial_accumulator_value) for t, w in enumerate(self.tables)]
+        self.plan = K.LookupPlan(self.tables, plan_fields, self.adam_m, self.adam_v, accum=self.accum)
         if self.dense_tables:
             self.plan.set_dense_grads(table_grads)
 
@@ -390,7 +401,7 @@ class DeepFMEngine:
         dz, lddz = self.dZ[-1], self.layer_ld[-1]
         tc_step = self.use_tc and B == self.B
         op = _lib.OptParams()
-        op.opt = _lib.OPT_SGD if self.emb_opt == "sgd" else _lib.OPT_ADAM_LAZY
+        op.opt = {"sgd": _lib.OPT_SGD, "adagrad": _lib.OPT_ADAGRAD}.get(self.emb_opt, _lib.OPT_ADAM_LAZY)
         op.lr, op.beta1, op.beta2, op.eps, op.l2_scale = self.lr, self.beta1, self.beta2, self.eps, 2.0 * self.l2_embd
         op.bias_corr1, op.bias_corr2 = 1.0 - self.beta1 ** self.step_count, 1.0 - self.beta2 ** self.step_count
         emb_done = [False]
@@ -499,6 +510,8 @@ class DeepFMEngine:
             if self.optimizer == "adam":
                 call("hrb_adam_step", pp(self.params), pp(self.grads), pp(self.opt_m), pp(self.opt_v), length, self.lr, self.beta1,
                      self.beta2, self.eps, op.bias_corr1, op.bias_corr2, l2s, st)
+            elif self.optimizer == "adagrad":
+                call("hrb_adagrad_step", pp(self.params), pp(self.grads), pp(self.opt_m), length, self.lr, self.eps, l2s, st)
             else:
                 call("hrb_sgd_step", pp(self.params), pp(self.grads), length, self.lr, l2s, st)
         self._refresh_wt()

@@ -353,6 +353,28 @@ class Adam:
         K.adam_step_multi(ps, gs, ms, vs, l2s, self.lr, self.b1, self.b2, self.eps, self.t)  # all variables in one launch
 
 
+class Adagrad:
+    """tf.keras.optimizers.Adagrad (Keras 2.6): acc += g^2; w -= lr * g / (sqrt(acc) + eps), acc starting at
+    initial_accumulator_value.  Large tables take the same step on the rows a batch touches (CustomEmbedding.apply_sparse)."""
+
+    def __init__(self, learning_rate=0.001, initial_accumulator_value=0.1, epsilon=1e-7, lr=None):
+        if initial_accumulator_value < 0.0:
+            raise ValueError(f"initial_accumulator_value must be non-negative: {initial_accumulator_value}")
+        self.lr = float(lr if lr is not None else learning_rate)
+        self.initial_accumulator_value, self.eps = float(initial_accumulator_value), float(epsilon)
+        self.state: Dict[int, torch.Tensor] = {}
+
+    def step(self, params_l2: Sequence[Tuple[torch.nn.Parameter, float]]):
+        from . import kernels as K
+
+        live = [(p, l2) for p, l2 in params_l2 if p.grad is not None and p.requires_grad]
+        for p, _ in live:
+            if id(p) not in self.state:
+                self.state[id(p)] = torch.full_like(p.data, self.initial_accumulator_value)
+        K.adagrad_step_multi([p.data for p, _ in live], [p.grad.contiguous() for p, _ in live], [self.state[id(p)] for p, _ in live],
+                             [2.0 * l2 for _, l2 in live], self.lr, self.eps)  # all variables in one launch
+
+
 class SGD:
     def __init__(self, learning_rate=0.01, lr=None):
         self.lr = float(lr if lr is not None else learning_rate)
@@ -518,7 +540,7 @@ class Model:
             from .sharded import TorchDistComm
 
             self._comm = distribute if not isinstance(distribute, bool) else TorchDistComm()
-        if self.fuse and self.loss is binary_crossentropy and isinstance(self.optimizer, (Adam, SGD)):
+        if self.fuse and self.loss is binary_crossentropy and isinstance(self.optimizer, (Adam, SGD, Adagrad)):
             from .lowering import lower  # a DeepFM-shaped graph runs on the fused engine (one lookup, tcgen05 towers)
 
             self._fused = lower(self)

@@ -18,6 +18,7 @@ __all__ = [
     "init_uniform", "embedding_fwd", "embedding_bwd_dense", "seq_pool_fwd", "seq_pool_bwd", "LookupPlan",
     "fm_fwd", "fm_bwd", "dense_fwd", "dense_bwd_x", "dense_bwd_w", "act_bwd", "dice_fwd", "dice_bwd",
     "lau_fwd", "lau_pack_params", "sigmoid_bce", "adam_step", "sgd_step", "adam_step_multi", "sgd_step_multi",
+    "adagrad_step", "adagrad_step_multi",
 ]
 
 
@@ -155,11 +156,19 @@ def seq_pool_bwd(x: torch.Tensor, mask: torch.Tensor, dout: torch.Tensor, method
 # a7 / a13 fused plan
 # --------------------------------------------------------------------------------------------
 class LookupPlan:
-    """Device plan of one feature group: tables + (table, seq_len, pool, ids_col, out_col) per field."""
+    """Device plan of one feature group: tables + (table, seq_len, pool, ids_col, out_col) per field.
+
+    Optimiser state per table (None entries for tables without): `adam_m` / `adam_v` for lazy Adam, or `accum` for Adagrad
+    (it takes the ABI's adam_m slot, so the two cannot be given together)."""
 
     def __init__(self, tables: Sequence[torch.Tensor], fields: Sequence[Tuple[int, int, str, int, int]],
-                 adam_m: Optional[Sequence[torch.Tensor]] = None, adam_v: Optional[Sequence[torch.Tensor]] = None):
+                 adam_m: Optional[Sequence[torch.Tensor]] = None, adam_v: Optional[Sequence[torch.Tensor]] = None,
+                 accum: Optional[Sequence[torch.Tensor]] = None):
         self.tables = [_chk(t, torch.float32, "table") for t in tables]
+        if accum is not None:
+            if adam_m is not None:
+                raise ValueError("LookupPlan: pass either adam_m (Adam) or accum (Adagrad), not both")
+            adam_m = accum
         self.adam_m = list(adam_m) if adam_m is not None else None
         self.adam_v = list(adam_v) if adam_v is not None else None
         self.fields = [tuple(f) for f in fields]
@@ -237,7 +246,9 @@ class LookupPlan:
     def backward_update(self, ids: torch.Tensor, dout: torch.Tensor, opt: str = "sgd", lr: float = 0.01, l2_scale: float = 0.0,
                         beta1: float = 0.9, beta2: float = 0.999, eps: float = 1e-7, step: int = 1,
                         workspace: Optional[torch.Tensor] = None, autotune: bool = False) -> None:
-        """Segment-reduce the gradient rows per table row and update the touched rows of every table in place."""
+        """Segment-reduce the gradient rows per table row and update the touched rows of every table in place.
+
+        opt: "sgd", "adam" (lazy Adam: beta1, beta2, eps, step) or "adagrad" (eps; the plan's `accum`)."""
         B = ids.shape[0]
         ids_ld = self._ids_ld(ids)
         dout_ld = _row_major_2d(_chk(dout, torch.float32, "dout", contiguous=False), "dout")
@@ -247,7 +258,7 @@ class LookupPlan:
                 self._ws = torch.empty(need, device=self.device, dtype=torch.uint8)
             workspace = self._ws
         op = OptParams()
-        op.opt = _lib.OPT_SGD if opt == "sgd" else _lib.OPT_ADAM_LAZY
+        op.opt = _lib.OPT_SGD if opt == "sgd" else _lib.OPT_ADAGRAD if opt == "adagrad" else _lib.OPT_ADAM_LAZY
         op.lr, op.beta1, op.beta2, op.eps, op.l2_scale = lr, beta1, beta2, eps, l2_scale
         op.bias_corr1, op.bias_corr2 = 1.0 - beta1 ** step, 1.0 - beta2 ** step
         trial = self._next_bwd_trial(B) if autotune else None
@@ -438,6 +449,10 @@ def sgd_step(param, grad, lr, l2_scale=0.0):
     call("hrb_sgd_step", _p(param), _p(grad), param.numel(), lr, l2_scale, _stream())
 
 
+def adagrad_step(param, grad, acc, lr, eps=1e-7, l2_scale=0.0):
+    call("hrb_adagrad_step", _p(param), _p(grad), _p(acc), param.numel(), lr, eps, l2_scale, _stream())
+
+
 def _ptr_array(tensors):
     return (ctypes.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors])
 
@@ -462,6 +477,17 @@ def sgd_step_multi(params, grads, l2_scales, lr):
         _chk(t, torch.float32, "tensor")
     call("hrb_sgd_step_multi", n, _ptr_array(params), _ptr_array(grads), (ctypes.c_int64 * n)(*[p.numel() for p in params]),
          (ctypes.c_float * n)(*l2_scales), lr, _stream())
+
+
+def adagrad_step_multi(params, grads, accs, l2_scales, lr, eps=1e-7):
+    """hrb_adagrad_step for a list of tensors in one launch (per HRB_MULTI_MAX tensors)."""
+    n = len(params)
+    if n == 0:
+        return
+    for t in list(params) + list(grads) + list(accs):
+        _chk(t, torch.float32, "tensor")
+    call("hrb_adagrad_step_multi", n, _ptr_array(params), _ptr_array(grads), _ptr_array(accs),
+         (ctypes.c_int64 * n)(*[p.numel() for p in params]), (ctypes.c_float * n)(*l2_scales), lr, eps, _stream())
 
 
 # --------------------------------------------------------------------------------------------

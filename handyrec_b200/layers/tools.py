@@ -74,7 +74,8 @@ class CustomEmbedding(Layer):
         self.built = True
 
     # Tables with at least this many rows keep their gradient sparse (TF: IndexedSlices) and take the touched-rows-only update
-    # (lazy Adam: a declared deviation from Keras' dense Adam step, DESIGN.md 3); smaller ones get the dense Keras-exact step.
+    # (lazy Adam: a declared deviation from Keras' dense Adam step, DESIGN.md 3; Adagrad: Keras' own sparse step, exact while
+    # l2 = 0); smaller ones get the dense Keras-exact step.
     SPARSE_UPDATE_MIN_ROWS = 131072
 
     _sharded = None  # (rank, n_ranks, full rows) when `embeddings` is this rank's row shard
@@ -101,19 +102,23 @@ class CustomEmbedding(Layer):
         if not pending:
             return
         from .. import kernels as K
-        from ..keras_lite import Adam
+        from ..keras_lite import Adagrad, Adam
 
         ids = torch.cat([i for i, _ in pending]).reshape(-1, 1).contiguous()
         rows = torch.cat([g for _, g in pending]).contiguous()
         pending.clear()
-        adam = isinstance(optimizer, Adam)
+        adam, adagrad = isinstance(optimizer, Adam), isinstance(optimizer, Adagrad)
         if getattr(self, "_plan", None) is None:
             w = self.embeddings.data
             self._m, self._v = (torch.zeros_like(w), torch.zeros_like(w)) if adam else (None, None)
-            self._plan = K.LookupPlan([w], [(0, 1, "none", 0, 0)], [self._m] if adam else None, [self._v] if adam else None)
+            self._accum = torch.full_like(w, optimizer.initial_accumulator_value) if adagrad else None
+            self._plan = K.LookupPlan([w], [(0, 1, "none", 0, 0)], [self._m] if adam else None, [self._v] if adam else None,
+                                      accum=[self._accum] if adagrad else None)
         if adam:
             self._plan.backward_update(ids, rows, opt="adam", lr=optimizer.lr, l2_scale=2.0 * self.l2, beta1=optimizer.b1, beta2=optimizer.b2,
                                        eps=optimizer.eps, step=max(optimizer.t, 1), autotune=True)
+        elif adagrad:
+            self._plan.backward_update(ids, rows, opt="adagrad", lr=optimizer.lr, l2_scale=2.0 * self.l2, eps=optimizer.eps, autotune=True)
         else:
             self._plan.backward_update(ids, rows, opt="sgd", lr=optimizer.lr, l2_scale=2.0 * self.l2, autotune=True)
 

@@ -235,14 +235,16 @@ class FusedDeepFM:
 
     def build(self, batch_size: int, optimizer) -> None:
         from .engine import DeepFMEngine
-        from .keras_lite import Adam, SGD
+        from .keras_lite import Adagrad, Adam, SGD
 
         if isinstance(optimizer, Adam):
             opt, lr = "adam", optimizer.lr
         elif isinstance(optimizer, SGD):
             opt, lr = "sgd", optimizer.lr
+        elif isinstance(optimizer, Adagrad):
+            opt, lr = "adagrad", optimizer.lr
         else:
-            raise ValueError("the fused DeepFM path takes keras_lite.Adam or keras_lite.SGD")
+            raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD or keras_lite.Adagrad")
         if self.engine is not None and self.engine.B >= batch_size and self._opt_key == (opt, lr):
             return
         self.sync_to_layers()
@@ -252,6 +254,8 @@ class FusedDeepFM:
         small = getattr(self.model, "dense_table_max_rows", 131072)
         common = dict(dnn_hidden_units=tuple(dnn.hidden_units), dnn_activation=dnn.activation or "linear", batch_size=batch_size, optimizer=opt,
                       lr=lr, l2_embd=self.spec.fields[0].emb.l2, l2_dnn=float(dnn.l2_reg or 0.0), seed=dnn.seed)
+        if opt == "adagrad":  # the engine fills its accumulators when it is built
+            common["initial_accumulator_value"] = optimizer.initial_accumulator_value
         comm = getattr(self.model, "_comm", None)
         if comm is not None and comm.N > 1:
             eng = self._build_sharded(comm, dev, fields, small, common)
@@ -260,6 +264,8 @@ class FusedDeepFM:
             eng = DeepFMEngine(tabs, fields, self.n_dense, dense_table_max_rows=small, **common)
         if opt == "adam":
             eng.beta1, eng.beta2, eng.eps = optimizer.b1, optimizer.b2, optimizer.eps
+        elif opt == "adagrad":
+            eng.eps = optimizer.eps
         for i, d in enumerate(self._dense_layers()):
             eng.set_dense_weights(i, d.kernel.data.cpu(), d.bias.data.cpu())
         eng.fm_w.copy_(self.spec.fm.linear.data.reshape(-1).to(dev))

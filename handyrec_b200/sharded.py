@@ -342,7 +342,8 @@ class ShardedDeepFMEngine(DeepFMEngine):
                 return None
             m = [self.adam_m[t] for t in tabs] if (with_moments and self.adam_m is not None) else None
             v = [self.adam_v[t] for t in tabs] if (with_moments and self.adam_v is not None) else None
-            return K.LookupPlan([self.tables[t] for t in tabs], flds, m, v)
+            acc = [self.accum[t] for t in tabs] if (with_moments and self.accum is not None) else None
+            return K.LookupPlan([self.tables[t] for t in tabs], flds, m, v, accum=acc)
 
         if self.replicated:
             self.plan_shard = sub_plan(self.sharded, True)

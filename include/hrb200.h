@@ -102,8 +102,8 @@ int hrb_seq_pool_bwd(const float* x, const uint8_t* mask, const float* dout, int
  * ------------------------------------------------------------------------------------------ */
 typedef struct hrb_table_desc {
   float* weight;  /* (rows, dim) fp32, 16-byte aligned                        */
-  float* adam_m;  /* optional first moment  (same shape) or NULL              */
-  float* adam_v;  /* optional second moment (same shape) or NULL              */
+  float* adam_m;  /* optimiser state: Adam m / Adagrad accumulator (same shape) or NULL */
+  float* adam_v;  /* Adam second moment (same shape) or NULL; NULL under Adagrad     */
   int64_t rows;   /* vocab_size                                               */
   int32_t dim;    /* embedding dim                                            */
   int32_t pad_;
@@ -142,8 +142,10 @@ int hrb_lookup_fm_fwd(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, 
  *   Sort (table,row) keys -> segment-reduce -> per-unique-row update, no atomics.
  *   opt = HRB_OPT_SGD:       w[r] -= lr * (g[r] + l2_scale*w[r])        (touched rows only)
  *   opt = HRB_OPT_ADAM_LAZY: Adam moments/weights updated for touched rows only (needs adam_m/adam_v)
+ *   opt = HRB_OPT_ADAGRAD:   g' = g[r] + l2_scale*w[r]; acc[r] += g'^2; w[r] -= lr * g' / (sqrt(acc[r]) + eps)
+ *                            (touched rows only, acc in adam_m; Keras ResourceSparseApplyAdagradV2 on the summed rows)
  *   max-pooled fields are not supported here (use a6 bwd + hrb_embedding_bwd_dense). */
-typedef enum hrb_opt { HRB_OPT_SGD = 0, HRB_OPT_ADAM_LAZY = 1 } hrb_opt;
+typedef enum hrb_opt { HRB_OPT_SGD = 0, HRB_OPT_ADAM_LAZY = 1, HRB_OPT_ADAGRAD = 2 } hrb_opt;
 typedef struct hrb_opt_params {
   int32_t opt;
   float lr, beta1, beta2, eps, l2_scale; /* l2_scale = 2*l2_embd (features/group.py:289) */
@@ -360,10 +362,12 @@ int hrb_host_pack_f32(const void* const* cols_host, const int32_t* dtype_host, c
  * write-back off (measurements); returns what the CPU offers: 2 clwb, 1 clflushopt, 0 neither (then the call has no effect). */
 int hrb_host_pack_set_writeback(int32_t on);
 
-/* Dense-parameter optimisers on a flat fp32 buffer (Keras Adam / SGD formulas). */
+/* Dense-parameter optimisers on a flat fp32 buffer (Keras Adam / SGD / Adagrad formulas).  Adagrad (ResourceApplyAdagradV2):
+ * g' = grad + l2_scale*param; acc += g'^2; param -= lr * g' / (sqrt(acc) + eps), acc starting at initial_accumulator_value. */
 int hrb_adam_step(float* param, const float* grad, float* m, float* v, int64_t n, float lr, float beta1,
                   float beta2, float eps, float bias_corr1, float bias_corr2, float l2_scale, void* stream);
 int hrb_sgd_step(float* param, const float* grad, int64_t n, float lr, float l2_scale, void* stream);
+int hrb_adagrad_step(float* param, const float* grad, float* acc, int64_t n, float lr, float eps, float l2_scale, void* stream);
 /* The same steps for `count` parameter tensors in one launch per HRB_MULTI_MAX tensors (host arrays of device pointers / sizes /
  * per-tensor l2 scales; l2_scale_host may be NULL).  The layer-by-layer models (DIN, the retrieval towers) hold 12-27 small
  * tensors; Keras applies one optimiser op per variable (keras optimizer_v2 _resource_apply_dense), here they share a launch. */
@@ -373,6 +377,8 @@ int hrb_adam_step_multi(int32_t count, float* const* param_host, const float* co
                         float beta2, float eps, float bias_corr1, float bias_corr2, void* stream);
 int hrb_sgd_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, const int64_t* n_host,
                        const float* l2_scale_host, float lr, void* stream);
+int hrb_adagrad_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, float* const* acc_host,
+                           const int64_t* n_host, const float* l2_scale_host, float lr, float eps, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * (e) row-sharded tables: owner(r) = r % n_ranks, local row r / n_ranks  (SURVEY §8e).
@@ -385,7 +391,7 @@ int hrb_sgd_step_multi(int32_t count, float* const* param_host, const float* con
  *   owner      hrb_rows_by_key   out[j,:] = shard row addressed by keys[j]
  *   requester  hrb_scatter_rows  rows -> output block (plain features) / position buffer + pooling (sequence features)
  *   requester  hrb_gather_grads  send[j,:] = dout[b, field(perm[j]) columns] * (1/n_valid for mean pooling)
- *   owner      hrb_keyed_bwd_update  (key, gradient row) pairs -> sort -> segment-reduce -> SGD / lazy-Adam row update */
+ *   owner      hrb_keyed_bwd_update  (key, gradient row) pairs -> sort -> segment-reduce -> SGD / lazy-Adam / Adagrad row update */
 /* Peer-mapped lookup: peer_tables_host[r*n_tables + t] = device pointer of rank r's shard of table t as mapped into this
  * process (CUDA IPC / symmetric memory over NVLink), full_rows_host[t] = full vocabulary size.  After this call
  * hrb_lookup_fwd / hrb_lookup_fm_fwd take GLOBAL ids and read row id from rank id % n_ranks at local row id / n_ranks:
