@@ -20,7 +20,7 @@ HRB_OK, HRB_BAD_ARG, HRB_UNSUPPORTED, HRB_CUDA_ERROR, HRB_WORKSPACE = 0, 1, 2, 3
 # enums
 POOL = {"none": 0, None: 0, "mean": 1, "sum": 2, "max": 3}
 ACT = {None: 0, "linear": 0, "relu": 1, "sigmoid": 2, "tanh": 3, "dice": 4}
-OPT_SGD, OPT_ADAM_LAZY, OPT_ADAGRAD = 0, 1, 2
+OPT_SGD, OPT_ADAM_LAZY, OPT_ADAGRAD, OPT_FTRL = 0, 1, 2, 3
 GEMM_AUTO, GEMM_FP32, GEMM_3XTF32 = 0, 1, 2
 BWD_AUTO, BWD_UNITS, BWD_SORT = 0, 1, 2
 
@@ -63,6 +63,10 @@ class OptParams(ctypes.Structure):
         ("l2_scale", ctypes.c_float),
         ("bias_corr1", ctypes.c_float),
         ("bias_corr2", ctypes.c_float),
+        ("l1", ctypes.c_float),  # Ftrl only (l2: with beta / (2*lr) added)
+        ("l2", ctypes.c_float),
+        ("lr_power", ctypes.c_float),
+        ("l2_shrinkage", ctypes.c_float),
     ]
 
 

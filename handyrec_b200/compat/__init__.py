@@ -93,7 +93,7 @@ def _tf_module() -> types.ModuleType:
     losses = types.ModuleType("tensorflow.keras.losses")
     losses.binary_crossentropy = KL.binary_crossentropy
     opts = types.ModuleType("tensorflow.keras.optimizers")
-    opts.Adam, opts.SGD, opts.Adagrad = KL.Adam, KL.SGD, KL.Adagrad
+    opts.Adam, opts.SGD, opts.Adagrad, opts.Ftrl = KL.Adam, KL.SGD, KL.Adagrad, KL.Ftrl
     keras.layers, keras.models, keras.initializers, keras.regularizers, keras.losses, keras.optimizers = layers, models, inits, regs, losses, opts
     tf.keras = keras
     tf._submodules = {"tensorflow.nn": nn, "tensorflow.keras": keras, "tensorflow.keras.layers": layers, "tensorflow.keras.models": models,

@@ -74,6 +74,24 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// Keras Ftrl (TF ApplyFtrl / ApplyFtrlV2 functors) on one element; acc and lin are its accumulator and linear slots, g already
+// holds the l2 regulariser term, l2 has beta / (2*lr) added.  Returns the new weight.  The row update (plan.cuh), the dense step
+// and the multi-tensor step (misc.cu) all call this: every operation is rounded explicitly (no contraction left to the
+// compiler), so a step from the same slots gives the same bits on every path.  The final select (not a multiply) keeps a
+// y of 0 (acc = 0, l2 = 0) from turning the 0 of a small |linear| into NaN.
+__device__ __forceinline__ float ftrl_pow(float a, float lr_power) { return lr_power == -0.5f ? __fsqrt_rn(a) : powf(a, -lr_power); }
+__device__ __forceinline__ float ftrl_elem(float w, float& acc, float& lin, float g, float lr, float l1, float l2, float lr_power,
+                                           float l2_shrinkage) {
+  const float gs = __fadd_rn(g, __fmul_rn(__fmul_rn(2.f, l2_shrinkage), w));
+  const float acc_new = __fadd_rn(acc, __fmul_rn(g, g));
+  const float p_new = ftrl_pow(acc_new, lr_power);
+  const float sigma = __fdiv_rn(__fsub_rn(p_new, ftrl_pow(acc, lr_power)), lr);
+  lin = __fadd_rn(lin, __fsub_rn(gs, __fmul_rn(sigma, w)));
+  acc = acc_new;
+  const float y = __fadd_rn(__fdiv_rn(p_new, lr), __fmul_rn(2.f, l2));
+  return fabsf(lin) > l1 ? __fdiv_rn(__fsub_rn(copysignf(l1, lin), lin), y) : 0.f;
+}
+
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
 
 __device__ __forceinline__ float act_apply(int act, float x) {

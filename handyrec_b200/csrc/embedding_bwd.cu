@@ -996,6 +996,7 @@ int run_unit_update(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, in
 #define HRB_UNITS(GG)                                                                      \
   rc = mode == UPD_ADAM      ? launch_units<UPD_ADAM, GG>(a, us, gi, st)                   \
        : mode == UPD_ADAGRAD ? launch_units<UPD_ADAGRAD, GG>(a, us, gi, st)                \
+       : mode == UPD_FTRL    ? launch_units<UPD_FTRL, GG>(a, us, gi, st)                   \
                              : launch_units<UPD_SGD, GG>(a, us, gi, st);                   \
   break;
     switch (us.g_values[gi]) {

@@ -556,7 +556,7 @@ __device__ __forceinline__ int find_table(const TableDev* __restrict__ t, int n,
   return lo;
 }
 
-template <int MODE>  // UpdMode: sgd, adam lazy, adagrad, or dense gradient add
+template <int MODE>  // UpdMode: sgd, adam lazy, adagrad, ftrl, or dense gradient add
 __device__ __forceinline__ void apply_row(const ApplyCtx& c, uint32_t key, int q, float4 g) {
   if (MODE == UPD_DENSE_ADD) {
     float4* p = reinterpret_cast<float4*>(c.dense_out + (int64_t)key * c.tables[0].dim) + q;
@@ -973,6 +973,8 @@ static int run_sorted_update(int mode, const BwdWorkspace& w, int64_t n, uint32_
     HRB_RUN_MODE(UPD_ADAM)
   } else if (mode == UPD_ADAGRAD) {
     HRB_RUN_MODE(UPD_ADAGRAD)
+  } else if (mode == UPD_FTRL) {
+    HRB_RUN_MODE(UPD_FTRL)
   } else {
     HRB_RUN_MODE(UPD_DENSE_ADD)
   }
@@ -1284,6 +1286,126 @@ HRB_API int hrb_lookup_fm_fwd(const hrb_plan* plan, const int32_t* ids, int64_t 
                            (cudaStream_t)stream);
 }
 
+// ---------------------------------------------------------------------------------------------
+// Touched rows for Ftrl, whose step with a zero gradient is not a no-op.  Keras gathers id 0 at the padding positions of a
+// pooled field, so row 0 is in the IndexedSlices gradient (with a zero gradient) and steps; the backward above drops those
+// positions.  mark_rows_kernel flags the touched rows of dense-updated tables; pad_flags_kernel notes per table whether the
+// batch holds padding (flags[2t]) and whether a valid position names row 0 (flags[2t+1], then the backward steps row 0 with
+// the gradient sum); ftrl_pad_kernel gives row 0 its zero-gradient step where only padding named it.  Every writer of a flag
+// stores the same value, so plain stores suffice.
+// ---------------------------------------------------------------------------------------------
+constexpr int MARK_MAX_TABLES = 512;
+struct TouchedPtrs {
+  float* p[MARK_MAX_TABLES];
+};
+
+__global__ void __launch_bounds__(256) mark_rows_kernel(const FieldDev* __restrict__ fields, int32_t n_fields, const int32_t* __restrict__ ids,
+                                                       int64_t ids_ld, int64_t batch, const TouchedPtrs tp) {
+  const int64_t total = batch * n_fields;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = i / n_fields;
+    const FieldDev& f = fields[i - b * n_fields];
+    float* touched = tp.p[f.table_idx];
+    if (touched == nullptr) continue;
+    const int32_t* idp = ids + b * ids_ld + f.ids_col;
+    for (int l = 0; l < f.seq_len; ++l) {
+      const int32_t id = idp[l];
+      if (id >= 0 && (int64_t)id < f.rows) touched[id] = 1.0f;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(256) pad_flags_kernel(const FieldDev* __restrict__ fields, int32_t n_fields, const int32_t* __restrict__ ids,
+                                                       int64_t ids_ld, int64_t batch, float* __restrict__ flags) {
+  const int64_t total = batch * n_fields;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = i / n_fields;
+    const FieldDev& f = fields[i - b * n_fields];
+    const int32_t* idp = ids + b * ids_ld + f.ids_col;
+    bool zero = false;
+    for (int l = 0; l < f.seq_len; ++l) zero |= idp[l] == 0;
+    float* fl = flags + 2 * f.table_idx + (f.pool == HRB_POOL_NONE ? 1 : 0);  // id 0 of a pooled field is padding
+    if (zero && *fl == 0.f) *fl = 1.0f;
+  }
+}
+
+// one CTA: row 0 of every row-updated table whose batch held padding and no valid id 0 takes a zero-gradient step
+__global__ void __launch_bounds__(256) ftrl_pad_kernel(const TableDev* __restrict__ tables, int32_t n_tables, const float* __restrict__ flags,
+                                                      const hrb_opt_params opt) {
+  for (int32_t ti = 0; ti < n_tables; ++ti) {
+    const TableDev& t = tables[ti];
+    if (t.grad != nullptr || flags[2 * ti] == 0.f || flags[2 * ti + 1] != 0.f) continue;
+    for (int e = threadIdx.x; e < t.dim; e += blockDim.x) {
+      const float w = t.w[e];
+      float a = t.m[e], l = t.v[e];
+      t.w[e] = ftrl_elem(w, a, l, fmaf(opt.l2_scale, w, 0.f), opt.lr, opt.l1, opt.l2, opt.lr_power, opt.l2_shrinkage);
+      t.m[e] = a;
+      t.v[e] = l;
+    }
+  }
+}
+
+static bool has_pooled(const hrb_plan* plan) {
+  for (const auto& f : plan->fdev_host)
+    if (f.pool != HRB_POOL_NONE) return true;
+  return false;
+}
+// the padding flags of hrb_lookup_bwd_update under Ftrl sit in the last bytes of its workspace
+static size_t pad_flag_bytes(const hrb_plan* plan) { return has_pooled(plan) ? align_up((size_t)plan->n_tables * 8) : 0; }
+
+static int ftrl_tables_ok(const hrb_plan* plan, const char* who) {
+  for (const auto& t : plan->tdev_host)
+    HRB_REQUIRE(t.grad || (t.m && t.v), "%s: Ftrl needs an accumulator (adam_m) and a linear slot (adam_v) for every row-updated table", who);
+  return HRB_OK;
+}
+
+static int launch_pad_flags(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, float* flags, cudaStream_t st) {
+  HRB_CUDA(cudaMemsetAsync(flags, 0, (size_t)plan->n_tables * 8, st));
+  pad_flags_kernel<<<grid_for(batch * plan->n_fields, 256), 256, 0, st>>>(plan->d_fields, plan->n_fields, ids, ids_ld, batch, flags);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+static int launch_ftrl_pad(const hrb_plan* plan, const float* flags, const hrb_opt_params& opt, cudaStream_t st) {
+  ftrl_pad_kernel<<<1, 256, 0, st>>>(plan->d_tables, plan->n_tables, flags, opt);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+HRB_API int hrb_plan_mark_rows(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, float* const* touched_host,
+                               void* stream) {
+  HRB_REQUIRE(plan && ids && touched_host && batch >= 0, "hrb_plan_mark_rows: null/negative argument");
+  if (plan->n_tables > MARK_MAX_TABLES) return fail(HRB_UNSUPPORTED, "hrb_plan_mark_rows: more than %d tables", MARK_MAX_TABLES);
+  TouchedPtrs tp{};
+  bool any = false;
+  for (int32_t t = 0; t < plan->n_tables; ++t) {
+    tp.p[t] = touched_host[t];
+    any |= touched_host[t] != nullptr;
+  }
+  if (batch == 0 || !any) return HRB_OK;
+  mark_rows_kernel<<<grid_for(batch * plan->n_fields, 256), 256, 0, (cudaStream_t)stream>>>(plan->d_fields, plan->n_fields, ids, ids_ld,
+                                                                                           batch, tp);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+HRB_API int hrb_plan_pad_flags(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, float* flags, void* stream) {
+  HRB_REQUIRE(plan && ids && flags && batch >= 0, "hrb_plan_pad_flags: null/negative argument");
+  if (batch == 0) return HRB_OK;
+  pad_flags_kernel<<<grid_for(batch * plan->n_fields, 256), 256, 0, (cudaStream_t)stream>>>(plan->d_fields, plan->n_fields, ids, ids_ld,
+                                                                                           batch, flags);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+HRB_API int hrb_plan_ftrl_pad_step(const hrb_plan* plan, const float* flags, const hrb_opt_params* opt_host, void* stream) {
+  HRB_REQUIRE(plan && flags && opt_host, "hrb_plan_ftrl_pad_step: null argument");
+  HRB_REQUIRE(opt_host->opt == HRB_OPT_FTRL, "hrb_plan_ftrl_pad_step: needs HRB_OPT_FTRL, got %d", opt_host->opt);
+  int rc = ftrl_tables_ok(plan, "hrb_plan_ftrl_pad_step");
+  if (rc != HRB_OK) return rc;
+  return launch_ftrl_pad(plan, flags, load_opt(opt_host), (cudaStream_t)stream);
+}
+
 HRB_API int hrb_lookup_bwd_workspace(const hrb_plan* plan, int64_t ids_ld, int64_t batch, size_t* bytes) {
   HRB_REQUIRE(plan && bytes && batch >= 0, "hrb_lookup_bwd_workspace: null/negative argument");
   (void)ids_ld;
@@ -1294,8 +1416,12 @@ HRB_API int hrb_lookup_bwd_workspace(const hrb_plan* plan, int64_t ids_ld, int64
   if (rc != HRB_OK) return rc;
   *bytes = w.total;
   if (unit_path_supported(plan, batch)) *bytes = std::max(w.total, unit_workspace_bytes(plan, batch));
+  if (const size_t fb = pad_flag_bytes(plan)) *bytes = align_up(*bytes) + fb;  // hrb_lookup_bwd_update keeps the flags in the last fb bytes
   return HRB_OK;
 }
+
+static int run_plan_sorted_update(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, const float* dout,
+                                  int64_t dout_ld, const hrb_opt_params& opt, void* workspace, size_t workspace_bytes, cudaStream_t st);
 
 HRB_API int hrb_lookup_bwd_update(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch,
                                   const float* dout, int64_t dout_ld, const float* inv_count,
@@ -1306,37 +1432,64 @@ HRB_API int hrb_lookup_bwd_update(const hrb_plan* plan, const int32_t* ids, int6
   HRB_REQUIRE(aligned16(dout) && dout_ld % 4 == 0, "hrb_lookup_bwd_update: dout must be 16-byte aligned, dout_ld %% 4 == 0");
   if (plan->has_max)
     return fail(HRB_UNSUPPORTED, "hrb_lookup_bwd_update: max-pooled fields go through hrb_seq_pool_bwd + hrb_embedding_bwd_dense");
-  HRB_REQUIRE(opt_host->opt == HRB_OPT_SGD || opt_host->opt == HRB_OPT_ADAM_LAZY || opt_host->opt == HRB_OPT_ADAGRAD,
-              "hrb_lookup_bwd_update: unknown optimiser %d", opt_host->opt);
-  if (opt_host->opt == HRB_OPT_ADAM_LAZY)
+  const hrb_opt_params opt = load_opt(opt_host);
+  HRB_REQUIRE(opt.opt == HRB_OPT_SGD || opt.opt == HRB_OPT_ADAM_LAZY || opt.opt == HRB_OPT_ADAGRAD || opt.opt == HRB_OPT_FTRL,
+              "hrb_lookup_bwd_update: unknown optimiser %d", opt.opt);
+  if (opt.opt == HRB_OPT_ADAM_LAZY)
     for (const auto& t : plan->tdev_host)
       HRB_REQUIRE(t.grad || (t.m && t.v), "hrb_lookup_bwd_update: lazy Adam needs adam_m/adam_v for every table");
-  if (opt_host->opt == HRB_OPT_ADAGRAD)
+  if (opt.opt == HRB_OPT_ADAGRAD)
     for (const auto& t : plan->tdev_host)
       HRB_REQUIRE(t.grad || t.m, "hrb_lookup_bwd_update: Adagrad needs an accumulator (adam_m) for every row-updated table");
+  if (opt.opt == HRB_OPT_FTRL) {
+    int rc = ftrl_tables_ok(plan, "hrb_lookup_bwd_update");
+    if (rc != HRB_OK) return rc;
+  }
   const int G = plan->max_dim / 4;
   if (G > 256) return fail(HRB_UNSUPPORTED, "hrb_lookup_bwd_update: dim %d too large", plan->max_dim);
   if (batch == 0) return HRB_OK;
   const int64_t n = batch * plan->pos_cols;
   HRB_REQUIRE(n < 0x7FFFFFFFll, "hrb_lookup_bwd_update: batch*sum(seq_len) exceeds 2^31-1");
+  cudaStream_t st = (cudaStream_t)stream;
+  // Ftrl with pooled fields: the padding flags come from the ids before the backward, row 0 takes its padding step after it
+  float* pad_flags = nullptr;
+  if (opt.opt == HRB_OPT_FTRL && has_pooled(plan)) {
+    const size_t fb = pad_flag_bytes(plan);
+    if (workspace_bytes < fb) return fail(HRB_WORKSPACE, "hrb_lookup_bwd_update: workspace %zu < %zu bytes of padding flags", workspace_bytes, fb);
+    workspace_bytes = (workspace_bytes - fb) / 256 * 256;
+    pad_flags = (float*)((char*)workspace + workspace_bytes);
+    int rc = launch_pad_flags(plan, ids, ids_ld, batch, pad_flags, st);
+    if (rc != HRB_OK) return rc;
+  }
+  int rc = HRB_OK;
   if (plan->bwd_algo != HRB_BWD_SORT && unit_path_supported(plan, batch))  // two-level partition, one CTA per row range (embedding_bwd.cu)
-    return run_unit_update(plan, ids, ids_ld, batch, dout, dout_ld, *opt_host, workspace, workspace_bytes, (cudaStream_t)stream);
+    rc = run_unit_update(plan, ids, ids_ld, batch, dout, dout_ld, opt, workspace, workspace_bytes, st);
+  else
+    rc = run_plan_sorted_update(plan, ids, ids_ld, batch, dout, dout_ld, opt, workspace, workspace_bytes, st);
+  if (rc != HRB_OK || pad_flags == nullptr) return rc;
+  return launch_ftrl_pad(plan, pad_flags, opt, st);
+}
+
+// the SORT algorithm of hrb_lookup_bwd_update (global radix sort of the (table,row) keys)
+static int run_plan_sorted_update(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, const float* dout,
+                                  int64_t dout_ld, const hrb_opt_params& opt, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const int G = plan->max_dim / 4;
+  const int64_t n = batch * plan->pos_cols;
   BwdWorkspace w;
   int rc = carve_bwd_ws(n, batch * plan->n_fields + 1, plan->max_dim, plan->key_bits, workspace, w);
   if (rc != HRB_OK) return rc;
   if (w.total > workspace_bytes)
     return fail(HRB_WORKSPACE, "hrb_lookup_bwd_update: workspace %zu < required %zu bytes", workspace_bytes, w.total);
-  cudaStream_t st = (cudaStream_t)stream;
   const uint32_t sentinel = (uint32_t)plan->total_rows;
   bwd_keys_kernel<<<grid_for(batch * plan->n_fields, 256), 256, 0, st>>>(plan->d_fields, plan->n_fields, plan->pos_cols,
                                                                         ids, ids_ld, batch, sentinel, w.keys_in,
                                                                         w.vals_in, w.scale);
   HRB_LAUNCH_CHECK();
   PlanGrad src{plan->d_fields, plan->d_pos_field, dout, w.scale, dout_ld, plan->pos_cols, plan->n_fields};
-  ApplyCtx ctx{plan->d_tables, plan->n_tables, *opt_host, nullptr, 0.f};
-  if (opt_host->opt == HRB_OPT_ADAM_LAZY)
-    ctx.lr_t = opt_host->lr * sqrtf(opt_host->bias_corr2) / opt_host->bias_corr1;
-  return run_sorted_update(upd_mode(opt_host->opt), w, n, sentinel, plan->key_bits, G, src, ctx, hot_from_plan(plan), st);
+  ApplyCtx ctx{plan->d_tables, plan->n_tables, opt, nullptr, 0.f};
+  if (opt.opt == HRB_OPT_ADAM_LAZY)
+    ctx.lr_t = opt.lr * sqrtf(opt.bias_corr2) / opt.bias_corr1;
+  return run_sorted_update(upd_mode(opt.opt), w, n, sentinel, plan->key_bits, G, src, ctx, hot_from_plan(plan), st);
 }
 
 HRB_API int hrb_embedding_bwd_dense_workspace(int64_t n_ids, int32_t dim, size_t* bytes) {
@@ -1742,12 +1895,16 @@ HRB_API int hrb_keyed_bwd_update(const hrb_plan* plan, const uint32_t* keys, con
   if (n == 0) return HRB_OK;
   HRB_REQUIRE(keys && grads && aligned16(grads), "hrb_keyed_bwd_update: null/misaligned pointer");
   if (!plan->uniform_dim) return fail(HRB_UNSUPPORTED, "hrb_keyed_bwd_update: needs one embedding dim");
-  HRB_REQUIRE(opt_host->opt == HRB_OPT_SGD || opt_host->opt == HRB_OPT_ADAM_LAZY || opt_host->opt == HRB_OPT_ADAGRAD,
-              "hrb_keyed_bwd_update: unknown optimiser %d", opt_host->opt);
-  if (opt_host->opt == HRB_OPT_ADAM_LAZY)
+  const hrb_opt_params opt = load_opt(opt_host);
+  HRB_REQUIRE(opt.opt == HRB_OPT_SGD || opt.opt == HRB_OPT_ADAM_LAZY || opt.opt == HRB_OPT_ADAGRAD || opt.opt == HRB_OPT_FTRL,
+              "hrb_keyed_bwd_update: unknown optimiser %d", opt.opt);
+  if (opt.opt == HRB_OPT_ADAM_LAZY)
     for (const auto& t : plan->tdev_host) HRB_REQUIRE(t.m && t.v, "hrb_keyed_bwd_update: lazy Adam needs adam_m/adam_v for every table");
-  if (opt_host->opt == HRB_OPT_ADAGRAD)
+  if (opt.opt == HRB_OPT_ADAGRAD)
     for (const auto& t : plan->tdev_host) HRB_REQUIRE(t.m, "hrb_keyed_bwd_update: Adagrad needs an accumulator (adam_m) for every table");
+  if (opt.opt == HRB_OPT_FTRL)
+    for (const auto& t : plan->tdev_host)
+      HRB_REQUIRE(t.m && t.v, "hrb_keyed_bwd_update: Ftrl needs an accumulator (adam_m) and a linear slot (adam_v) for every table");
   BwdWorkspace w;
   int rc = carve_bwd_ws(n, 1, plan->max_dim, plan->key_bits, workspace, w);
   if (rc != HRB_OK) return rc;
@@ -1759,9 +1916,9 @@ HRB_API int hrb_keyed_bwd_update(const hrb_plan* plan, const uint32_t* keys, con
                                                     (uint32_t)plan->total_rows, w.keys_in, w.vals_in);
   HRB_LAUNCH_CHECK();
   FlatGrad src{grads, plan->max_dim};
-  ApplyCtx ctx{plan->d_tables, plan->n_tables, *opt_host, nullptr, 0.f};
-  if (opt_host->opt == HRB_OPT_ADAM_LAZY) ctx.lr_t = opt_host->lr * sqrtf(opt_host->bias_corr2) / opt_host->bias_corr1;
-  return run_sorted_update(upd_mode(opt_host->opt), w, n, (uint32_t)plan->total_rows, plan->key_bits, plan->max_dim / 4, src, ctx,
+  ApplyCtx ctx{plan->d_tables, plan->n_tables, opt, nullptr, 0.f};
+  if (opt.opt == HRB_OPT_ADAM_LAZY) ctx.lr_t = opt.lr * sqrtf(opt.bias_corr2) / opt.bias_corr1;
+  return run_sorted_update(upd_mode(opt.opt), w, n, (uint32_t)plan->total_rows, plan->key_bits, plan->max_dim / 4, src, ctx,
                            hot_from_plan(plan), st);
 }
 

@@ -2,7 +2,7 @@
 //
 // Reference: models/ranking/context_aware/DeepFM.py:86-88 (dnn + fm -> sigmoid), Keras
 // binary_crossentropy on a sigmoid output (= sigmoid cross-entropy with logits),
-// layers/activation.py:27-42 (Dice), Keras Adam / SGD update formulas.
+// layers/activation.py:27-42 (Dice), Keras Adam / SGD / Adagrad / Ftrl update formulas.
 #include "common.cuh"
 
 namespace hrb {
@@ -94,9 +94,24 @@ __global__ void __launch_bounds__(256) adagrad_kernel(float* __restrict__ p, con
   }
 }
 
+// Keras Ftrl (ResourceApplyFtrl / V2; ftrl_elem, common.cuh).  row_touched != nullptr: elements of rows (dim floats) whose flag is
+// 0 are neither read nor written -- the rows an embedding table's IndexedSlices gradient does not list keep their bits.
+__global__ void __launch_bounds__(256) ftrl_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ acc,
+                                                  float* __restrict__ lin, int64_t n, float lr, float l1, float l2, float lr_power,
+                                                  float l2_shrinkage, float l2_scale, const float* __restrict__ row_touched, int32_t dim) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    if (row_touched != nullptr && row_touched[i / dim] == 0.f) continue;
+    const float w = p[i];
+    float a = acc[i], l = lin[i];
+    p[i] = ftrl_elem(w, a, l, fmaf(l2_scale, w, g[i]), lr, l1, l2, lr_power, l2_shrinkage);
+    acc[i] = a;
+    lin[i] = l;
+  }
+}
+
 // Many small parameter tensors in ONE launch (the layer-by-layer models step 12-27 tensors: one launch each was 0.4 ms of
 // host time per step).  Block b works on the tensor whose block range contains it; same arithmetic as adam_kernel / sgd_kernel /
-// adagrad_kernel.  m holds the Adagrad accumulator.
+// adagrad_kernel / ftrl_kernel.  m holds the Adagrad or Ftrl accumulator, v the Ftrl linear slot.
 struct MultiArgs {
   float* p[HRB_MULTI_MAX];
   const float* g[HRB_MULTI_MAX];
@@ -107,9 +122,12 @@ struct MultiArgs {
   int32_t first_block[HRB_MULTI_MAX + 1];
   int32_t count;
 };
-enum MultiOpt { MULTI_SGD, MULTI_ADAM, MULTI_ADAGRAD };
+enum MultiOpt { MULTI_SGD, MULTI_ADAM, MULTI_ADAGRAD, MULTI_FTRL };
+struct FtrlArgs {
+  float l1, l2, lr_power, l2_shrinkage;
+};
 template <int OPT>
-__global__ void __launch_bounds__(256) multi_step_kernel(const MultiArgs a, float lr_t, float b1, float b2, float eps) {
+__global__ void __launch_bounds__(256) multi_step_kernel(const MultiArgs a, float lr_t, float b1, float b2, float eps, const FtrlArgs f) {
   int t = 0;
   while (t + 1 < a.count && (int)blockIdx.x >= a.first_block[t + 1]) ++t;
   const int64_t nb = a.first_block[t + 1] - a.first_block[t];
@@ -130,6 +148,11 @@ __global__ void __launch_bounds__(256) multi_step_kernel(const MultiArgs a, floa
       float acc = a.m[t][i];
       p[i] = adagrad_update(w, acc, gi, lr_t, eps);
       a.m[t][i] = acc;
+    } else if (OPT == MULTI_FTRL) {
+      float acc = a.m[t][i], lin = a.v[t][i];
+      p[i] = ftrl_elem(w, acc, lin, gi, lr_t, f.l1, f.l2, f.lr_power, f.l2_shrinkage);
+      a.m[t][i] = acc;
+      a.v[t][i] = lin;
     } else {
       p[i] = w - lr_t * gi;
     }
@@ -309,6 +332,17 @@ HRB_API int hrb_adagrad_step(float* param, const float* grad, float* acc, int64_
   return HRB_OK;
 }
 
+HRB_API int hrb_ftrl_step(float* param, const float* grad, float* acc, float* lin, int64_t n, float lr, float l1, float l2, float lr_power,
+                          float l2_shrinkage, float l2_scale, const float* row_touched, int32_t dim, void* stream) {
+  HRB_REQUIRE(param && grad && acc && lin && n >= 0 && lr > 0.f, "hrb_ftrl_step: bad argument");
+  HRB_REQUIRE(row_touched == nullptr || (dim > 0 && n % dim == 0), "hrb_ftrl_step: n = %lld is not a multiple of dim = %d", (long long)n, dim);
+  if (n == 0) return HRB_OK;
+  ftrl_kernel<<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(param, grad, acc, lin, n, lr, l1, l2, lr_power, l2_shrinkage, l2_scale,
+                                                            row_touched, dim);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
 HRB_API int hrb_sgd_step(float* param, const float* grad, int64_t n, float lr, float l2_scale, void* stream) {
   HRB_REQUIRE(param && grad && n >= 0, "hrb_sgd_step: bad argument");
   if (n == 0) return HRB_OK;
@@ -318,19 +352,20 @@ HRB_API int hrb_sgd_step(float* param, const float* grad, int64_t n, float lr, f
 }
 
 static int multi_step(int opt, int32_t count, float* const* param, const float* const* grad, float* const* m, float* const* v,
-                      const int64_t* n, const float* l2_scale, float lr_t, float b1, float b2, float eps, cudaStream_t st) {
+                      const int64_t* n, const float* l2_scale, float lr_t, float b1, float b2, float eps, cudaStream_t st,
+                      FtrlArgs f = FtrlArgs{}) {
   for (int32_t c0 = 0; c0 < count; c0 += HRB_MULTI_MAX) {
     MultiArgs a{};
     int blocks = 0;
     for (int32_t i = c0; i < count && i < c0 + HRB_MULTI_MAX; ++i) {
-      HRB_REQUIRE(n[i] >= 0 && (n[i] == 0 || (param[i] && grad[i] && (opt == MULTI_SGD || m[i]) && (opt != MULTI_ADAM || v[i]))),
+      HRB_REQUIRE(n[i] >= 0 && (n[i] == 0 || (param[i] && grad[i] && (opt == MULTI_SGD || m[i]) && ((opt != MULTI_ADAM && opt != MULTI_FTRL) || v[i]))),
                   "multi-tensor step: null tensor %d", i);
       if (n[i] == 0) continue;
       const int k = a.count++;
       a.p[k] = param[i];
       a.g[k] = grad[i];
       a.m[k] = opt != MULTI_SGD ? m[i] : nullptr;
-      a.v[k] = opt == MULTI_ADAM ? v[i] : nullptr;
+      a.v[k] = (opt == MULTI_ADAM || opt == MULTI_FTRL) ? v[i] : nullptr;
       a.n[k] = n[i];
       a.l2[k] = l2_scale ? l2_scale[i] : 0.f;
       a.first_block[k] = blocks;
@@ -338,9 +373,10 @@ static int multi_step(int opt, int32_t count, float* const* param, const float* 
     }
     if (a.count == 0) continue;
     a.first_block[a.count] = blocks;
-    if (opt == MULTI_ADAM) multi_step_kernel<MULTI_ADAM><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
-    else if (opt == MULTI_ADAGRAD) multi_step_kernel<MULTI_ADAGRAD><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
-    else multi_step_kernel<MULTI_SGD><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps);
+    if (opt == MULTI_ADAM) multi_step_kernel<MULTI_ADAM><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps, f);
+    else if (opt == MULTI_ADAGRAD) multi_step_kernel<MULTI_ADAGRAD><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps, f);
+    else if (opt == MULTI_FTRL) multi_step_kernel<MULTI_FTRL><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps, f);
+    else multi_step_kernel<MULTI_SGD><<<blocks, 256, 0, st>>>(a, lr_t, b1, b2, eps, f);
     HRB_LAUNCH_CHECK();
   }
   return HRB_OK;
@@ -366,6 +402,15 @@ HRB_API int hrb_adagrad_step_multi(int32_t count, float* const* param_host, cons
   HRB_REQUIRE(count >= 0 && (count == 0 || (param_host && grad_host && acc_host && n_host)), "hrb_adagrad_step_multi: bad argument");
   return multi_step(MULTI_ADAGRAD, count, param_host, grad_host, acc_host, nullptr, n_host, l2_scale_host, lr, 0.f, 0.f, eps,
                     (cudaStream_t)stream);
+}
+
+HRB_API int hrb_ftrl_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, float* const* acc_host,
+                                float* const* lin_host, const int64_t* n_host, const float* l2_scale_host, float lr, float l1, float l2,
+                                float lr_power, float l2_shrinkage, void* stream) {
+  HRB_REQUIRE(count >= 0 && (count == 0 || (param_host && grad_host && acc_host && lin_host && n_host)) && lr > 0.f,
+              "hrb_ftrl_step_multi: bad argument");
+  return multi_step(MULTI_FTRL, count, param_host, grad_host, acc_host, lin_host, n_host, l2_scale_host, lr, 0.f, 0.f, 0.f,
+                    (cudaStream_t)stream, FtrlArgs{l1, l2, lr_power, l2_shrinkage});
 }
 
 HRB_API int hrb_dice_fwd(const float* x, int64_t rows, int32_t units, const float* alpha, float* mean, float* var,

@@ -1,6 +1,7 @@
 // plan.cuh -- the lookup plan (hrb_plan) and its device-side field / table descriptors, shared by lookup.cu and
 // embedding_bwd.cu.
 #pragma once
+#include <cstddef>
 #include <mutex>
 #include <vector>
 
@@ -23,8 +24,8 @@ struct FieldDev {
 
 struct TableDev {
   float* w;
-  float* m;     // optimiser state: Adam first moment / Adagrad accumulator
-  float* v;     // Adam second moment
+  float* m;     // optimiser state: Adam first moment / Adagrad or Ftrl accumulator
+  float* v;     // Adam second moment / Ftrl linear
   int64_t rows;
   uint32_t key_base;
   int32_t dim;
@@ -33,11 +34,33 @@ struct TableDev {
 
 // Row-update modes of apply_table_row(s) and of every kernel that dispatches on them.  UPD_DENSE_ADD is lookup.cu's
 // dense-gradient face (hrb_embedding_bwd_dense), which never reaches apply_table_row(s).
-enum UpdMode : int { UPD_SGD = 0, UPD_ADAM = 1, UPD_DENSE_ADD = 2, UPD_ADAGRAD = 3 };
+enum UpdMode : int { UPD_SGD = 0, UPD_ADAM = 1, UPD_DENSE_ADD = 2, UPD_ADAGRAD = 3, UPD_FTRL = 4 };
 
 // hrb_opt -> UpdMode of the row update
 inline int upd_mode(int32_t opt) {
-  return opt == HRB_OPT_ADAM_LAZY ? UPD_ADAM : opt == HRB_OPT_ADAGRAD ? UPD_ADAGRAD : UPD_SGD;
+  return opt == HRB_OPT_ADAM_LAZY ? UPD_ADAM : opt == HRB_OPT_ADAGRAD ? UPD_ADAGRAD : opt == HRB_OPT_FTRL ? UPD_FTRL : UPD_SGD;
+}
+
+// The caller's hrb_opt_params: the Ftrl fields at its end are read only when opt == HRB_OPT_FTRL (a caller built against the
+// shorter struct of the other optimisers passes fewer bytes), zero otherwise.
+inline hrb_opt_params load_opt(const hrb_opt_params* p) {
+  hrb_opt_params o{};
+  memcpy(&o, p, offsetof(hrb_opt_params, l1));
+  if (o.opt == HRB_OPT_FTRL) {
+    o.l1 = p->l1;
+    o.l2 = p->l2;
+    o.lr_power = p->lr_power;
+    o.l2_shrinkage = p->l2_shrinkage;
+  }
+  return o;
+}
+
+// Keras Ftrl on the four floats of a row chunk (ftrl_elem, common.cuh); a: accumulator, l: linear
+__device__ __forceinline__ void ftrl_row4(float4& w, float4& a, float4& l, const float4& g, const hrb_opt_params& o) {
+  w.x = ftrl_elem(w.x, a.x, l.x, g.x, o.lr, o.l1, o.l2, o.lr_power, o.l2_shrinkage);
+  w.y = ftrl_elem(w.y, a.y, l.y, g.y, o.lr, o.l1, o.l2, o.lr_power, o.l2_shrinkage);
+  w.z = ftrl_elem(w.z, a.z, l.z, g.z, o.lr, o.l1, o.l2, o.lr_power, o.l2_shrinkage);
+  w.w = ftrl_elem(w.w, a.w, l.w, g.w, o.lr, o.l1, o.l2, o.lr_power, o.l2_shrinkage);
 }
 
 // Keras Adagrad (ResourceSparseApplyAdagradV2, eps outside the square root) on one float of a row; acc is the table's
@@ -47,7 +70,7 @@ __device__ __forceinline__ void adagrad_elem(float& w, float& acc, float g, floa
   w -= lr * g / (sqrtf(acc) + eps);
 }
 
-// One touched row of one table takes its update (a13).  MODE: UpdMode (SGD, lazy Adam, Adagrad).  A table with a dense-gradient
+// One touched row of one table takes its update (a13).  MODE: UpdMode (SGD, lazy Adam, Adagrad, Ftrl).  A table with a dense-gradient
 // buffer (hrb_plan_set_dense_grads) receives the gradient sum instead and is stepped by the caller's dense optimiser.
 template <int MODE>
 __device__ __forceinline__ void apply_table_row(const TableDev& t, const hrb_opt_params& opt, float lr_t, int64_t row, int q, float4 g) {
@@ -62,6 +85,18 @@ __device__ __forceinline__ void apply_table_row(const TableDev& t, const hrb_opt
   }
   float4* wp = reinterpret_cast<float4*>(t.w) + off;
   float4 w = *wp;
+  if (MODE == UPD_FTRL) {  // issue the accumulator and linear loads with the weight's
+    float4* ap = reinterpret_cast<float4*>(t.m) + off;
+    float4* lp = reinterpret_cast<float4*>(t.v) + off;
+    float4 a = *ap, l = *lp;
+    const float l2 = opt.l2_scale;
+    g.x = fmaf(l2, w.x, g.x); g.y = fmaf(l2, w.y, g.y); g.z = fmaf(l2, w.z, g.z); g.w = fmaf(l2, w.w, g.w);
+    ftrl_row4(w, a, l, g, opt);
+    *ap = a;
+    *lp = l;
+    *wp = w;
+    return;
+  }
   const float l2 = opt.l2_scale;
   g.x = fmaf(l2, w.x, g.x); g.y = fmaf(l2, w.y, g.y); g.z = fmaf(l2, w.z, g.z); g.w = fmaf(l2, w.w, g.w);
   if (MODE == UPD_SGD) {
@@ -123,7 +158,7 @@ __device__ __forceinline__ void apply_table_rows(const TableDev& t, const hrb_op
     if (ok[i]) {
       w[i] = reinterpret_cast<float4*>(t.w)[off[i]];
       if (MODE != UPD_SGD) m[i] = reinterpret_cast<float4*>(t.m)[off[i]];
-      if (MODE == UPD_ADAM) v[i] = reinterpret_cast<float4*>(t.v)[off[i]];
+      if (MODE == UPD_ADAM || MODE == UPD_FTRL) v[i] = reinterpret_cast<float4*>(t.v)[off[i]];
     }
   }
   const float l2 = opt.l2_scale;
@@ -141,6 +176,11 @@ __device__ __forceinline__ void apply_table_rows(const TableDev& t, const hrb_op
       adagrad_elem(wi.x, ai.x, gi.x, lr, e); adagrad_elem(wi.y, ai.y, gi.y, lr, e);
       adagrad_elem(wi.z, ai.z, gi.z, lr, e); adagrad_elem(wi.w, ai.w, gi.w, lr, e);
       reinterpret_cast<float4*>(t.m)[off[i]] = ai;
+    } else if (MODE == UPD_FTRL) {
+      float4 ai = m[i], li = v[i];
+      ftrl_row4(wi, ai, li, gi, opt);
+      reinterpret_cast<float4*>(t.m)[off[i]] = ai;
+      reinterpret_cast<float4*>(t.v)[off[i]] = li;
     } else {
       float4 mi = m[i], vi = v[i];
       const float b1 = opt.beta1, b2 = opt.beta2, e = opt.eps, lr = lr_t;

@@ -12,7 +12,8 @@ Data layout of one batch in HBM (all fp32, row-major):
   A_i  (B, ld_i)  activations of Dense layer i (ld_i = round-up-4(units_i))
   params          ONE flat buffer: W_0 | b_0 | ... | W_n | b_n | fm_w (D) | fm_w0 (1), every block padded
                   to 4 floats; W_i is (K_i_padded, ld_i) with zero rows/columns at the padding
-  grads / adam m,v  same layout as params (Adagrad: its accumulator in the place of m, no v)
+  grads / adam m,v  same layout as params (Adagrad: its accumulator in the place of m, no v; Ftrl: accumulator in m, linear in v,
+                  and grads ends with one touched flag per row of the dense-updated tables)
 Reference order of the DNN input is kept (dense first, layers/utils.py:70-84); the padding rows of
 W_0 multiply zero columns of X0 and receive zero gradients, so they stay zero.
 """
@@ -52,8 +53,11 @@ class DeepFMEngine:
     they take the same optimiser step as the dense parameters -- exactly Keras' treatment of an IndexedSlices
     gradient (dense moment decay and dense l2_embd).  Every other table gets the touched-rows-only update.
 
-    optimizer: "adam", "sgd" or "adagrad" (Keras Adagrad; accumulators start at `initial_accumulator_value`).  Under
-    Adagrad the touched-rows-only update is exactly Keras' step whenever l2_embd = 0 (DESIGN.md 3).
+    optimizer: "adam", "sgd", "adagrad" (Keras Adagrad; accumulators start at `initial_accumulator_value`) or "ftrl" (Keras Ftrl
+    with Keras' hyperparameter names: learning_rate_power, initial_accumulator_value, l1, l2, l2_shrinkage, beta).  Under
+    Adagrad and Ftrl the touched-rows-only update is exactly Keras' step whenever l2_embd = 0 (DESIGN.md 3).  Under Ftrl a
+    zero-gradient step is not a no-op, so with l2_embd = 0 the dense-updated tables step only the rows the batch gathers
+    (padding id 0 of pooled fields included): `plan.mark_rows` flags them in the tail of the flat gradient buffer.
     """
 
     def __init__(
@@ -75,6 +79,11 @@ class DeepFMEngine:
         dense_table_max_rows: int = 0,
         dense_update_tables: Optional[Sequence[int]] = None,
         initial_accumulator_value: float = 0.1,
+        learning_rate_power: float = -0.5,
+        l1: float = 0.0,
+        l2: float = 0.0,
+        l2_shrinkage: float = 0.0,
+        beta: float = 0.0,
     ):
         if dnn_hidden_units[-1] != 1:  # DeepFM.py:59-60
             raise ValueError("Output size of dnn should be 1")
@@ -84,6 +93,9 @@ class DeepFMEngine:
             raise ValueError("fused engine implements task='binary'")
         if initial_accumulator_value < 0:
             raise ValueError(f"initial_accumulator_value must be non-negative, got {initial_accumulator_value}")
+        if learning_rate_power > 0 or min(l1, l2, l2_shrinkage) < 0:
+            raise ValueError(f"Ftrl needs learning_rate_power <= 0 and non-negative l1 / l2 / l2_shrinkage, got {learning_rate_power}, "
+                             f"{l1}, {l2}, {l2_shrinkage}")
         self.dev = tables[0].device
         self.tables = list(tables)
         self.D = int(tables[0].shape[1])
@@ -95,10 +107,12 @@ class DeepFMEngine:
         self.B = int(batch_size)
         self.act = dnn_activation or "linear"
         self.optimizer = optimizer
-        self.emb_opt = embedding_optimizer or {"adam": "adam_lazy", "adagrad": "adagrad"}.get(optimizer, "sgd")
+        self.emb_opt = embedding_optimizer or {"adam": "adam_lazy", "adagrad": "adagrad", "ftrl": "ftrl"}.get(optimizer, "sgd")
         self.lr, self.l2_embd, self.l2_dnn = float(lr), float(l2_embd), float(l2_dnn)
         self.beta1, self.beta2, self.eps = 0.9, 0.999, 1e-7  # Keras Adam defaults (eps: also Keras Adagrad's)
         self.initial_accumulator_value = float(initial_accumulator_value)
+        self.lr_power, self.l1, self.l2_shrinkage, self.beta = float(learning_rate_power), float(l1), float(l2_shrinkage), float(beta)
+        self.ftrl_l2 = float(l2) + self.beta / (2.0 * self.lr)  # the l2 Keras hands its Ftrl kernel
         self.gemm_mode = gemm_mode
         self.step_count = 0
 
@@ -135,17 +149,27 @@ class DeepFMEngine:
         self._segments.append((self.fm_off, off - self.fm_off, False))
         self.n_dense_params = off
         self._table_off = {}
-        for t in self.dense_tables:  # dense-updated tables live behind the dense parameters, rows on 128-byte lines like any table
-            off = (off + 31) // 32 * 32
+        # dense-updated tables live behind the dense parameters, rows on 128-byte lines like any table (under Ftrl also on a
+        # multiple of D floats, so that the whole table block is rows of D floats for the touched flags)
+        align = 32 if optimizer != "ftrl" else 32 * self.D // math.gcd(32, self.D)
+        for t in self.dense_tables:
+            off = (off + align - 1) // align * align
             self._table_off[t] = off
             off += self.tables[t].numel()
         self.n_params = off
+        self.tab0 = min(self._table_off.values()) if self._table_off else off  # first float of the table block
+        # Ftrl: one touched flag per D floats of the table block at the tail of the gradient buffer, then the sharded engine's
+        # padding flags (zeroed with the table gradients, all-reduced with them by the sharded engine)
+        n_touched = (off - self.tab0) // self.D if optimizer == "ftrl" else 0
         self.params = torch.zeros(off, device=self.dev, dtype=torch.float32)
-        self.grads = torch.zeros(off, device=self.dev, dtype=torch.float32)
+        self.grads = torch.zeros(off + n_touched + self._n_pad_flags, device=self.dev, dtype=torch.float32)
+        self.touched = self.grads[off : off + n_touched] if n_touched else None
         self.opt_m = torch.zeros(off, device=self.dev, dtype=torch.float32) if optimizer == "adam" else None
         self.opt_v = torch.zeros(off, device=self.dev, dtype=torch.float32) if optimizer == "adam" else None
-        if optimizer == "adagrad":  # opt_m is the accumulator
+        if optimizer in ("adagrad", "ftrl"):  # opt_m is the accumulator (Ftrl: opt_v the linear slot)
             self.opt_m = torch.full((off,), self.initial_accumulator_value, device=self.dev, dtype=torch.float32)
+        if optimizer == "ftrl":
+            self.opt_v = torch.zeros(off, device=self.dev, dtype=torch.float32)
         self.W, self.b, self.dW, self.db = [], [], [], []
         for (wo, bo), Kp, ld in zip(offs, self.layer_K, self.layer_ld):
             self.W.append(self.params[wo : wo + Kp * ld].view(Kp, ld))
@@ -164,13 +188,20 @@ class DeepFMEngine:
             self.tables[t] = live
             table_grads[t] = self.grads[o : o + n].view_as(live)
         self.table_grads = table_grads
-        self.adam_m = self.adam_v = self.accum = None
+        self.adam_m = self.adam_v = self.accum = self.linear = None
         if self.emb_opt == "adam_lazy":
             self.adam_m = [None if t in self._table_off else torch.zeros_like(w) for t, w in enumerate(self.tables)]
             self.adam_v = [None if t in self._table_off else torch.zeros_like(w) for t, w in enumerate(self.tables)]
-        elif self.emb_opt == "adagrad":
+        elif self.emb_opt in ("adagrad", "ftrl"):
             self.accum = [None if t in self._table_off else torch.full_like(w, self.initial_accumulator_value) for t, w in enumerate(self.tables)]
-        self.plan = K.LookupPlan(self.tables, plan_fields, self.adam_m, self.adam_v, accum=self.accum)
+        if self.emb_opt == "ftrl":
+            self.linear = [None if t in self._table_off else torch.zeros_like(w) for t, w in enumerate(self.tables)]
+        self.plan = K.LookupPlan(self.tables, plan_fields, self.adam_m, self.adam_v, accum=self.accum, linear=self.linear)
+        self.table_touched: List[Optional[torch.Tensor]] = [None] * len(self.tables)  # Ftrl: touched flags of the dense-updated tables
+        if self.touched is not None:
+            for t, o in self._table_off.items():
+                r0 = (o - self.tab0) // self.D
+                self.table_touched[t] = self.touched[r0 : r0 + self.tables[t].shape[0]]
         if self.dense_tables:
             self.plan.set_dense_grads(table_grads)
 
@@ -200,6 +231,8 @@ class DeepFMEngine:
         self.label_dev = torch.zeros(B, **f32)
         self.loss_host = torch.zeros(1, dtype=torch.float32).pin_memory()
         self._ws_emb = torch.empty(self.plan.workspace_bytes(B), device=self.dev, dtype=torch.uint8)
+
+    _n_pad_flags = 0  # floats the sharded engine keeps behind the touched flags
 
     # ------------------------------------------------------------------------------------------
     _marks = None  # when a list: (phase name, cuda event) recorded after every phase of a step
@@ -331,8 +364,14 @@ class DeepFMEngine:
         self._mark("lookup_fm_fwd")
 
     def _zero_table_grads(self) -> None:
-        if self.n_params > self.n_dense_params:
+        if self.grads.numel() > self.n_dense_params:
             self.grads[self.n_dense_params :].zero_()
+
+    def _mark_touched(self, plan, ids, tables) -> None:
+        """Ftrl with l2_embd = 0: flag the rows of the dense-updated tables among `tables` (the plan's tables, in order) that the
+        batch gathers; the flat step then steps those rows only (with l2_embd > 0 Keras' table gradient is dense: every row steps)."""
+        if self.touched is not None and self.l2_embd == 0.0:
+            plan.mark_rows(ids, [self.table_touched[t] for t in tables])
 
     # The library has two implementations of the embedding backward (hrb200.h: hrb_bwd_algo); which one is faster depends on the
     # id distribution (spread ids: UNITS, a few very hot rows: SORT).  The engine times both on the caller's own data during
@@ -343,6 +382,7 @@ class DeepFMEngine:
 
     def _embedding_backward(self, ids, B, st, op) -> None:
         self._zero_table_grads()
+        self._mark_touched(self.plan, ids, range(len(self.tables)))
         trial = None
         n_trials = len(self._bwd_trials or [])
         if self.autotune_embedding_bwd and self._marks is None and B == self.B and self.step_count >= 3 and n_trials < 4 and self.bwd_algo == "auto":
@@ -401,9 +441,11 @@ class DeepFMEngine:
         dz, lddz = self.dZ[-1], self.layer_ld[-1]
         tc_step = self.use_tc and B == self.B
         op = _lib.OptParams()
-        op.opt = {"sgd": _lib.OPT_SGD, "adagrad": _lib.OPT_ADAGRAD}.get(self.emb_opt, _lib.OPT_ADAM_LAZY)
+        op.opt = {"sgd": _lib.OPT_SGD, "adagrad": _lib.OPT_ADAGRAD, "ftrl": _lib.OPT_FTRL}.get(self.emb_opt, _lib.OPT_ADAM_LAZY)
         op.lr, op.beta1, op.beta2, op.eps, op.l2_scale = self.lr, self.beta1, self.beta2, self.eps, 2.0 * self.l2_embd
         op.bias_corr1, op.bias_corr2 = 1.0 - self.beta1 ** self.step_count, 1.0 - self.beta2 ** self.step_count
+        op.l1, op.l2, op.lr_power, op.l2_shrinkage = self.l1, self.ftrl_l2, self.lr_power, self.l2_shrinkage
+        self._op = op
         emb_done = [False]
 
         def bwd_x_0(dz0, lddz0) -> None:
@@ -495,7 +537,8 @@ class DeepFMEngine:
         self._sync_dense_grads()
         # dense parameters
         segs = [(o_, n_, 2.0 * self.l2_dnn if reg else 0.0) for o_, n_, reg in self._segments]
-        if self.n_params > self.n_dense_params:  # dense-updated tables: Keras adds d(l2_embd*sum w^2) for every row (group.py:289)
+        ftrl_rows = self.optimizer == "ftrl" and self.touched is not None and self.l2_embd == 0.0
+        if self.n_params > self.n_dense_params and not ftrl_rows:  # dense-updated tables: Keras adds d(l2_embd*sum w^2) for every row (group.py:289)
             segs.append((self.n_dense_params, self.n_params - self.n_dense_params, 2.0 * self.l2_embd))
         merged = [segs[0]]
         for o_, n_, l2_ in segs[1:]:  # neighbouring segments with the same regulariser take one launch
@@ -512,8 +555,16 @@ class DeepFMEngine:
                      self.beta2, self.eps, op.bias_corr1, op.bias_corr2, l2s, st)
             elif self.optimizer == "adagrad":
                 call("hrb_adagrad_step", pp(self.params), pp(self.grads), pp(self.opt_m), length, self.lr, self.eps, l2s, st)
+            elif self.optimizer == "ftrl":
+                call("hrb_ftrl_step", pp(self.params), pp(self.grads), pp(self.opt_m), pp(self.opt_v), length, self.lr, self.l1, self.ftrl_l2,
+                     self.lr_power, self.l2_shrinkage, l2s, None, 0, st)
             else:
                 call("hrb_sgd_step", pp(self.params), pp(self.grads), length, self.lr, l2s, st)
+        if ftrl_rows:  # the table block: only the rows the batch gathered (IndexedSlices) step
+            o = self.tab0 * 4
+            pp = lambda t: ctypes.c_void_p(t.data_ptr() + o)
+            call("hrb_ftrl_step", pp(self.params), pp(self.grads), pp(self.opt_m), pp(self.opt_v), self.n_params - self.tab0, self.lr, self.l1,
+                 self.ftrl_l2, self.lr_power, self.l2_shrinkage, 0.0, K._p(self.touched), self.D, st)
         self._refresh_wt()
         if self._side_pending:  # the next step's lookup must see the updated rows
             torch.cuda.current_stream().wait_stream(self._side)

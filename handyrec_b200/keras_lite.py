@@ -375,6 +375,59 @@ class Adagrad:
                              [2.0 * l2 for _, l2 in live], self.lr, self.eps)  # all variables in one launch
 
 
+class Ftrl:
+    """tf.keras.optimizers.Ftrl (Keras 2.6, FTRL-Proximal): per element, with g the gradient (plus 2*l2*w of a Keras regulariser)
+    and p(a) = a^(-learning_rate_power),
+
+        linear += g + 2*l2_shrinkage*w - (p(acc + g^2) - p(acc)) / lr * w;  acc += g^2
+        w = |linear| > l1 ? (sign(linear)*l1 - linear) / (p(acc) / lr + 2*l2') : 0,   l2' = l2 + beta / (2*lr)
+
+    acc starting at initial_accumulator_value, linear at 0.  A step with a zero gradient is not a no-op (it recomputes w from the
+    slots), so embedding tables step only the rows a batch gathers, as Keras does for their IndexedSlices gradient
+    (CustomEmbedding.apply_sparse)."""
+
+    def __init__(self, learning_rate=0.001, learning_rate_power=-0.5, initial_accumulator_value=0.1, l1_regularization_strength=0.0,
+                 l2_regularization_strength=0.0, name="Ftrl", l2_shrinkage_regularization_strength=0.0, beta=0.0, lr=None):
+        if initial_accumulator_value < 0.0:
+            raise ValueError(f"initial_accumulator_value {initial_accumulator_value} needs to be positive or zero")
+        if learning_rate_power > 0.0:
+            raise ValueError(f"learning_rate_power {learning_rate_power} needs to be negative or zero")
+        if l1_regularization_strength < 0.0:
+            raise ValueError(f"l1_regularization_strength {l1_regularization_strength} needs to be positive or zero")
+        if l2_regularization_strength < 0.0:
+            raise ValueError(f"l2_regularization_strength {l2_regularization_strength} needs to be positive or zero")
+        if l2_shrinkage_regularization_strength < 0.0:
+            raise ValueError(f"l2_shrinkage_regularization_strength {l2_shrinkage_regularization_strength} needs to be positive or zero")
+        self.lr = float(lr if lr is not None else learning_rate)
+        self.name = name
+        self.learning_rate_power = float(learning_rate_power)
+        self.initial_accumulator_value = float(initial_accumulator_value)
+        self.l1 = float(l1_regularization_strength)
+        self.l2 = float(l2_regularization_strength)
+        self.l2_shrinkage = float(l2_shrinkage_regularization_strength)
+        self.beta = float(beta)
+        self.state: Dict[int, Tuple[torch.Tensor, torch.Tensor]] = {}
+
+    @property
+    def kernel_l2(self) -> float:
+        """The l2 the TF kernel takes: l2_regularization_strength + beta / (2 * learning_rate)."""
+        return self.l2 + self.beta / (2.0 * self.lr)
+
+    def hyper(self) -> Dict[str, float]:
+        """Keyword arguments of the library's Ftrl entry points."""
+        return dict(l1=self.l1, l2=self.kernel_l2, lr_power=self.learning_rate_power, l2_shrinkage=self.l2_shrinkage)
+
+    def step(self, params_l2: Sequence[Tuple[torch.nn.Parameter, float]]):
+        from . import kernels as K
+
+        live = [(p, l2) for p, l2 in params_l2 if p.grad is not None and p.requires_grad]
+        for p, _ in live:
+            if id(p) not in self.state:
+                self.state[id(p)] = (torch.full_like(p.data, self.initial_accumulator_value), torch.zeros_like(p.data))
+        K.ftrl_step_multi([p.data for p, _ in live], [p.grad.contiguous() for p, _ in live], [self.state[id(p)][0] for p, _ in live],
+                          [self.state[id(p)][1] for p, _ in live], [2.0 * l2 for _, l2 in live], self.lr, **self.hyper())
+
+
 class SGD:
     def __init__(self, learning_rate=0.01, lr=None):
         self.lr = float(lr if lr is not None else learning_rate)
@@ -540,7 +593,10 @@ class Model:
             from .sharded import TorchDistComm
 
             self._comm = distribute if not isinstance(distribute, bool) else TorchDistComm()
-        if self.fuse and self.loss is binary_crossentropy and isinstance(self.optimizer, (Adam, SGD, Adagrad)):
+        for l in self._all_layers():  # under Ftrl a dense step would move the rows a batch does not gather
+            if hasattr(l, "SPARSE_UPDATE_MIN_ROWS"):
+                l._ftrl = isinstance(self.optimizer, Ftrl)
+        if self.fuse and self.loss is binary_crossentropy and isinstance(self.optimizer, (Adam, SGD, Adagrad, Ftrl)):
             from .lowering import lower  # a DeepFM-shaped graph runs on the fused engine (one lookup, tcgen05 towers)
 
             self._fused = lower(self)

@@ -18,7 +18,7 @@ __all__ = [
     "init_uniform", "embedding_fwd", "embedding_bwd_dense", "seq_pool_fwd", "seq_pool_bwd", "LookupPlan",
     "fm_fwd", "fm_bwd", "dense_fwd", "dense_bwd_x", "dense_bwd_w", "act_bwd", "dice_fwd", "dice_bwd",
     "lau_fwd", "lau_pack_params", "sigmoid_bce", "adam_step", "sgd_step", "adam_step_multi", "sgd_step_multi",
-    "adagrad_step", "adagrad_step_multi",
+    "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi",
 ]
 
 
@@ -158,17 +158,21 @@ def seq_pool_bwd(x: torch.Tensor, mask: torch.Tensor, dout: torch.Tensor, method
 class LookupPlan:
     """Device plan of one feature group: tables + (table, seq_len, pool, ids_col, out_col) per field.
 
-    Optimiser state per table (None entries for tables without): `adam_m` / `adam_v` for lazy Adam, or `accum` for Adagrad
-    (it takes the ABI's adam_m slot, so the two cannot be given together)."""
+    Optimiser state per table (None entries for tables without): `adam_m` / `adam_v` for lazy Adam, `accum` for Adagrad, or
+    `accum` and `linear` for Ftrl (they take the ABI's adam_m / adam_v slots, so they cannot be given with the Adam moments)."""
 
     def __init__(self, tables: Sequence[torch.Tensor], fields: Sequence[Tuple[int, int, str, int, int]],
                  adam_m: Optional[Sequence[torch.Tensor]] = None, adam_v: Optional[Sequence[torch.Tensor]] = None,
-                 accum: Optional[Sequence[torch.Tensor]] = None):
+                 accum: Optional[Sequence[torch.Tensor]] = None, linear: Optional[Sequence[torch.Tensor]] = None):
         self.tables = [_chk(t, torch.float32, "table") for t in tables]
         if accum is not None:
             if adam_m is not None:
-                raise ValueError("LookupPlan: pass either adam_m (Adam) or accum (Adagrad), not both")
+                raise ValueError("LookupPlan: pass either adam_m (Adam) or accum (Adagrad / Ftrl), not both")
             adam_m = accum
+        if linear is not None:
+            if adam_v is not None:
+                raise ValueError("LookupPlan: pass either adam_v (Adam) or linear (Ftrl), not both")
+            adam_v = linear
         self.adam_m = list(adam_m) if adam_m is not None else None
         self.adam_v = list(adam_v) if adam_v is not None else None
         self.fields = [tuple(f) for f in fields]
@@ -200,6 +204,27 @@ class LookupPlan:
         self._dense_grads = list(grads)  # keep the buffers alive
         arr = (ctypes.c_void_p * len(grads))(*[(g.data_ptr() if g is not None else None) for g in grads])
         call("hrb_plan_set_dense_grads", self._h, arr)
+
+    def mark_rows(self, ids: torch.Tensor, touched: Sequence[Optional[torch.Tensor]]) -> None:
+        """touched[t] (rows,) fp32 or None: store 1.0 at every row of table t that the batch names (every in-range id of a plain
+        field, every position of a pooled field, padding id 0 included) -- the rows Keras' IndexedSlices gradient lists."""
+        assert len(touched) == len(self.tables)
+        ids_ld = self._ids_ld(ids)
+        for t in touched:
+            if t is not None:
+                _chk(t, torch.float32, "touched")
+        arr = (ctypes.c_void_p * len(touched))(*[(t.data_ptr() if t is not None else None) for t in touched])
+        call("hrb_plan_mark_rows", self._h, _p(ids), ids_ld, ids.shape[0], arr, _stream())
+
+    def pad_flags(self, ids: torch.Tensor, flags: torch.Tensor) -> None:
+        """flags (2 * n_tables,) fp32, caller-zeroed: flags[2t] = 1 where a pooled field of table t holds padding, flags[2t+1] = 1
+        where a valid position names row 0 of table t (hrb_plan_pad_flags)."""
+        _chk(flags, torch.float32, "flags")
+        call("hrb_plan_pad_flags", self._h, _p(ids), self._ids_ld(ids), ids.shape[0], _p(flags), _stream())
+
+    def ftrl_pad_step(self, flags: torch.Tensor, op: OptParams) -> None:
+        """Row 0 of every row-updated table whose flags show padding and no valid id 0 takes its zero-gradient Ftrl step."""
+        call("hrb_plan_ftrl_pad_step", self._h, _p(flags), ctypes.byref(op), _stream())
 
     def __del__(self):
         try:  # module globals may already be gone at interpreter shutdown
@@ -245,10 +270,12 @@ class LookupPlan:
 
     def backward_update(self, ids: torch.Tensor, dout: torch.Tensor, opt: str = "sgd", lr: float = 0.01, l2_scale: float = 0.0,
                         beta1: float = 0.9, beta2: float = 0.999, eps: float = 1e-7, step: int = 1,
-                        workspace: Optional[torch.Tensor] = None, autotune: bool = False) -> None:
+                        workspace: Optional[torch.Tensor] = None, autotune: bool = False, l1: float = 0.0, l2: float = 0.0,
+                        lr_power: float = -0.5, l2_shrinkage: float = 0.0) -> None:
         """Segment-reduce the gradient rows per table row and update the touched rows of every table in place.
 
-        opt: "sgd", "adam" (lazy Adam: beta1, beta2, eps, step) or "adagrad" (eps; the plan's `accum`)."""
+        opt: "sgd", "adam" (lazy Adam: beta1, beta2, eps, step), "adagrad" (eps; the plan's `accum`) or "ftrl" (l1, l2 with
+        Keras' beta / (2*lr) added, lr_power, l2_shrinkage; the plan's `accum` and `linear`)."""
         B = ids.shape[0]
         ids_ld = self._ids_ld(ids)
         dout_ld = _row_major_2d(_chk(dout, torch.float32, "dout", contiguous=False), "dout")
@@ -258,9 +285,10 @@ class LookupPlan:
                 self._ws = torch.empty(need, device=self.device, dtype=torch.uint8)
             workspace = self._ws
         op = OptParams()
-        op.opt = _lib.OPT_SGD if opt == "sgd" else _lib.OPT_ADAGRAD if opt == "adagrad" else _lib.OPT_ADAM_LAZY
+        op.opt = {"sgd": _lib.OPT_SGD, "adagrad": _lib.OPT_ADAGRAD, "ftrl": _lib.OPT_FTRL}.get(opt, _lib.OPT_ADAM_LAZY)
         op.lr, op.beta1, op.beta2, op.eps, op.l2_scale = lr, beta1, beta2, eps, l2_scale
         op.bias_corr1, op.bias_corr2 = 1.0 - beta1 ** step, 1.0 - beta2 ** step
+        op.l1, op.l2, op.lr_power, op.l2_shrinkage = l1, l2, lr_power, l2_shrinkage
         trial = self._next_bwd_trial(B) if autotune else None
         if trial is not None:
             call("hrb_plan_set_bwd_algo", self._h, _lib.BWD_UNITS if trial == "units" else _lib.BWD_SORT)
@@ -453,6 +481,15 @@ def adagrad_step(param, grad, acc, lr, eps=1e-7, l2_scale=0.0):
     call("hrb_adagrad_step", _p(param), _p(grad), _p(acc), param.numel(), lr, eps, l2_scale, _stream())
 
 
+def ftrl_step(param, grad, acc, lin, lr, l1=0.0, l2=0.0, lr_power=-0.5, l2_shrinkage=0.0, l2_scale=0.0, row_touched=None, dim=0):
+    """Keras Ftrl over every element (l2 with beta / (2*lr) added); with row_touched (one float per row of `dim` elements) the
+    rows flagged 0 keep their bits."""
+    if row_touched is not None:
+        _chk(row_touched, torch.float32, "row_touched")
+    call("hrb_ftrl_step", _p(param), _p(grad), _p(acc), _p(lin), param.numel(), lr, l1, l2, lr_power, l2_shrinkage, l2_scale,
+         _p(row_touched), dim, _stream())
+
+
 def _ptr_array(tensors):
     return (ctypes.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors])
 
@@ -488,6 +525,18 @@ def adagrad_step_multi(params, grads, accs, l2_scales, lr, eps=1e-7):
         _chk(t, torch.float32, "tensor")
     call("hrb_adagrad_step_multi", n, _ptr_array(params), _ptr_array(grads), _ptr_array(accs),
          (ctypes.c_int64 * n)(*[p.numel() for p in params]), (ctypes.c_float * n)(*l2_scales), lr, eps, _stream())
+
+
+def ftrl_step_multi(params, grads, accs, lins, l2_scales, lr, l1=0.0, l2=0.0, lr_power=-0.5, l2_shrinkage=0.0):
+    """hrb_ftrl_step for a list of tensors in one launch (per HRB_MULTI_MAX tensors), every element stepping."""
+    n = len(params)
+    if n == 0:
+        return
+    for t in list(params) + list(grads) + list(accs) + list(lins):
+        _chk(t, torch.float32, "tensor")
+    call("hrb_ftrl_step_multi", n, _ptr_array(params), _ptr_array(grads), _ptr_array(accs), _ptr_array(lins),
+         (ctypes.c_int64 * n)(*[p.numel() for p in params]), (ctypes.c_float * n)(*l2_scales), lr, l1, l2, lr_power, l2_shrinkage,
+         _stream())
 
 
 # --------------------------------------------------------------------------------------------

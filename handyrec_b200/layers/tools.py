@@ -75,8 +75,11 @@ class CustomEmbedding(Layer):
 
     # Tables with at least this many rows keep their gradient sparse (TF: IndexedSlices) and take the touched-rows-only update
     # (lazy Adam: a declared deviation from Keras' dense Adam step, DESIGN.md 3; Adagrad: Keras' own sparse step, exact while
-    # l2 = 0); smaller ones get the dense Keras-exact step.
+    # l2 = 0); smaller ones get the dense Keras-exact step.  Under Ftrl a table with l2 = 0 takes the touched-rows update at
+    # every size: Keras steps only the rows its IndexedSlices gradient lists, and an Ftrl step with a zero gradient is not a
+    # no-op, so the dense step would move every other row.
     SPARSE_UPDATE_MIN_ROWS = 131072
+    _ftrl = False  # set by Model.compile
 
     _sharded = None  # (rank, n_ranks, full rows) when `embeddings` is this rank's row shard
 
@@ -86,7 +89,10 @@ class CustomEmbedding(Layer):
                                "(a DeepFM-shaped model compiled under ShardedTables / distribute=True) reads it")
         ids = inputs.to(torch.int32)
         sink = None
-        if self.trainable and self.input_dim >= self.SPARSE_UPDATE_MIN_ROWS and torch.is_grad_enabled() and self.output_dim % 4 == 0:
+        rows_only = self.input_dim >= self.SPARSE_UPDATE_MIN_ROWS or (self._ftrl and not self.l2)
+        if self._ftrl and not self.l2 and self.output_dim % 4 != 0 and self.trainable and torch.is_grad_enabled():
+            raise ValueError(f"{self.name}: the touched-rows Ftrl update needs output_dim % 4 == 0, got {self.output_dim}")
+        if self.trainable and rows_only and torch.is_grad_enabled() and self.output_dim % 4 == 0:
             if not hasattr(self, "_sparse_grads"):
                 self._sparse_grads = []
             sink = self._sparse_grads
@@ -102,23 +108,26 @@ class CustomEmbedding(Layer):
         if not pending:
             return
         from .. import kernels as K
-        from ..keras_lite import Adagrad, Adam
+        from ..keras_lite import Adagrad, Adam, Ftrl
 
         ids = torch.cat([i for i, _ in pending]).reshape(-1, 1).contiguous()
         rows = torch.cat([g for _, g in pending]).contiguous()
         pending.clear()
-        adam, adagrad = isinstance(optimizer, Adam), isinstance(optimizer, Adagrad)
+        adam, adagrad, ftrl = isinstance(optimizer, Adam), isinstance(optimizer, Adagrad), isinstance(optimizer, Ftrl)
         if getattr(self, "_plan", None) is None:
             w = self.embeddings.data
             self._m, self._v = (torch.zeros_like(w), torch.zeros_like(w)) if adam else (None, None)
-            self._accum = torch.full_like(w, optimizer.initial_accumulator_value) if adagrad else None
+            self._accum = torch.full_like(w, optimizer.initial_accumulator_value) if (adagrad or ftrl) else None
+            self._linear = torch.zeros_like(w) if ftrl else None
             self._plan = K.LookupPlan([w], [(0, 1, "none", 0, 0)], [self._m] if adam else None, [self._v] if adam else None,
-                                      accum=[self._accum] if adagrad else None)
+                                      accum=[self._accum] if (adagrad or ftrl) else None, linear=[self._linear] if ftrl else None)
         if adam:
             self._plan.backward_update(ids, rows, opt="adam", lr=optimizer.lr, l2_scale=2.0 * self.l2, beta1=optimizer.b1, beta2=optimizer.b2,
                                        eps=optimizer.eps, step=max(optimizer.t, 1), autotune=True)
         elif adagrad:
             self._plan.backward_update(ids, rows, opt="adagrad", lr=optimizer.lr, l2_scale=2.0 * self.l2, eps=optimizer.eps, autotune=True)
+        elif ftrl:  # every gathered id is a plain-field position here: row 0 of mask_zero padding steps like any other row
+            self._plan.backward_update(ids, rows, opt="ftrl", lr=optimizer.lr, l2_scale=2.0 * self.l2, autotune=True, **optimizer.hyper())
         else:
             self._plan.backward_update(ids, rows, opt="sgd", lr=optimizer.lr, l2_scale=2.0 * self.l2, autotune=True)
 

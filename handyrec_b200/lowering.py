@@ -235,17 +235,23 @@ class FusedDeepFM:
 
     def build(self, batch_size: int, optimizer) -> None:
         from .engine import DeepFMEngine
-        from .keras_lite import Adagrad, Adam, SGD
+        from .keras_lite import Adagrad, Adam, Ftrl, SGD
 
+        key = None
         if isinstance(optimizer, Adam):
             opt, lr = "adam", optimizer.lr
         elif isinstance(optimizer, SGD):
             opt, lr = "sgd", optimizer.lr
         elif isinstance(optimizer, Adagrad):
             opt, lr = "adagrad", optimizer.lr
+        elif isinstance(optimizer, Ftrl):
+            opt, lr = "ftrl", optimizer.lr
+            key = (opt, lr, optimizer.learning_rate_power, optimizer.initial_accumulator_value, optimizer.l1, optimizer.l2,
+                   optimizer.l2_shrinkage, optimizer.beta)
         else:
-            raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD or keras_lite.Adagrad")
-        if self.engine is not None and self.engine.B >= batch_size and self._opt_key == (opt, lr):
+            raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD, keras_lite.Adagrad or keras_lite.Ftrl")
+        key = key or (opt, lr)
+        if self.engine is not None and self.engine.B >= batch_size and self._opt_key == key:
             return
         self.sync_to_layers()
         dev = torch.device("cuda", torch.cuda.current_device())
@@ -254,8 +260,11 @@ class FusedDeepFM:
         small = getattr(self.model, "dense_table_max_rows", 131072)
         common = dict(dnn_hidden_units=tuple(dnn.hidden_units), dnn_activation=dnn.activation or "linear", batch_size=batch_size, optimizer=opt,
                       lr=lr, l2_embd=self.spec.fields[0].emb.l2, l2_dnn=float(dnn.l2_reg or 0.0), seed=dnn.seed)
-        if opt == "adagrad":  # the engine fills its accumulators when it is built
+        if opt in ("adagrad", "ftrl"):  # the engine fills its accumulators when it is built
             common["initial_accumulator_value"] = optimizer.initial_accumulator_value
+        if opt == "ftrl":
+            common.update(l1=optimizer.l1, l2=optimizer.l2, learning_rate_power=optimizer.learning_rate_power,
+                          l2_shrinkage=optimizer.l2_shrinkage, beta=optimizer.beta)
         comm = getattr(self.model, "_comm", None)
         if comm is not None and comm.N > 1:
             eng = self._build_sharded(comm, dev, fields, small, common)
@@ -273,7 +282,7 @@ class FusedDeepFM:
         eng.step_count = getattr(optimizer, "t", 0)
         for t, lay in enumerate(self.tables):  # the layer and the engine share ONE copy of every table
             lay.embeddings.data = eng.tables[t]
-        self.engine, self._opt_key = eng, (opt, lr)
+        self.engine, self._opt_key = eng, key
         self._slots = []
 
     def _build_sharded(self, comm, dev, fields, small: int, common: dict):

@@ -325,6 +325,9 @@ class ShardedDeepFMEngine(DeepFMEngine):
         if replicated is None:
             replicated = [t for t, v in enumerate(vocabs) if v <= replicate_max_rows]
         self.replicated = sorted(set(int(t) for t in replicated))
+        n_sharded = len(tables) - len(self.replicated)
+        pooled = any(pool not in (None, "none") for ti, L, pool in fields if ti not in self.replicated)
+        self._n_pad_flags = 2 * n_sharded if kw.get("optimizer") == "ftrl" and pooled else 0
         for t in self.replicated:
             if tables[t].shape[0] != vocabs[t]:
                 raise ValueError(f"replicated table {t} must be a full copy ({vocabs[t]} rows), got {tables[t].shape[0]}")
@@ -343,7 +346,8 @@ class ShardedDeepFMEngine(DeepFMEngine):
             m = [self.adam_m[t] for t in tabs] if (with_moments and self.adam_m is not None) else None
             v = [self.adam_v[t] for t in tabs] if (with_moments and self.adam_v is not None) else None
             acc = [self.accum[t] for t in tabs] if (with_moments and self.accum is not None) else None
-            return K.LookupPlan([self.tables[t] for t in tabs], flds, m, v, accum=acc)
+            lin = [self.linear[t] for t in tabs] if (with_moments and self.linear is not None) else None
+            return K.LookupPlan([self.tables[t] for t in tabs], flds, m, v, accum=acc, linear=lin)
 
         if self.replicated:
             self.plan_shard = sub_plan(self.sharded, True)
@@ -353,6 +357,10 @@ class ShardedDeepFMEngine(DeepFMEngine):
                 self._ws_rep = torch.empty(self.plan_rep.workspace_bytes(self.B), device=self.dev, dtype=torch.uint8)
         else:
             self.plan_shard, self.plan_rep = self.plan, None
+        # Ftrl: padding positions of pooled fields name row 0, which the row exchange does not route.  Every rank flags, per
+        # row-sharded table, padding seen / a valid id 0 seen in the tail of the flat gradient buffer (after the touched flags);
+        # the gradient all-reduce sums them and the owner of row 0 (rank 0) gives row 0 its zero-gradient step where needed.
+        self._pad_flags = self.grads[-self._n_pad_flags :] if self._n_pad_flags else None
         self.exchange = None
         if self.plan_shard is not None:
             self.provider = CudaShardProvider(self.plan_shard, [vocabs[t] for t in self.sharded], comm.N, self.B)
@@ -431,8 +439,16 @@ class ShardedDeepFMEngine(DeepFMEngine):
                 self._side2.wait_stream(cur)
                 with torch.cuda.stream(self._side2):
                     self._finish_sharded(op)
+        if self.plan_rep is None and self._pad_flags is not None:
+            self._zero_table_grads()
+            self.plan_shard.pad_flags(ids, self._pad_flags)
+            self._rep_done = torch.cuda.Event()  # the gradient all-reduce carries the flags
+            self._rep_done.record()
         if self.plan_rep is not None:  # replicated tables: local reduction into the flat gradient buffer
             self._zero_table_grads()
+            self._mark_touched(self.plan_rep, ids, self.replicated)
+            if self._pad_flags is not None:
+                self.plan_shard.pad_flags(ids, self._pad_flags)
             call("hrb_lookup_bwd_update", self.plan_rep._h, K._p(ids), ids.stride(0), B, K._p(self.dX0), self.K0p, None, ctypes.byref(op),
                  K._p(self._ws_rep), self._ws_rep.numel(), K._stream())
             self._rep_done = torch.cuda.Event()
@@ -461,3 +477,5 @@ class ShardedDeepFMEngine(DeepFMEngine):
             self._rep_done = None
         getattr(self.comm, "all_reduce_dense", self.comm.all_reduce_sum)(self.grads)
         self._mark("dense_allreduce")
+        if self._pad_flags is not None and self.comm.rank == 0:  # local row 0 of rank 0's shards is row 0 of every sharded table
+            self.plan_shard.ftrl_pad_step(self._pad_flags, self._op)

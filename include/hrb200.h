@@ -102,8 +102,8 @@ int hrb_seq_pool_bwd(const float* x, const uint8_t* mask, const float* dout, int
  * ------------------------------------------------------------------------------------------ */
 typedef struct hrb_table_desc {
   float* weight;  /* (rows, dim) fp32, 16-byte aligned                        */
-  float* adam_m;  /* optimiser state: Adam m / Adagrad accumulator (same shape) or NULL */
-  float* adam_v;  /* Adam second moment (same shape) or NULL; NULL under Adagrad     */
+  float* adam_m;  /* optimiser state: Adam m / Adagrad or Ftrl accumulator (same shape) or NULL */
+  float* adam_v;  /* Adam second moment / Ftrl linear (same shape) or NULL; NULL under Adagrad */
   int64_t rows;   /* vocab_size                                               */
   int32_t dim;    /* embedding dim                                            */
   int32_t pad_;
@@ -144,12 +144,22 @@ int hrb_lookup_fm_fwd(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, 
  *   opt = HRB_OPT_ADAM_LAZY: Adam moments/weights updated for touched rows only (needs adam_m/adam_v)
  *   opt = HRB_OPT_ADAGRAD:   g' = g[r] + l2_scale*w[r]; acc[r] += g'^2; w[r] -= lr * g' / (sqrt(acc[r]) + eps)
  *                            (touched rows only, acc in adam_m; Keras ResourceSparseApplyAdagradV2 on the summed rows)
+ *   opt = HRB_OPT_FTRL:      Keras Ftrl (ResourceSparseApplyFtrl / V2) on the summed rows, accum in adam_m, linear in adam_v:
+ *                            g' = g[r] + l2_scale*w[r]; gs = g' + 2*l2_shrinkage*w[r]; acc' = acc + g'^2;
+ *                            linear += gs - (p(acc') - p(acc)) / lr * w[r], p(a) = a^(-lr_power);
+ *                            w[r] = |linear| > l1 ? (sign(linear)*l1 - linear) / (p(acc') / lr + 2*l2) : 0; acc = acc'.
+ *                            Touched rows: every in-range id of a plain field and every position of a pooled field -- the
+ *                            padding id 0 included, with a zero gradient (Keras gathers row 0 there): when a batch holds
+ *                            padding for a row-updated table, row 0 of that table takes exactly one step.
  *   max-pooled fields are not supported here (use a6 bwd + hrb_embedding_bwd_dense). */
-typedef enum hrb_opt { HRB_OPT_SGD = 0, HRB_OPT_ADAM_LAZY = 1, HRB_OPT_ADAGRAD = 2 } hrb_opt;
+typedef enum hrb_opt { HRB_OPT_SGD = 0, HRB_OPT_ADAM_LAZY = 1, HRB_OPT_ADAGRAD = 2, HRB_OPT_FTRL = 3 } hrb_opt;
 typedef struct hrb_opt_params {
   int32_t opt;
   float lr, beta1, beta2, eps, l2_scale; /* l2_scale = 2*l2_embd (features/group.py:289) */
   float bias_corr1, bias_corr2;          /* 1-beta1^t, 1-beta2^t */
+  /* read only when opt == HRB_OPT_FTRL: Keras' l1 / l2 / learning_rate_power / l2_shrinkage strengths, l2 with beta / (2*lr)
+   * already added */
+  float l1, l2, lr_power, l2_shrinkage;
 } hrb_opt_params;
 int hrb_lookup_bwd_workspace(const hrb_plan* plan, int64_t ids_ld, int64_t batch, size_t* bytes);
 int hrb_lookup_bwd_update(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch,
@@ -172,6 +182,21 @@ int hrb_plan_set_bwd_algo(hrb_plan* plan, int32_t algo);
  * exactly what Keras does for an IndexedSlices gradient under Adam (dense moment decay).  NULL keeps the in-place
  * touched-rows update.  The array has n_tables entries. */
 int hrb_plan_set_dense_grads(hrb_plan* plan, float* const* grads_host);
+
+/* Touched rows of a batch, for optimisers whose step with a zero gradient is not a no-op (Ftrl): for every table t with
+ * touched_host[t] != NULL (one float per row, caller-zeroed), store 1.0f at every row a position of the batch names --
+ * every in-range id of a plain field, every position of a pooled field, the padding id 0 included.  Plain stores: every
+ * writer stores the same value.  The array has n_tables entries. */
+int hrb_plan_mark_rows(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, float* const* touched_host,
+                       void* stream);
+/* Row 0 and the padding of pooled fields, for callers that apply the row update themselves (the owner of row 0 of a
+ * row-sharded table): hrb_plan_pad_flags stores 1.0f in flags[2t] when a pooled field of table t holds padding in the batch
+ * and in flags[2t+1] when a valid position names row 0 of table t (2*n_tables floats, caller-zeroed, plain stores; flags of
+ * several batches may be summed).  hrb_plan_ftrl_pad_step then gives row 0 of every row-updated table t with
+ * flags[2t] != 0 and flags[2t+1] == 0 its zero-gradient Ftrl step (opt_host->opt must be HRB_OPT_FTRL).
+ * hrb_lookup_bwd_update does both itself. */
+int hrb_plan_pad_flags(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, float* flags, void* stream);
+int hrb_plan_ftrl_pad_step(const hrb_plan* plan, const float* flags, const hrb_opt_params* opt_host, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * a9  FM.call   (layers/interaction.py:15-39) on a materialised (B,F,D) tensor.
@@ -368,6 +393,12 @@ int hrb_adam_step(float* param, const float* grad, float* m, float* v, int64_t n
                   float beta2, float eps, float bias_corr1, float bias_corr2, float l2_scale, void* stream);
 int hrb_sgd_step(float* param, const float* grad, int64_t n, float lr, float l2_scale, void* stream);
 int hrb_adagrad_step(float* param, const float* grad, float* acc, int64_t n, float lr, float eps, float l2_scale, void* stream);
+/* Keras Ftrl (ResourceApplyFtrl, or V2 when l2_shrinkage > 0) with the arithmetic of HRB_OPT_FTRL above; l2 with beta / (2*lr)
+ * added.  row_touched NULL: every element steps.  Otherwise it holds one float per row of `dim` elements (n % dim == 0) and
+ * the elements of rows whose value is 0 are left bit-identical (param, acc and lin): a dense-updated embedding table steps the
+ * rows its IndexedSlices gradient lists (hrb_plan_mark_rows) and no others. */
+int hrb_ftrl_step(float* param, const float* grad, float* acc, float* lin, int64_t n, float lr, float l1, float l2, float lr_power,
+                  float l2_shrinkage, float l2_scale, const float* row_touched, int32_t dim, void* stream);
 /* The same steps for `count` parameter tensors in one launch per HRB_MULTI_MAX tensors (host arrays of device pointers / sizes /
  * per-tensor l2 scales; l2_scale_host may be NULL).  The layer-by-layer models (DIN, the retrieval towers) hold 12-27 small
  * tensors; Keras applies one optimiser op per variable (keras optimizer_v2 _resource_apply_dense), here they share a launch. */
@@ -379,6 +410,9 @@ int hrb_sgd_step_multi(int32_t count, float* const* param_host, const float* con
                        const float* l2_scale_host, float lr, void* stream);
 int hrb_adagrad_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, float* const* acc_host,
                            const int64_t* n_host, const float* l2_scale_host, float lr, float eps, void* stream);
+int hrb_ftrl_step_multi(int32_t count, float* const* param_host, const float* const* grad_host, float* const* acc_host,
+                        float* const* lin_host, const int64_t* n_host, const float* l2_scale_host, float lr, float l1, float l2,
+                        float lr_power, float l2_shrinkage, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * (e) row-sharded tables: owner(r) = r % n_ranks, local row r / n_ranks  (SURVEY §8e).
@@ -391,7 +425,7 @@ int hrb_adagrad_step_multi(int32_t count, float* const* param_host, const float*
  *   owner      hrb_rows_by_key   out[j,:] = shard row addressed by keys[j]
  *   requester  hrb_scatter_rows  rows -> output block (plain features) / position buffer + pooling (sequence features)
  *   requester  hrb_gather_grads  send[j,:] = dout[b, field(perm[j]) columns] * (1/n_valid for mean pooling)
- *   owner      hrb_keyed_bwd_update  (key, gradient row) pairs -> sort -> segment-reduce -> SGD / lazy-Adam / Adagrad row update */
+ *   owner      hrb_keyed_bwd_update  (key, gradient row) pairs -> sort -> segment-reduce -> SGD / lazy-Adam / Adagrad / Ftrl row update */
 /* Peer-mapped lookup: peer_tables_host[r*n_tables + t] = device pointer of rank r's shard of table t as mapped into this
  * process (CUDA IPC / symmetric memory over NVLink), full_rows_host[t] = full vocabulary size.  After this call
  * hrb_lookup_fwd / hrb_lookup_fm_fwd take GLOBAL ids and read row id from rank id % n_ranks at local row id / n_ranks:

@@ -1,4 +1,4 @@
-"""One-GPU step time of the Criteo-shape DeepFM engine under Adam, Adagrad and SGD, uniform and Zipf ids.
+"""One-GPU step time of the Criteo-shape DeepFM engine under Adam, Adagrad, Ftrl and SGD, uniform and Zipf ids.
 
     python profiles/tools/optimizer_step.py [--steps 30] [--warmup 10] [--rounds 2]
 
@@ -102,7 +102,7 @@ def main():
     lines = []
     for rnd in range(args.rounds):
         for ids in ("uniform", "zipf"):
-            for opt in ("adam", "adagrad", "sgd"):
+            for opt in ("adam", "adagrad", "ftrl", "sgd"):
                 rec = dict(measure(dev, opt, ids, args.steps, args.warmup), round=rnd, **info)
                 line = json.dumps(rec)
                 print(line, flush=True)
