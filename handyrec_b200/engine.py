@@ -233,6 +233,7 @@ class DeepFMEngine:
         self._ws_emb = torch.empty(self.plan.workspace_bytes(B), device=self.dev, dtype=torch.uint8)
 
     _n_pad_flags = 0  # floats the sharded engine keeps behind the touched flags
+    metrics = None  # handyrec_b200.metrics.MetricSet: counted from every training step's probabilities (one launch), None: nothing
 
     # ------------------------------------------------------------------------------------------
     _marks = None  # when a list: (phase name, cuda event) recorded after every phase of a step
@@ -433,6 +434,9 @@ class DeepFMEngine:
         dlogit = self.dZ[-1]  # (B, 1): the logit layer has one unit (DeepFM.py:59-60)
         call("hrb_sigmoid_bce", K._p(self.A[-1]), K._p(self.fm_out), K._p(label), B, 1.0 / (B * self.grad_scale_div), K._p(self.prob), K._p(dlogit), K._p(self.loss_sum), st)
         self._mark("sigmoid_bce")
+        if self.metrics is not None:  # Keras counts its metrics from the training forward, before the weight update
+            self.metrics.update(self.prob[:B], label)
+            self._mark("metric_update")
         self._backward(ids, B, st)
 
     def _backward(self, ids: torch.Tensor, B: int, st) -> None:
@@ -660,12 +664,19 @@ class DeepFMEngine:
         main.synchronize()
         return [float(l[0]) / b for l, b in zip(losses_host, sizes)]
 
-    def predict(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor]) -> torch.Tensor:
+    def predict(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor], label_host: Optional[torch.Tensor] = None,
+                metrics=None) -> torch.Tensor:
+        """Probabilities of one host batch; with `metrics` (a MetricSet) and the batch's labels, also counts them (one launch)."""
         B = ids_host.shape[0]
         self.ids_dev[:B].copy_(ids_host, non_blocking=True)
         if self.n_dense:
             self.dense_dev[:B].copy_(dense_host, non_blocking=True)
-        return self.predict_on_device(self.ids_dev[:B], self.dense_dev[:B] if self.n_dense else None).cpu().reshape(B, 1)
+        if metrics is not None:
+            self.label_dev[:B].copy_(label_host, non_blocking=True)
+        prob = self.predict_on_device(self.ids_dev[:B], self.dense_dev[:B] if self.n_dense else None)
+        if metrics is not None:
+            metrics.update(prob, self.label_dev[:B])
+        return prob.cpu().reshape(B, 1)
 
     def h2d_bytes_per_step(self, B: int) -> int:
         return B * (self.ids_cols * 4 + self.n_dense * 4 + 4)

@@ -579,10 +579,20 @@ class Model:
         return torch.cat(outs).numpy()
 
     _comm = None
+    _metric_set = None  # handyrec_b200.metrics.MetricSet of the compiled metrics, None without
+    _metric_list: Sequence = ()
 
-    def compile(self, optimizer=None, loss=None, distribute=None, **kwargs):
+    def compile(self, optimizer=None, loss=None, distribute=None, metrics=None, **kwargs):
         """keras.Model.compile.  `distribute` (extra): True under an initialised torch.distributed process group (one process per
-        GPU), or a `handyrec_b200.sharded.TorchDistComm` -- a DeepFM-shaped graph then trains on the row-sharded multi-GPU engine."""
+        GPU), or a `handyrec_b200.sharded.TorchDistComm` -- a DeepFM-shaped graph then trains on the row-sharded multi-GPU engine.
+        `metrics`: AUC / Precision / Recall / BinaryAccuracy objects or the strings "AUC", "Precision", "Recall", "accuracy", "acc",
+        "binary_accuracy" (handyrec_b200.metrics; counted on the GPU from each batch's forward output)."""
+        from . import metrics as M
+
+        if kwargs.get("weighted_metrics"):
+            raise NotImplementedError("weighted_metrics: sample weights are not supported")
+        self._metric_list = M.from_compile(metrics)
+        self._metric_set = M.MetricSet(self._metric_list) if self._metric_list else None
         self.optimizer = optimizer if optimizer is not None else Adam()
         self.loss = loss if loss is not None else binary_crossentropy
         self._fused = None
@@ -603,7 +613,47 @@ class Model:
         if self._comm is not None and self._comm.N > 1 and self._fused is None:
             raise ValueError("distribute: only graphs the fused DeepFM engine covers train multi-GPU (lowering.py lists the conditions)")
 
-    def train_on_batch(self, x, y) -> float:
+    # ---- metrics ---------------------------------------------------------------------------------
+    @property
+    def metrics(self) -> list:
+        """The compiled metric objects (Keras also lists its loss tracker here; this list holds the compiled metrics only)."""
+        return list(self._metric_list)
+
+    @property
+    def metrics_names(self) -> List[str]:
+        return ["loss"] + [m.name for m in self._metric_list]
+
+    def reset_metrics(self) -> None:
+        if self._metric_set is not None:
+            self._metric_set.reset()
+
+    def _metric_values(self) -> "OrderedDict[str, Any]":
+        """Every compiled metric's result (a host read; under a multi-GPU communicator a collective summing the ranks' variables)."""
+        comm = self._comm if self._comm is not None and self._comm.N > 1 else None
+        res = self._metric_set.results(comm)
+        return OrderedDict((k, float(v) if np.ndim(v) == 0 else v) for k, v in res.items())
+
+    def _with_metrics(self, loss: float, res, return_dict: bool):
+        if return_dict:
+            return OrderedDict([("loss", loss)] + list(res.items()))
+        return loss if self._metric_set is None else [loss] + list(res.values())
+
+    def train_on_batch(self, x, y, sample_weight=None, class_weight=None, reset_metrics=True, return_dict=False):
+        """keras.Model.train_on_batch: the loss, or [loss, *metric results] when metrics are compiled (a dict with return_dict).
+        reset_metrics=False accumulates the metrics over calls."""
+        from .metrics import _no_sample_weight
+
+        _no_sample_weight(sample_weight)
+        if class_weight is not None:
+            raise NotImplementedError("class_weight is not supported")
+        if self._metric_set is None and not return_dict:
+            return self._train_step(x, y)
+        if reset_metrics:
+            self.reset_metrics()
+        loss = self._train_step(x, y)
+        return self._with_metrics(loss, self._metric_values() if self._metric_set is not None else {}, return_dict)
+
+    def _train_step(self, x, y) -> float:
         if self._fused is not None and isinstance(x, dict):
             n = len(np.asarray(next(iter(x.values()))))
             self._fused.build(n, self.optimizer)
@@ -618,6 +668,8 @@ class Model:
         out = self(x, training=True)
         yt = torch.as_tensor(np.asarray(y), dtype=torch.float32).to(device()) if not isinstance(y, torch.Tensor) else y.to(device())
         loss = self.loss(yt, out)
+        if self._metric_set is not None:  # Keras updates the metrics from the training forward, before the weight update
+            self._metric_set.update(out, yt)
         params = self.weights_with_l2()
         for p, _ in params:
             p.grad = None
@@ -660,11 +712,15 @@ class Model:
                 fn()
 
     def fit(self, x=None, y=None, batch_size=32, epochs=1, validation_data=None, verbose=0, **kwargs):
+        from .metrics import _no_sample_weight
+
+        _no_sample_weight(kwargs.get("sample_weight"))
         history = {"loss": []}
         if isinstance(x, tuple) and len(x) == 2 and isinstance(x[0], dict) and y is None:
             x, y = x
         batches = _batches(x, y, batch_size)
         for _ in range(epochs):
+            self.reset_metrics()  # Keras resets the metrics at the start of every epoch
             if self._fused is not None and isinstance(x, dict):
                 # dict-of-arrays input: batches are packed into pinned memory one step ahead of the GPU and the whole epoch
                 # runs on the fused engine with asynchronous loss read-back (lowering.FusedDeepFM.fit_epoch)
@@ -678,27 +734,19 @@ class Model:
                 tot, cnt = 0.0, 0
                 for xb, yb in batches():  # Keras reports the sample-weighted running mean of the batch losses
                     nb = len(yb) if hasattr(yb, "__len__") else 1
-                    tot += self.train_on_batch(xb, yb) * nb
+                    tot += self._train_step(xb, yb) * nb
                     cnt += nb
                 history["loss"].append(tot / max(cnt, 1))
+            if self._metric_set is not None:
+                for k, v in self._metric_values().items():
+                    history.setdefault(k, []).append(v)
             # fused training leaves the dense / FM weights in the engine; they are handed back to the layers lazily, the first time
             # anything reads the layers (`layers`, `get_layer`, `predict` on the layer path, `save_weights`, `sync()`)
-            fused_val = (validation_data is not None and self._fused is not None and self._fused.engine is not None
-                         and isinstance(validation_data, tuple) and len(validation_data) == 2 and isinstance(validation_data[0], dict))
-            if fused_val:
-                # the fused engine's forward (the only reader a row-sharded table has); Keras' BCE on clipped probabilities
-                xv, yv = validation_data
-                p = np.clip(self._fused.predict(xv, batch_size).reshape(-1).astype(np.float64), 1e-7, 1.0 - 1e-7)
-                yt = np.asarray(yv, dtype=np.float64).reshape(-1)
-                history.setdefault("val_loss", []).append(float(-(yt * np.log(p) + (1.0 - yt) * np.log1p(-p)).mean()))
-            elif validation_data is not None:
-                vl, vc = 0.0, 0
-                with torch.no_grad():
-                    for xb, yb in _batches(validation_data, None, batch_size)():
-                        out = self(xb, training=False)
-                        vl += float(self.loss(torch.as_tensor(np.asarray(yb), dtype=torch.float32).to(device()), out))
-                        vc += 1
-                history.setdefault("val_loss", []).append(vl / max(vc, 1))
+            if validation_data is not None:
+                vl, vres = self._evaluate_pass(validation_data, batch_size)
+                history.setdefault("val_loss", []).append(vl)
+                for k, v in vres.items():
+                    history.setdefault("val_" + k, []).append(v)
 
         class H:
             pass
@@ -706,6 +754,51 @@ class Model:
         h = H()
         h.history = history
         return h
+
+    def _evaluate_pass(self, data, batch_size: int):
+        """The validation pass of `fit` and the body of `evaluate`: (loss, metric results), the metrics reset first."""
+        ms = self._metric_set
+        self.reset_metrics()
+        fused_val = (self._fused is not None and self._fused.engine is not None and isinstance(data, tuple) and len(data) == 2
+                     and isinstance(data[0], dict))
+        if fused_val:
+            # the fused engine's forward (the only reader a row-sharded table has); Keras' BCE on clipped probabilities
+            xv, yv = data
+            p = np.clip(self._fused.predict(xv, batch_size, y=yv, metrics=ms).reshape(-1).astype(np.float64), 1e-7, 1.0 - 1e-7)
+            yt = np.asarray(yv, dtype=np.float64).reshape(-1)
+            loss = float(-(yt * np.log(p) + (1.0 - yt) * np.log1p(-p)).mean())
+        else:
+            vl, vc = 0.0, 0
+            with torch.no_grad():
+                for xb, yb in _batches(data, None, batch_size)():
+                    out = self(xb, training=False)
+                    yt = torch.as_tensor(np.asarray(yb), dtype=torch.float32).to(device())
+                    vl += float(self.loss(yt, out))
+                    if ms is not None:
+                        ms.update(out, yt)
+                    vc += 1
+            loss = vl / max(vc, 1)
+        return loss, (self._metric_values() if ms is not None else OrderedDict())
+
+    def evaluate(self, x=None, y=None, batch_size=None, verbose=0, sample_weight=None, steps=None, callbacks=None, return_dict=False,
+                 **kwargs):
+        """keras.Model.evaluate: the loss, or [loss, *metric results] when metrics are compiled (a dict with return_dict).  The
+        loss is what `fit(validation_data=(x, y), batch_size=batch_size)` records as val_loss on the same path."""
+        from .metrics import _no_sample_weight
+
+        _no_sample_weight(sample_weight)
+        bs = batch_size or 32
+        data = x if (y is None and not isinstance(x, dict)) else (x, y)
+        if (self._fused is not None and self._fused.engine is None and isinstance(data, tuple) and isinstance(data[0], dict)
+                and self._comm is not None and self._comm.N > 1 and self.optimizer is not None):
+            # a multi-GPU model before its first fit: only the engine reads row-sharded tables (collective, as in predict)
+            n = len(np.asarray(next(iter(data[0].values()))))
+            self._fused.build(min(bs, n), self.optimizer)
+        loss, res = self._evaluate_pass(data, bs)
+        return self._with_metrics(loss, res, return_dict)
+
+
+from .metrics import AUC, BinaryAccuracy, Precision, Recall  # noqa: E402  (tf.keras.metrics look-alikes, re-exported)
 
 
 def _all_sublayers(l: Layer) -> List[Layer]:

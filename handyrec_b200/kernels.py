@@ -18,7 +18,7 @@ __all__ = [
     "init_uniform", "embedding_fwd", "embedding_bwd_dense", "seq_pool_fwd", "seq_pool_bwd", "LookupPlan",
     "fm_fwd", "fm_bwd", "dense_fwd", "dense_bwd_x", "dense_bwd_w", "act_bwd", "dice_fwd", "dice_bwd",
     "lau_fwd", "lau_pack_params", "sigmoid_bce", "adam_step", "sgd_step", "adam_step_multi", "sgd_step_multi",
-    "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi",
+    "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi", "metric_scratch_bytes", "metric_update",
 ]
 
 
@@ -633,3 +633,40 @@ def dense1_bwd(x, w, dy, act_prev=None, want_t=False):
     db = torch.empty(1, device=x.device, dtype=torch.float32)
     call("hrb_dense1_bwd", _p(x), _row_major_2d(x, "x"), _p(w), _p(dy), M, Kd, ACT[act_prev], _p(dz), ld, _p(dzt), M, _p(dw), _p(db), _p(ws), ws.numel(), _stream())
     return dz[:, :Kd], (dzt[:Kd] if want_t else None), dw, db
+
+
+# --------------------------------------------------------------------------------------------
+# Keras metrics: confusion / accuracy variables counted on the device (one launch per update)
+# --------------------------------------------------------------------------------------------
+METRIC_TP, METRIC_FP, METRIC_TN, METRIC_FN, METRIC_CORRECT, METRIC_COUNT = 0, 1, 2, 3, 4, 5
+METRIC_MAX_THRESHOLDS = 8192
+
+
+def metric_scratch_bytes(n_thr: int) -> int:
+    need = ctypes.c_size_t(0)
+    call("hrb_metric_scratch_bytes", int(n_thr), ctypes.byref(need))
+    return need.value
+
+
+def metric_update(prob: torch.Tensor, label: torch.Tensor, thresholds: torch.Tensor, var_kind: torch.Tensor, var_thr: torch.Tensor,
+                  vars: torch.Tensor, scratch: torch.Tensor, flags: Optional[torch.Tensor] = None) -> None:
+    """vars[v] += the batch's count of kind var_kind[v] at thresholds[var_thr[v]], one fp32 rounding per variable (hrb200.h:
+    hrb_metric_update).  thresholds ascending and distinct; scratch from metric_scratch_bytes, zeroed once; flags (int32, one per
+    variable, nullable): set for the TP / FP / TN / FN variables when a prob is outside [0, 1] or NaN."""
+    _chk(prob, torch.float32, "prob")
+    _chk(label, torch.float32, "label")
+    _chk(thresholds, torch.float32, "thresholds")
+    _chk(var_kind, torch.int32, "var_kind")
+    _chk(var_thr, torch.int32, "var_thr")
+    _chk(vars, torch.float32, "vars")
+    _chk(scratch, torch.uint8, "scratch")
+    if prob.numel() != label.numel():
+        raise ValueError(f"metric_update: {prob.numel()} predictions but {label.numel()} labels")
+    if not (var_kind.numel() == var_thr.numel() == vars.numel()):
+        raise ValueError("metric_update: var_kind, var_thr and vars must have one entry per variable")
+    if flags is not None and (_chk(flags, torch.int32, "flags").numel() != vars.numel()):
+        raise ValueError("metric_update: flags must have one entry per variable")
+    if scratch.numel() < metric_scratch_bytes(thresholds.numel()):
+        raise ValueError("metric_update: scratch too small (metric_scratch_bytes)")
+    call("hrb_metric_update", _p(prob), _p(label), prob.numel(), _p(thresholds), thresholds.numel(), _p(var_kind), _p(var_thr),
+         vars.numel(), _p(vars), _p(scratch), _p(flags), _stream())

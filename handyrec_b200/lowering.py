@@ -252,6 +252,7 @@ class FusedDeepFM:
             raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD, keras_lite.Adagrad or keras_lite.Ftrl")
         key = key or (opt, lr)
         if self.engine is not None and self.engine.B >= batch_size and self._opt_key == key:
+            self.engine.metrics = getattr(self.model, "_metric_set", None)
             return
         self.sync_to_layers()
         dev = torch.device("cuda", torch.cuda.current_device())
@@ -282,6 +283,7 @@ class FusedDeepFM:
         eng.step_count = getattr(optimizer, "t", 0)
         for t, lay in enumerate(self.tables):  # the layer and the engine share ONE copy of every table
             lay.embeddings.data = eng.tables[t]
+        eng.metrics = getattr(self.model, "_metric_set", None)  # counted by train_step_on_device right after the loss
         self.engine, self._opt_key = eng, key
         self._slots = []
 
@@ -416,15 +418,18 @@ class FusedDeepFM:
         ids, dense, label = slot.views()
         return self.engine.train_on_batch(ids, dense if self.n_dense else None, label)
 
-    def predict(self, x, batch_size: Optional[int]) -> np.ndarray:
+    def predict(self, x, batch_size: Optional[int], y=None, metrics=None) -> np.ndarray:
+        """Probabilities of `x`; with `metrics` (a MetricSet) and labels `y`, every batch is also counted on the device (the
+        validation pass of fit / evaluate: no second forward)."""
         id_cols, dense_cols, n = self._columns(x)
         bs = min(batch_size or n, self.engine.B)
         slot = self._get_slots(1)[0]
+        label_cols = _ColumnSet([np.asarray(y).reshape(-1, 1)]) if metrics is not None else None
         outs = []
         for start in range(0, n, bs):
-            self._pack(slot, id_cols, dense_cols, None, start, min(bs, n - start))
-            ids, dense, _ = slot.views()
-            outs.append(self.engine.predict(ids, dense if self.n_dense else None).numpy().copy())
+            self._pack(slot, id_cols, dense_cols, label_cols, start, min(bs, n - start))
+            ids, dense, label = slot.views()
+            outs.append(self.engine.predict(ids, dense if self.n_dense else None, label, metrics).numpy().copy())
             slot.copied = None
         return np.concatenate(outs, 0)
 

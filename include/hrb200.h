@@ -367,6 +367,34 @@ int hrb_topk_init(float* best_val, int32_t* best_idx, int64_t queries, int32_t k
 int hrb_topk_merge(const float* scores, int64_t ld, int64_t queries, int32_t n_cols, int64_t col_base, int32_t k, float* best_val,
                    int32_t* best_idx, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Keras metrics tf.keras.metrics.{AUC, Precision, Recall, BinaryAccuracy} (Keras 2.6
+ * metrics_utils.update_confusion_matrix_variables and the MeanMetricWrapper of binary_accuracy), one launch per update.
+ *   thresholds (n_thr fp32, ascending, distinct -- not checked, the pointer is a device pointer; 1 <= n_thr <= 8192): the
+ *   union of every metric's thresholds.  Variable v is vars[v] (fp32), of kind var_kind[v] at threshold thresholds[var_thr[v]]
+ *   (ignored for COUNT).  With above_c(j) = #{i : label class c, prob[i] > thresholds[j]} (strict, fp32), classes
+ *   0: label == 0, 1: label == 1, 2: any other label (NaN included; bool(label) is true for classes 1 and 2):
+ *     TP = above_1 + above_2      FP = above_0      TN = tot_0 - above_0      FN = tot_1 + tot_2 - TP
+ *     CORRECT = above_1 + tot_0 - above_0 (binary_accuracy's sum)           COUNT = n
+ *   and vars[v] = fl(vars[v] + (float)increment): the batch's integer count, added with one fp32 rounding (Keras assign_add).
+ *   flags (nullable, n_vars int32, caller-zeroed): when a prob of the batch is outside [0, 1] or NaN, flags[v] = 1 for every
+ *   TP / FP / TN / FN variable v (Keras asserts 0 <= y_pred <= 1 for the confusion metrics; accuracy variables are never
+ *   flagged).  scratch: hrb_metric_scratch_bytes(n_thr), zeroed by the caller once; every call leaves it zeroed (calls sharing a
+ *   scratch must be stream-ordered).  n = 0 launches nothing. */
+#define HRB_METRIC_MAX_THRESHOLDS 8192
+typedef enum hrb_metric_kind {
+  HRB_METRIC_TP = 0,
+  HRB_METRIC_FP = 1,
+  HRB_METRIC_TN = 2,
+  HRB_METRIC_FN = 3,
+  HRB_METRIC_CORRECT = 4,
+  HRB_METRIC_COUNT = 5
+} hrb_metric_kind;
+int hrb_metric_scratch_bytes(int32_t n_thr, size_t* bytes);
+int hrb_metric_update(const float* prob, const float* label, int64_t n, const float* thresholds, int32_t n_thr,
+                      const int32_t* var_kind, const int32_t* var_thr, int32_t n_vars, float* vars, void* scratch, int32_t* flags,
+                      void* stream);
+
 /* a8 concat glue (layers/utils.py:28-36,70-84): dense features (fp32, or int32 cast to fp32) go to the
  * head columns of the DNN input row; columns [n, n_pad) are zero-filled (alignment padding). */
 int hrb_pack_dense(const void* src, int32_t src_is_int32, int64_t src_ld, int64_t batch, int32_t n, int32_t n_pad,
