@@ -214,18 +214,19 @@ HRB_API int hrb_batchnorm_bwd(const float* x, const float* dy, int64_t rows, int
                               const float* var, float eps, int32_t training, float* dx, float* dgamma, float* dbeta,
                               float* scratch /* 2*units floats */, void* stream) {
   HRB_REQUIRE(rows >= 0 && units > 0, "hrb_batchnorm_bwd: bad sizes");
-  HRB_REQUIRE(x && dy && mean && var && dx && scratch, "hrb_batchnorm_bwd: null pointer");
+  HRB_REQUIRE(scratch && (rows == 0 || (x && dy && mean && var && dx)), "hrb_batchnorm_bwd: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   HRB_CUDA(cudaMemsetAsync(scratch, 0, sizeof(float) * 2 * units, st));
-  if (rows == 0) return HRB_OK;
-  dim3 grid;
-  int64_t rpb;
-  slab(rows, units, grid, rpb);
-  bn_colstat_kernel<2><<<grid, 256, 0, st>>>(x, dy, rows, units, rpb, mean, var, eps, scratch, scratch + units);
-  HRB_LAUNCH_CHECK();
-  bn_bwd_kernel<<<ew_grid2(rows * units), 256, 0, st>>>(x, dy, rows * units, units, rows, gamma, mean, var, eps, training, scratch, dx);
-  HRB_LAUNCH_CHECK();
-  // dbeta = sum dy ; dgamma = sum dy*xhat  (already in scratch)
+  if (rows > 0) {
+    dim3 grid;
+    int64_t rpb;
+    slab(rows, units, grid, rpb);
+    bn_colstat_kernel<2><<<grid, 256, 0, st>>>(x, dy, rows, units, rpb, mean, var, eps, scratch, scratch + units);
+    HRB_LAUNCH_CHECK();
+    bn_bwd_kernel<<<ew_grid2(rows * units), 256, 0, st>>>(x, dy, rows * units, units, rows, gamma, mean, var, eps, training, scratch, dx);
+    HRB_LAUNCH_CHECK();
+  }
+  // dbeta = sum dy ; dgamma = sum dy*xhat  (already in scratch; zero for an empty batch)
   if (dbeta != nullptr) HRB_CUDA(cudaMemcpyAsync(dbeta, scratch, sizeof(float) * units, cudaMemcpyDeviceToDevice, st));
   if (dgamma != nullptr) HRB_CUDA(cudaMemcpyAsync(dgamma, scratch + units, sizeof(float) * units, cudaMemcpyDeviceToDevice, st));
   return HRB_OK;

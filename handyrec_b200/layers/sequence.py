@@ -3,6 +3,7 @@ from __future__ import annotations
 
 import torch
 
+from .._lib import HRB_UNSUPPORTED, HrbError
 from ..autograd_ops import TC_MIN_ROWS, AttInputFn, LAUFirstLayerFn, MaskScoresFn, SeqPoolFn
 from ..keras_lite import Layer
 from .core import DNN
@@ -65,8 +66,15 @@ class LocalActivationUnit(Layer):
         params = K.lau_pack_params([d.kernel.data for d in dense], [d.bias.data for d in dense], stats)
         table, q_ids = src_q
         _, k_ids = src_k
-        score, _ = K.lau_fwd(table, q_ids.reshape(-1).contiguous(), k_ids.contiguous(), params, [d.units for d in dense], dnn.activation or "linear",
-                             want_pooled=False)
+        try:
+            score, _ = K.lau_fwd(table, q_ids.reshape(-1).contiguous(), k_ids.contiguous(), params, [d.units for d in dense],
+                                 dnn.activation or "linear", want_pooled=False)
+        except HrbError as e:
+            # widths the fused kernel cannot hold in shared memory (4D or a hidden layer of about 400 and more) are declared
+            # unsupported before anything is launched; the layer-by-layer path computes the same scores
+            if e.status != HRB_UNSUPPORTED:
+                raise
+            return None
         return score
 
     def call(self, inputs, mask=None, **kwargs):

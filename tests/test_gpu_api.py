@@ -333,6 +333,53 @@ def test_din_predict_takes_the_fused_attention_kernel(dev):
     np.testing.assert_allclose(fused, plain, rtol=2e-4, atol=2e-6)
 
 
+def test_din_inference_too_wide_for_the_fused_kernel_takes_the_layer_path(dev):
+    """A 128-wide movie embedding makes the attention MLP's input 4D = 512 wide: more than hrb_lau_fwd's shared-memory tiles hold.
+    The kernel declares that unsupported before launching anything, and inference (predict, and evaluate through it) falls back to
+    the layer path instead of raising: the same probabilities as the forward with gradients enabled."""
+    import bench_models
+    from bench_models import DIN_T, GENRES_L, ML
+    from handyrec_b200 import _lib
+    from handyrec_b200 import keras_lite as KL
+    from handyrec_b200 import kernels as K
+    from handyrec_b200.features import FeatureGroup, FeaturePool, SparseFeature, SparseSeqFeature
+    from handyrec_b200.models import DIN
+
+    torch.manual_seed(0)
+    movie = SparseFeature("movie_id", ML["movie_id"][0], 128)  # bench_models.build_din with a wider movie embedding
+    pool = FeaturePool()
+    seq_group = FeatureGroup("item_seq", [SparseSeqFeature(movie, "hist_movie", DIN_T)], pool, l2_embd=0.0)
+    other = [SparseFeature(k, *ML[k]) for k in ("user_id", "gender", "occupation", "zip", "age")] + [movie, SparseFeature("year", *ML["year"])]
+    other.append(SparseSeqFeature(SparseFeature("genre_id", *ML["genre_id"]), "genres", GENRES_L))
+    m = DIN(seq_group, FeatureGroup("other_feats", other, pool, l2_embd=0.0), dnn_hidden_units=(64, 32), dnn_activation="dice",
+            lau_dnn_hidden_units=(32, 1), lau_dnn_activation="dice")
+    m.compile(optimizer=KL.Adam(learning_rate=1e-3), loss=KL.binary_crossentropy)
+    for l in m._all_layers():
+        if type(l).__name__ == "Dice":
+            l.alphas.data.uniform_(-0.3, 0.3)
+            l.moving_mean.data.uniform_(-0.2, 0.2)
+            l.moving_variance.data.uniform_(0.5, 1.5)
+    x, _ = bench_models.din_data(257)
+    declined = []
+    orig = K.lau_fwd
+
+    def lau_fwd(*a, **k):
+        try:
+            return orig(*a, **k)
+        except _lib.HrbError as e:
+            declined.append(e.status)
+            raise
+
+    K.lau_fwd = lau_fwd
+    try:
+        fused = m.predict(x)
+    finally:
+        K.lau_fwd = orig
+    assert declined == [_lib.HRB_UNSUPPORTED]
+    plain = m(x, training=False).detach().cpu().numpy()
+    np.testing.assert_allclose(fused, plain, rtol=2e-4, atol=2e-6)
+
+
 @pytest.mark.parametrize("Q,N,D,n", [(7, 3883, 32, 100), (600, 20000, 64, 10), (3, 50, 8, 50), (33, 9000, 16, 1)])
 def test_topn_inner_product_search_is_exact(dev, Q, N, D, n):
     """search_embedding == faiss.IndexFlatIP.search: exact top-n by inner product, best first, duplicates (ties) by lower index."""
@@ -365,17 +412,27 @@ def test_ranking_metrics_match_reference_definitions():
     assert abs(search.hr_at_k(actual, pred, 1) - 1 / 3) < 1e-12
 
 
-@pytest.mark.parametrize("act", ["dice", "relu"])
-def test_local_activation_unit_training_path_without_the_4d_tensor(dev, act):
-    """B*T >= 4096 rows: the first LAU layer runs as a per-sample q-term + a [k | q*k] tensor-core GEMM (LAUFirstLayerFn); scores and
-    every gradient (query, keys, all MLP weights, Dice alphas) against the oracle's materialised [q,k,q-k,q*k] path, Dice in training mode."""
+@pytest.mark.parametrize("B,T,D,hidden,act", [
+    (96, 50, 32, (32, 1), "dice"), (96, 50, 32, (32, 1), "relu"),
+    (91, 45, 32, (32, 1), "dice"),          # B*T = 4095: one row short of the tensor-core path, the (B,T,4D) tensor is built
+    (4096, 1, 32, (32, 1), "sigmoid"),      # T = 1, exactly 4096 rows
+    (82, 50, 8, (16, 1), "dice"),           # 4100 rows; 2D = 16, less than one 32-wide k-block
+    (100, 41, 16, (32, 1), "sigmoid"),
+    (1000, 50, 32, (32, 1), "dice"),        # 50 000 rows: the last partial batch of a DIN fit
+    (1000, 50, 64, (32, 1), "tanh"),
+    (96, 50, 128, (64, 1), "sigmoid"),      # 4D = 512
+])
+def test_local_activation_unit_training_path_without_the_4d_tensor(dev, B, T, D, hidden, act):
+    """B*T >= 4096 rows: the first LAU layer runs as a per-sample q-term + a [k | q*k] tensor-core GEMM (LAUFirstLayerFn); below that
+    the (B,T,4D) tensor is materialised.  Scores and every gradient (query, keys, all MLP weights, Dice alphas) against float64
+    autograd of the oracle's materialised [q,k,q-k,q*k] path, Dice in training mode.  Without Dice (whose column statistics use
+    atomics) every reduction runs in fixed order: a second forward + backward gives the same bits."""
     from handyrec_b200.layers import LocalActivationUnit
     from handyrec_b200.layers.activation import Dice
     from handyrec_b200.layers.core import Dense
 
-    B, T, D = 96, 50, 32
     torch.manual_seed(1)
-    lau = LocalActivationUnit(hidden_units=(32, 1), activation=act)
+    lau = LocalActivationUnit(hidden_units=hidden, activation=act)
     lau.build([(None, 1, D), (None, T, D)])
     dense = [l for l in lau.dnn.layers if isinstance(l, Dense)]
     dices = [l for l in lau.dnn.layers if isinstance(l, Dice)]
@@ -385,29 +442,37 @@ def test_local_activation_unit_training_path_without_the_4d_tensor(dev, act):
         d.alphas.data.uniform_(-0.3, 0.3)
     q, k = rnd(B, 1, D, seed=2, scale=0.5), rnd(B, T, D, seed=3, scale=0.5)
     mask = torch.from_numpy(rand_ids(B, T, 100, seed=4).numpy() != 0)
-    p = oracle.dnn_init(4 * D, (32, 1))
-    p.W = [d.kernel.detach().cpu().clone().requires_grad_(True) for d in dense]
-    p.b = [d.bias.detach().cpu().clone().requires_grad_(True) for d in dense]
+    p = oracle.dnn_init(4 * D, hidden)
+    p.W = [d.kernel.detach().cpu().double().requires_grad_(True) for d in dense]
+    p.b = [d.bias.detach().cpu().double().requires_grad_(True) for d in dense]
+    p.dice_mean = [m.double() for m in p.dice_mean]
+    p.dice_var = [v.double() for v in p.dice_var]
     for i, d in enumerate(dices):
-        p.dice_alpha[i] = d.alphas.detach().cpu().clone().requires_grad_(True)
-    ql, kl = q.clone().requires_grad_(True), k.clone().requires_grad_(True)
+        p.dice_alpha[i] = d.alphas.detach().cpu().double().requires_grad_(True)
+    ql, kl = q.double().requires_grad_(True), k.double().requires_grad_(True)
     want = oracle.local_activation_unit(ql, kl, mask, p, act=act, training=True)
     g = rnd(B, 1, T, seed=5)
-    (want * g).sum().backward()
-    qd, kd = q.to(dev).requires_grad_(True), k.to(dev).requires_grad_(True)
-    seen = []
-    from handyrec_b200 import autograd_ops as A
+    (want * g.double()).sum().backward()
 
-    orig = A.LAUFirstLayerFn.apply
-    got = lau.call([qd, kd], mask=[None, mask.to(dev)], training=True)
+    def run():
+        for d in dense:
+            d.kernel.grad, d.bias.grad = None, None
+        for d in dices:
+            d.alphas.grad = None
+        qd, kd = q.to(dev).requires_grad_(True), k.to(dev).requires_grad_(True)
+        got = lau.call([qd, kd], mask=[None, mask.to(dev)], training=True)
+        (got * g.to(dev)).sum().backward()
+        return [got.detach(), qd.grad, kd.grad] + [t.grad for d in dense for t in (d.kernel, d.bias)] + [d.alphas.grad for d in dices]
+
+    res = run()
+    got, dq, dk = res[:3]
     close(got, want, 1e-5)
-    assert got.grad_fn is not None and "LAUFirstLayerFn" in repr(got.grad_fn.next_functions) + repr(
-        [f for fn in got.grad_fn.next_functions for f in (fn[0].next_functions if fn[0] is not None else [])]) or True
-    (got * g.to(dev)).sum().backward()
-    close(qd.grad, ql.grad, 1e-4)
-    close(kd.grad, kl.grad, 1e-4)
+    close(dq, ql.grad, 1e-4)
+    close(dk, kl.grad, 1e-4)
     for d, W, b in zip(dense, p.W, p.b):
         close(d.kernel.grad, W.grad, 1e-4)
         close(d.bias.grad, b.grad, 1e-4)
     for i, d in enumerate(dices):
         close(d.alphas.grad, p.dice_alpha[i].grad, 1e-4)
+    if not dices:
+        assert all(torch.equal(a, b) for a, b in zip(res, run()))

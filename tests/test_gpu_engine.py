@@ -51,9 +51,11 @@ def _oracle_step(eng, tables, fields, ids, dense, label, B, hidden):
     return leaf, p, fm_w, fm_w0, logit, loss
 
 
-@pytest.mark.parametrize("B,D,n_dense,hidden,seq,dense_int", [(1024, 8, 3, (32, 16, 1), True, False), (2048, 16, 13, (64, 8, 1), False, False), (33, 8, 3, (8, 1), True, False), (257, 16, 13, (32, 16, 1), False, False), (64, 8, 1, (4, 1), True, True)])
+@pytest.mark.parametrize("B,D,n_dense,hidden,seq,dense_int", [(1024, 8, 3, (32, 16, 1), True, False), (2048, 16, 13, (64, 8, 1), False, False), (33, 8, 3, (8, 1), True, False), (257, 16, 13, (32, 16, 1), False, False), (64, 8, 1, (4, 1), True, True),
+                                                              (1000, 16, 13, (64, 8, 1), False, False), (4100, 8, 3, (32, 16, 1), True, False)])
 def test_engine_sgd_step_matches_oracle(dev, B, D, n_dense, hidden, seq, dense_int):
     eng, tables, fields, ids, dense, label = _setup(dev, B, D, n_dense, hidden, "sgd", seq, dense_int)
+    assert eng.use_tc == (B >= 512 and B % 4 == 0)  # B = 1000, 4100: the batch is the weight gradients' reduction, a partial k-block
     leaf, p, fm_w, fm_w0, logit, loss = _oracle_step(eng, tables, fields, ids, dense, label, B, hidden)
     prob = eng.predict_on_device(ids.to(dev), dense.to(dev))
     close(prob, torch.sigmoid(logit[:, 0]), 1e-5)

@@ -36,7 +36,7 @@ def test_dense_fwd_t(dev, M, Kd, N, act):
     assert err < 2e-6 * float(want.abs().max()) * np.sqrt(Kd)
 
 
-@pytest.mark.parametrize("M,Kd,N", [(2048, 432, 429), (1024, 256, 128), (4096, 128, 256)])
+@pytest.mark.parametrize("M,Kd,N", [(2048, 432, 429), (1024, 256, 128), (4096, 128, 256), (1000, 256, 128), (4100, 64, 20)])
 def test_dense_bwd_x_t(dev, M, Kd, N):
     k = K()
     a_prev = torch.relu(rnd(M, Kd, seed=1))
@@ -60,7 +60,7 @@ def test_dense_bwd_x_t(dev, M, Kd, N):
     close(out2, (dz.double() @ W.double().T).float(), 1e-4)
 
 
-@pytest.mark.parametrize("M,Kd,N", [(65536, 432, 429), (4096, 256, 128), (2048, 128, 32), (1024, 40, 16)])
+@pytest.mark.parametrize("M,Kd,N", [(65536, 432, 429), (4096, 256, 128), (2048, 128, 32), (1024, 40, 16), (1000, 128, 64), (50000, 64, 128)])
 def test_dense_bwd_w_t(dev, M, Kd, N):
     k = K()
     x = rnd(M, Kd, seed=1)
@@ -76,7 +76,7 @@ def test_dense_bwd_w_t(dev, M, Kd, N):
     assert torch.equal(dw, k.dense_bwd_w_t(xt, dzt, dz.to(dev))[0])  # deterministic
 
 
-@pytest.mark.parametrize("M,Kd,N", [(65536, 432, 429), (4096, 256, 128), (2048, 132, 32), (1024, 40, 16)])
+@pytest.mark.parametrize("M,Kd,N", [(65536, 432, 429), (4096, 256, 128), (2048, 132, 32), (1024, 40, 16), (1000, 64, 128), (50000, 128, 20)])
 def test_dense_bwd_w_untransposed_x(dev, M, Kd, N):
     """The weight gradient from x as stored: the kernel transposes the tile on its way into tensor memory."""
     k = K()

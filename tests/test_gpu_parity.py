@@ -556,24 +556,24 @@ def test_dense_bwd_x_fused_activation_grad_and_padded_ld(dev):
 
 
 @pytest.mark.parametrize("training", [False, True])
-@pytest.mark.parametrize("shape", [(4096, 128), (64, 50, 32), (7, 36)])
+@pytest.mark.parametrize("shape", [(4096, 128), (64, 50, 32), (7, 36), (204800, 128), (4096, 50, 32)])
 def test_dice_fwd_bwd(dev, training, shape):
     k = K()
     units = shape[-1]
-    x = rnd(*shape, seed=1).requires_grad_(True)
-    alpha = rnd(units, seed=2, scale=0.3).requires_grad_(True)
+    x = rnd(*shape, seed=1).double().requires_grad_(True)
+    alpha = rnd(units, seed=2, scale=0.3).double().requires_grad_(True)
     mm, mv = rnd(units, seed=3, scale=0.1), torch.rand(units, generator=torch.Generator().manual_seed(4)) + 0.5
-    want = oracle.dice(x, alpha, mm, mv, training=training)
+    want = oracle.dice(x, alpha, mm.double(), mv.double(), training=training)
     dmean, dvar = mm.clone().to(dev), mv.clone().to(dev)
-    got = k.dice_fwd(x.detach().to(dev), alpha.detach().to(dev), dmean, dvar, training)
+    got = k.dice_fwd(x.detach().float().to(dev), alpha.detach().float().to(dev), dmean, dvar, training)
     close(got, want, FWD_TOL)
     if training:
         red = tuple(range(len(shape) - 1))
         close(dmean, x.detach().mean(red), FWD_TOL)
         close(dvar, x.detach().var(red, unbiased=False), 1e-4)
     dy = rnd(*shape, seed=5)
-    want.backward(dy)
-    dx, dalpha = k.dice_bwd(x.detach().to(dev), dy.to(dev), alpha.detach().to(dev), dmean, dvar, training)
+    want.backward(dy.double())
+    dx, dalpha = k.dice_bwd(x.detach().float().to(dev), dy.to(dev), alpha.detach().float().to(dev), dmean, dvar, training)
     close(dx, x.grad, GRAD_TOL)
     close(dalpha, alpha.grad, GRAD_TOL)
 
@@ -582,7 +582,8 @@ def test_dice_fwd_bwd(dev, training, shape):
 # a10: DIN local activation unit
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("act", ["sigmoid", "relu", "dice"])
-@pytest.mark.parametrize("B,T,D,hidden", [(64, 50, 32, (32, 1)), (5, 2, 8, (36, 1)), (130, 7, 16, (64, 32, 1))])
+@pytest.mark.parametrize("B,T,D,hidden", [(64, 50, 32, (32, 1)), (5, 2, 8, (36, 1)), (130, 7, 16, (64, 32, 1)), (33, 7, 4, (16, 1)),
+                                         (200, 1, 32, (32, 1)), (50, 13, 64, (64, 8, 1))])
 def test_lau_fwd(dev, act, B, T, D, hidden):
     k = K()
     V = 3953
@@ -674,7 +675,7 @@ def test_multi_tensor_optimizer_steps_match_the_single_tensor_ones(dev):
 # ------------------------------------------------------------------------------------------------
 # a11: BatchNormalization / Dropout inside DNN (layers/core.py:71-73)
 # ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("shape", [(777, 37), (64, 50, 36), (4096, 128), (3, 5)])
+@pytest.mark.parametrize("shape", [(777, 37), (64, 50, 36), (4096, 128), (3, 5), (204800, 128), (4096, 50, 32)])
 @pytest.mark.parametrize("training", [True, False])
 def test_batchnorm_fwd_bwd(dev, shape, training):
     """hrb_batchnorm_fwd/bwd against oracle.batch_norm + autograd: training (biased batch statistics over every axis but the
@@ -682,15 +683,15 @@ def test_batchnorm_fwd_bwd(dev, shape, training):
     from handyrec_b200.autograd_ops import BatchNormFn
 
     u = shape[-1]
-    x = (rnd(*shape, seed=1) * 1.7 + 0.3).requires_grad_(True)
-    gamma = (1.0 + 0.2 * rnd(u, seed=2)).requires_grad_(True)
-    beta = (0.1 * rnd(u, seed=3)).requires_grad_(True)
+    x = (rnd(*shape, seed=1) * 1.7 + 0.3).double().requires_grad_(True)
+    gamma = (1.0 + 0.2 * rnd(u, seed=2)).double().requires_grad_(True)
+    beta = (0.1 * rnd(u, seed=3)).double().requires_grad_(True)
     mm, mv = 0.2 * rnd(u, seed=4), 0.5 + rnd(u, seed=5).abs()
     dy = rnd(*shape, seed=6)
-    y, bm, bv = oracle.batch_norm(x, mm, mv, gamma, beta, 1e-3, training)
-    (y * dy).sum().backward()
-    xd = x.detach().to(dev).requires_grad_(True)
-    gd, bd = gamma.detach().to(dev).requires_grad_(True), beta.detach().to(dev).requires_grad_(True)
+    y, bm, bv = oracle.batch_norm(x, mm.double(), mv.double(), gamma, beta, 1e-3, training)
+    (y * dy.double()).sum().backward()
+    xd = x.detach().float().to(dev).requires_grad_(True)
+    gd, bd = gamma.detach().float().to(dev).requires_grad_(True), beta.detach().float().to(dev).requires_grad_(True)
     yd = BatchNormFn.apply(xd, gd, bd, mm.to(dev), mv.to(dev), training, 1e-3)
     close(yd, y, FWD_TOL)
     if training:
@@ -701,6 +702,22 @@ def test_batchnorm_fwd_bwd(dev, shape, training):
     close(xd.grad, x.grad, GRAD_TOL)
     close(gd.grad, gamma.grad, GRAD_TOL)
     close(bd.grad, beta.grad, GRAD_TOL)
+
+
+@pytest.mark.parametrize("training", [True, False])
+def test_batchnorm_bwd_empty_batch_zeroes_parameter_gradients(dev, training):
+    """rows = 0: the gradients of gamma and beta are sums over no rows, i.e. 0 -- written, not left as whatever the output buffers
+    held (BatchNormFn allocates them uninitialised)."""
+    from handyrec_b200._lib import call
+
+    k = K()
+    u = 37
+    x, dy, dx, dgamma, dbeta, scratch = (torch.full((n,), float("nan"), device=dev) for n in (u, u, u, u, u, 2 * u))
+    gamma, mean, var = torch.ones(u, device=dev), torch.zeros(u, device=dev), torch.ones(u, device=dev)
+    call("hrb_batchnorm_bwd", k._p(x), k._p(dy), 0, u, k._p(gamma), k._p(mean), k._p(var), 1e-3, int(training), k._p(dx), k._p(dgamma),
+         k._p(dbeta), k._p(scratch), k._stream())
+    assert torch.equal(dgamma.cpu(), torch.zeros(u)) and torch.equal(dbeta.cpu(), torch.zeros(u))
+    assert bool(dx.isnan().all())  # no rows: nothing else is written
 
 
 @pytest.mark.parametrize("rate", [0.1, 0.5, 0.9])
