@@ -15,6 +15,9 @@ from . import kernels as K
 from ._lib import ACT, POOL, call
 
 
+_grad_clip = None  # handyrec_b200.clip.GradClip while Model._train_on_batch_layers runs a clipped backward
+
+
 class EmbeddingFn(torch.autograd.Function):
     """layers/tools.py:87-101 forward; TF IndexedSlices gradient as a dense, sorted-segment reduction."""
 
@@ -24,6 +27,7 @@ class EmbeddingFn(torch.autograd.Function):
         ctx.save_for_backward(ids)
         ctx.vocab = table.shape[0]
         ctx.sink = sparse_sink
+        ctx.table_id = id(table)
         ctx.mark_non_differentiable(*( [mask] if mask is not None else []))
         return (out, mask) if mask is not None else (out, torch.empty(0, device=table.device, dtype=torch.bool))
 
@@ -36,7 +40,12 @@ class EmbeddingFn(torch.autograd.Function):
             # (CustomEmbedding.apply_sparse) instead of materialising vocab x D floats per step
             ctx.sink.append((ids.reshape(-1), dout.contiguous().reshape(-1, D)))
             return None, None, None, None
-        return K.embedding_bwd_dense(ids.reshape(-1), dout.contiguous().reshape(-1, D), ctx.vocab), None, None, None
+        rows = dout.contiguous().reshape(-1, D)
+        var = _grad_clip.table_vars.get(ctx.table_id) if _grad_clip is not None else None
+        if var is not None:  # Keras clips this lookup's IndexedSlices values, one row per position, before duplicates are summed
+            rows = rows.clone()
+            _grad_clip.prepare([rows], None, None, [var])
+        return K.embedding_bwd_dense(ids.reshape(-1), rows, ctx.vocab), None, None, None
 
 
 class SeqPoolFn(torch.autograd.Function):

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libhrb200.so")
-SOURCES = ["common.cu", "lookup.cu", "embedding_bwd.cu", "fm.cu", "dense.cu", "gemm_tc.cu", "misc.cu", "lau.cu", "layers_misc.cu", "host_pack.cu", "retrieval.cu", "search.cu", "metrics.cu"]
+SOURCES = ["common.cu", "lookup.cu", "embedding_bwd.cu", "fm.cu", "dense.cu", "gemm_tc.cu", "misc.cu", "lau.cu", "layers_misc.cu", "host_pack.cu", "retrieval.cu", "search.cu", "metrics.cu", "clip.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -84,6 +84,9 @@ class DeepFMEngine:
         l2: float = 0.0,
         l2_shrinkage: float = 0.0,
         beta: float = 0.0,
+        clipvalue: Optional[float] = None,
+        clipnorm: Optional[float] = None,
+        global_clipnorm: Optional[float] = None,
     ):
         if dnn_hidden_units[-1] != 1:  # DeepFM.py:59-60
             raise ValueError("Output size of dnn should be 1")
@@ -231,6 +234,53 @@ class DeepFMEngine:
         self.label_dev = torch.zeros(B, **f32)
         self.loss_host = torch.zeros(1, dtype=torch.float32).pin_memory()
         self._ws_emb = torch.empty(self.plan.workspace_bytes(B), device=self.dev, dtype=torch.uint8)
+        self.clip = None
+        if clipvalue is not None or clipnorm is not None or global_clipnorm is not None:
+            self._init_clip((clipvalue, clipnorm, global_clipnorm))
+
+    def _init_clip(self, args) -> None:
+        """Keras gradient clipping (handyrec_b200.clip): one variable per Dense kernel / bias, FM kernel, FM w_0 and table.  With
+        l2_embd = 0 the tables' gradients are their lookups' IndexedSlices, clipped per position in dX0 (the FM part apart, in
+        fm_dx); with l2_embd > 0 they are dense, so every table must be dense-updated and its block is clipped like a Dense kernel."""
+        from .clip import GradClip
+
+        if self.l2_embd > 0.0 and len(self.dense_tables) != len(self.tables):
+            raise ValueError("gradient clipping with l2_embd > 0 needs every table dense-updated (dense_table_max_rows): Keras' "
+                             "clipped gradient of a regularised table covers every row, which the touched-rows update never forms")
+        segs = self._segments[:-1] + [(self.fm_off, self.D, False), (self.fm_off + self.D, 1, False)]
+        self._clip_nd = len(segs)
+        cg, cw, cl, cv = [], [], [], []
+        for k, (o, n, reg) in enumerate(segs):
+            cg.append(self.grads[o : o + n])
+            cw.append(self.params[o : o + n])
+            cl.append(2.0 * self.l2_dnn if reg else 0.0)
+            cv.append(k)
+        if self.l2_embd > 0.0:
+            for t, o in self._table_off.items():
+                n = self.tables[t].numel()
+                cg.append(self.grads[o : o + n])
+                cw.append(self.params[o : o + n])
+                cl.append(2.0 * self.l2_embd)
+                cv.append(self._clip_nd + t)
+        else:
+            self.fm_dx = torch.zeros(self.B, self.F * self.D, device=self.dev, dtype=torch.float32)
+        self._clip_segs = (cg, cw, cl, cv)
+        self.clip = GradClip(args, self._clip_nd + len(self.tables), len(self.tables), self.dev)
+
+    def _clip_gradients(self, ids: torch.Tensor, B: int) -> None:
+        """Keras' _transform_gradients in place, once every gradient of the step is known and before anything steps; the
+        optimisers then run with l2 = 0 where the prepare pass folded 2*l2*w in."""
+        c, nd = self.clip, self._clip_nd
+        cg, cw, cl, cv = self._clip_segs
+        c.begin()
+        if self.l2_embd == 0.0:
+            self.plan.clip_grads(ids, self.dX0[:B], self.fm_dx[:B], c.value, c.sumsq[nd:] if c.scales else None, c.ws)
+        c.prepare(cg, cw, cl, cv)
+        c.finish()
+        c.apply(cg, cv)
+        if self.l2_embd == 0.0 and c.scales:
+            self.plan.clip_apply(self.dX0[:B], B, c.scale[nd:])
+        self._mark("clip")
 
     _n_pad_flags = 0  # floats the sharded engine keeps behind the touched flags
     metrics = None  # handyrec_b200.metrics.MetricSet: counted from every training step's probabilities (one launch), None: nothing
@@ -465,10 +515,17 @@ class DeepFMEngine:
             emb_done[0] = True
             emb_x = self.X0[:, self.nd_pad :]
             emb_dx = self.dX0[:, self.nd_pad :]
-            # FM path adds dlogit * (w + S - x) into the embedding columns of dX0 (interaction.py:26-39)
-            call("hrb_fm_bwd", K._p(emb_x), self.K0p, B, self.F, self.D, K._p(self.fm_w), K._p(self.dZ[-1]), K._p(emb_dx), self.K0p, 1,
-                 K._p(self.d_fm), K._stream())
-            self._mark("fm_bwd")
+            if self.clip is not None and self.l2_embd == 0.0:
+                # clipping: the FM part stays apart (Keras clips the FM and the DNN lookup's values separately), then dX0 takes both
+                call("hrb_fm_bwd", K._p(emb_x), self.K0p, B, self.F, self.D, K._p(self.fm_w), K._p(self.dZ[-1]), K._p(self.fm_dx), self.F * self.D,
+                     0, K._p(self.d_fm), K._stream())
+                self._mark("fm_bwd")
+                self._clip_gradients(ids, B)
+            else:
+                # FM path adds dlogit * (w + S - x) into the embedding columns of dX0 (interaction.py:26-39)
+                call("hrb_fm_bwd", K._p(emb_x), self.K0p, B, self.F, self.D, K._p(self.fm_w), K._p(self.dZ[-1]), K._p(emb_dx), self.K0p, 1,
+                     K._p(self.d_fm), K._stream())
+                self._mark("fm_bwd")
             if side and self._marks is None:
                 main = torch.cuda.current_stream()
                 if self._side is None:
@@ -539,11 +596,14 @@ class DeepFMEngine:
         if not emb_done[0]:
             emb_part(side=False)
         self._sync_dense_grads()
-        # dense parameters
-        segs = [(o_, n_, 2.0 * self.l2_dnn if reg else 0.0) for o_, n_, reg in self._segments]
+        if self.clip is not None and self.l2_embd != 0.0:  # the table block holds the tables' dense gradients now
+            self._clip_gradients(ids, B)
+        # dense parameters (a clip folded every regulariser into the gradients)
+        fold = self.clip is not None
+        segs = [(o_, n_, 2.0 * self.l2_dnn if reg and not fold else 0.0) for o_, n_, reg in self._segments]
         ftrl_rows = self.optimizer == "ftrl" and self.touched is not None and self.l2_embd == 0.0
         if self.n_params > self.n_dense_params and not ftrl_rows:  # dense-updated tables: Keras adds d(l2_embd*sum w^2) for every row (group.py:289)
-            segs.append((self.n_dense_params, self.n_params - self.n_dense_params, 2.0 * self.l2_embd))
+            segs.append((self.n_dense_params, self.n_params - self.n_dense_params, 0.0 if fold else 2.0 * self.l2_embd))
         merged = [segs[0]]
         for o_, n_, l2_ in segs[1:]:  # neighbouring segments with the same regulariser take one launch
             po, pn, pl = merged[-1]

@@ -18,6 +18,8 @@ from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple, Union
 import numpy as np
 import torch
 
+from .clip import init_clip
+
 _uid = itertools.count()
 
 
@@ -326,10 +328,13 @@ class Activation(Layer):
 
 
 # ---------------------------------------------------------------------------------------------
-# optimisers / losses (Keras formulas, kernels from libhrb200)
+# optimisers / losses (Keras formulas, kernels from libhrb200).  Every optimiser takes Keras' clipnorm / clipvalue /
+# global_clipnorm (handyrec_b200.clip); the model clips the gradients before it calls `step`.
 # ---------------------------------------------------------------------------------------------
 class Adam:
-    def __init__(self, learning_rate=1e-3, lr=None, beta_1=0.9, beta_2=0.999, epsilon=1e-7):
+    def __init__(self, learning_rate=1e-3, lr=None, beta_1=0.9, beta_2=0.999, epsilon=1e-7, clipnorm=None, clipvalue=None,
+                 global_clipnorm=None):
+        init_clip(self, clipnorm, clipvalue, global_clipnorm)
         self.lr = float(lr if lr is not None else learning_rate)
         self.b1, self.b2, self.eps, self.t = beta_1, beta_2, epsilon, 0
         self.state: Dict[int, Tuple[torch.Tensor, torch.Tensor]] = {}
@@ -357,7 +362,9 @@ class Adagrad:
     """tf.keras.optimizers.Adagrad (Keras 2.6): acc += g^2; w -= lr * g / (sqrt(acc) + eps), acc starting at
     initial_accumulator_value.  Large tables take the same step on the rows a batch touches (CustomEmbedding.apply_sparse)."""
 
-    def __init__(self, learning_rate=0.001, initial_accumulator_value=0.1, epsilon=1e-7, lr=None):
+    def __init__(self, learning_rate=0.001, initial_accumulator_value=0.1, epsilon=1e-7, lr=None, clipnorm=None, clipvalue=None,
+                 global_clipnorm=None):
+        init_clip(self, clipnorm, clipvalue, global_clipnorm)
         if initial_accumulator_value < 0.0:
             raise ValueError(f"initial_accumulator_value must be non-negative: {initial_accumulator_value}")
         self.lr = float(lr if lr is not None else learning_rate)
@@ -387,7 +394,9 @@ class Ftrl:
     (CustomEmbedding.apply_sparse)."""
 
     def __init__(self, learning_rate=0.001, learning_rate_power=-0.5, initial_accumulator_value=0.1, l1_regularization_strength=0.0,
-                 l2_regularization_strength=0.0, name="Ftrl", l2_shrinkage_regularization_strength=0.0, beta=0.0, lr=None):
+                 l2_regularization_strength=0.0, name="Ftrl", l2_shrinkage_regularization_strength=0.0, beta=0.0, lr=None,
+                 clipnorm=None, clipvalue=None, global_clipnorm=None):
+        init_clip(self, clipnorm, clipvalue, global_clipnorm)
         if initial_accumulator_value < 0.0:
             raise ValueError(f"initial_accumulator_value {initial_accumulator_value} needs to be positive or zero")
         if learning_rate_power > 0.0:
@@ -429,7 +438,8 @@ class Ftrl:
 
 
 class SGD:
-    def __init__(self, learning_rate=0.01, lr=None):
+    def __init__(self, learning_rate=0.01, lr=None, clipnorm=None, clipvalue=None, global_clipnorm=None):
+        init_clip(self, clipnorm, clipvalue, global_clipnorm)
         self.lr = float(lr if lr is not None else learning_rate)
 
     def step(self, params_l2):
@@ -603,6 +613,14 @@ class Model:
             from .sharded import TorchDistComm
 
             self._comm = distribute if not isinstance(distribute, bool) else TorchDistComm()
+        from .clip import clip_args
+
+        clip = clip_args(self.optimizer)
+        self._clip_state = None
+        if clip is not None and self._comm is not None and self._comm.N > 1:
+            # Keras clips the global-batch gradient: the per-variable norms would have to ride in the ranks' all-reduce
+            raise ValueError("gradient clipping (clipnorm / clipvalue / global_clipnorm) is not supported on a multi-GPU compile: "
+                             "Keras clips the global-batch gradient, which the sharded step does not form before it updates")
         for l in self._all_layers():  # under Ftrl a dense step would move the rows a batch does not gather
             if hasattr(l, "SPARSE_UPDATE_MIN_ROWS"):
                 l._ftrl = isinstance(self.optimizer, Ftrl)
@@ -612,6 +630,18 @@ class Model:
             self._fused = lower(self)
         if self._comm is not None and self._comm.N > 1 and self._fused is None:
             raise ValueError("distribute: only graphs the fused DeepFM engine covers train multi-GPU (lowering.py lists the conditions)")
+        if clip is not None:
+            for l in self._all_layers():
+                if getattr(l, "l2", 0.0) and hasattr(l, "SPARSE_UPDATE_MIN_ROWS") and l.trainable and self._rows_updated(l):
+                    raise ValueError(f"{l.name}: gradient clipping with an l2 regulariser on a table that takes the touched-rows update "
+                                     f"({l.input_dim} rows): Keras' clipped gradient then covers every row of the table, which that "
+                                     "update never forms")
+
+    def _rows_updated(self, emb) -> bool:
+        """Whether the table of CustomEmbedding `emb` takes the touched-rows update on the path this compile chose."""
+        if self._fused is not None and any(t is emb for t in self._fused.tables):
+            return emb.input_dim > getattr(self, "dense_table_max_rows", 131072)
+        return emb.input_dim >= emb.SPARSE_UPDATE_MIN_ROWS and emb.output_dim % 4 == 0
 
     # ---- metrics ---------------------------------------------------------------------------------
     @property
@@ -673,17 +703,71 @@ class Model:
         params = self.weights_with_l2()
         for p, _ in params:
             p.grad = None
-        loss.backward()
+        clip = self._layer_clip(params)
+        if clip is None:
+            loss.backward()
+        else:
+            from . import autograd_ops
+
+            autograd_ops._grad_clip = clip  # EmbeddingFn clamps and counts the position rows of the dense-gradient tables
+            try:
+                loss.backward()
+            finally:
+                autograd_ops._grad_clip = None
         sparse = [l for l in self._all_layers() if getattr(l, "_sparse_grads", None)]
         skip = {id(l.embeddings) for l in sparse}
         # Keras adds the regularisation losses to the reported loss; their gradient 2*l2*W is applied inside the update kernels
         # (tables under the sparse row update are left out of the reported term: a full pass over them is what that update avoids)
         reg = sum(float(l2) * float((p.detach() * p.detach()).sum()) for p, l2 in params if l2 and id(p) not in skip)
+        if clip is not None:
+            params = self._clip_gradients(clip, params, sparse)
         self.optimizer.step(params)
         for l in sparse:  # large tables: IndexedSlices-style gradient -> sorted-segment row update
             l.apply_sparse(self.optimizer)
         self._update_moving_stats()
         return float(loss.detach()) + reg
+
+    _clip_state = None  # handyrec_b200.clip.GradClip of the layer path, built at the first clipped step
+
+    def _layer_clip(self, params):
+        """The GradClip of this step (sums zeroed, variables indexed), or None when the optimizer does not clip."""
+        from .clip import GradClip, clip_args
+
+        args = clip_args(self.optimizer)
+        if args is None:
+            return None
+        live = [p for p, _ in params if p.requires_grad]
+        st = self._clip_state
+        if st is None or st.n_vars != len(live):
+            st = self._clip_state = GradClip(args, len(live), 0, device())
+        st.var = {id(p): i for i, p in enumerate(live)}
+        # tables without a regulariser whose gradient is formed densely: their lookups' IndexedSlices values are clipped in
+        # EmbeddingFn.backward, position by position
+        st.table_vars = {id(l.embeddings): st.var[id(l.embeddings)] for l in self._all_layers()
+                         if hasattr(l, "SPARSE_UPDATE_MIN_ROWS") and not l.l2 and id(l.embeddings) in st.var}
+        st.begin()
+        return st
+
+    def _clip_gradients(self, clip, params, sparse):
+        """Keras' _transform_gradients on this step's gradients, in place: the dense gradients with 2*l2*w folded in, the large
+        tables' (ids, rows) per position; then the norm scales.  Returns params with l2 = 0 (folded)."""
+        var, tv = clip.var, clip.table_vars
+        rows = []
+        for l in sparse:  # the concatenated lookups of one table: Keras' aggregated IndexedSlices, in a buffer of our own
+            ids = torch.cat([i for i, _ in l._sparse_grads])
+            r = torch.cat([g for _, g in l._sparse_grads])
+            l._sparse_grads[:] = [(ids, r)]
+            rows.append((r, var[id(l.embeddings)]))
+        dense = [(p, l2) for p, l2 in params if p.grad is not None and p.requires_grad and id(p) not in tv]
+        for p, _ in dense:
+            p.grad = p.grad.contiguous()
+        gs = [p.grad for p, _ in dense] + [r for r, _ in rows]
+        vs = [var[id(p)] for p, _ in dense] + [v for _, v in rows]
+        clip.prepare(gs, [p.data for p, _ in dense] + [None] * len(rows), [2.0 * l2 for _, l2 in dense] + [0.0] * len(rows), vs)
+        clip.finish()
+        tabs = [p for p, _ in params if p.grad is not None and id(p) in tv]
+        clip.apply(gs + [p.grad for p in tabs], vs + [tv[id(p)] for p in tabs])
+        return [(p, 0.0) for p, _ in params]
 
     def save_weights(self, filepath, **kwargs):
         """keras.Model.save_weights: a directory of `.npy` files (tables row-sharded), see handyrec_b200.checkpoint."""

@@ -19,6 +19,7 @@ __all__ = [
     "fm_fwd", "fm_bwd", "dense_fwd", "dense_bwd_x", "dense_bwd_w", "act_bwd", "dice_fwd", "dice_bwd",
     "lau_fwd", "lau_pack_params", "sigmoid_bce", "adam_step", "sgd_step", "adam_step_multi", "sgd_step_multi",
     "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi", "metric_scratch_bytes", "metric_update",
+    "clip_workspace", "clip_prepare_multi", "clip_scales", "clip_apply_multi",
 ]
 
 
@@ -225,6 +226,23 @@ class LookupPlan:
     def ftrl_pad_step(self, flags: torch.Tensor, op: OptParams) -> None:
         """Row 0 of every row-updated table whose flags show padding and no valid id 0 takes its zero-gradient Ftrl step."""
         call("hrb_plan_ftrl_pad_step", self._h, _p(flags), ctypes.byref(op), _stream())
+
+    def clip_grads(self, ids: torch.Tensor, dx: torch.Tensor, fm: Optional[torch.Tensor], clipvalue: float,
+                   sumsq: Optional[torch.Tensor], workspace: torch.Tensor) -> None:
+        """hrb_plan_clip_grads: the DNN part (dx, the plan's column layout) and the FM part (fm, field f at column out_col_f -
+        out_col_0) of every field's gradient clamped per position, dx <- their sum; sumsq[t] += the table's squared norm."""
+        B = ids.shape[0]
+        dx_ld = _row_major_2d(_chk(dx, torch.float32, "dx", contiguous=False), "dx")
+        fm_ld = _row_major_2d(_chk(fm, torch.float32, "fm", contiguous=False), "fm") if fm is not None else 0
+        if sumsq is not None:
+            _chk(sumsq, torch.float32, "sumsq")
+        call("hrb_plan_clip_grads", self._h, _p(ids), self._ids_ld(ids), B, _p(dx), dx_ld, _p(fm), fm_ld, float(clipvalue), _p(sumsq),
+             _p(workspace), workspace.numel(), _stream())
+
+    def clip_apply(self, dx: torch.Tensor, batch: int, scale: torch.Tensor) -> None:
+        """hrb_plan_clip_apply: dx[:, columns of field f] *= scale[table of f]."""
+        dx_ld = _row_major_2d(_chk(dx, torch.float32, "dx", contiguous=False), "dx")
+        call("hrb_plan_clip_apply", self._h, _p(dx), dx_ld, batch, _p(_chk(scale, torch.float32, "scale")), _stream())
 
     def __del__(self):
         try:  # module globals may already be gone at interpreter shutdown
@@ -537,6 +555,50 @@ def ftrl_step_multi(params, grads, accs, lins, l2_scales, lr, l1=0.0, l2=0.0, lr
     call("hrb_ftrl_step_multi", n, _ptr_array(params), _ptr_array(grads), _ptr_array(accs), _ptr_array(lins),
          (ctypes.c_int64 * n)(*[p.numel() for p in params]), (ctypes.c_float * n)(*l2_scales), lr, l1, l2, lr_power, l2_shrinkage,
          _stream())
+
+
+# --------------------------------------------------------------------------------------------
+# gradient clipping (Keras OptimizerV2 clipvalue / clipnorm / global_clipnorm), in place
+# --------------------------------------------------------------------------------------------
+def clip_workspace(n_tables: int, device) -> torch.Tensor:
+    """A zeroed workspace for the clip entries (every call leaves it zeroed; calls sharing it must be stream-ordered)."""
+    need = ctypes.c_size_t(0)
+    call("hrb_clip_workspace_bytes", int(n_tables), ctypes.byref(need))
+    return torch.zeros(need.value, device=device, dtype=torch.uint8)
+
+
+def clip_prepare_multi(grads: Sequence[torch.Tensor], weights: Optional[Sequence[Optional[torch.Tensor]]], l2_scales: Optional[Sequence[float]],
+                       var: Sequence[int], clipvalue: float, sumsq: Optional[torch.Tensor], workspace: torch.Tensor) -> None:
+    """hrb_clip_prepare_multi: g <- clamp(g + l2_scale * w, -clipvalue, clipvalue) in place; sumsq[var[i]] += sum g^2."""
+    n = len(grads)
+    if n == 0:
+        return
+    for t in grads:
+        _chk(t, torch.float32, "grad")
+    if sumsq is not None:
+        _chk(sumsq, torch.float32, "sumsq")
+    w = None if weights is None else (ctypes.c_void_p * n)(*[(t.data_ptr() if t is not None else None) for t in weights])
+    call("hrb_clip_prepare_multi", n, _ptr_array(grads), w, (ctypes.c_int64 * n)(*[g.numel() for g in grads]),
+         None if l2_scales is None else (ctypes.c_float * n)(*l2_scales), (ctypes.c_int32 * n)(*var), float(clipvalue), _p(sumsq),
+         _p(workspace), workspace.numel(), _stream())
+
+
+def clip_scales(sumsq: torch.Tensor, clipnorm: float, global_norm: bool, scale: torch.Tensor) -> None:
+    """hrb_clip_scales: scale[k] = c / max(||g_k||, c), or one scale from the global norm (NaN when it is not finite)."""
+    _chk(sumsq, torch.float32, "sumsq")
+    _chk(scale, torch.float32, "scale")
+    call("hrb_clip_scales", _p(sumsq), sumsq.numel(), float(clipnorm), int(global_norm), _p(scale), _stream())
+
+
+def clip_apply_multi(grads: Sequence[torch.Tensor], var: Sequence[int], scale: torch.Tensor) -> None:
+    """hrb_clip_apply_multi: g *= scale[var[i]] in place."""
+    n = len(grads)
+    if n == 0:
+        return
+    for t in grads:
+        _chk(t, torch.float32, "grad")
+    call("hrb_clip_apply_multi", n, _ptr_array(grads), (ctypes.c_int64 * n)(*[g.numel() for g in grads]), (ctypes.c_int32 * n)(*var),
+         _p(_chk(scale, torch.float32, "scale")), _stream())
 
 
 # --------------------------------------------------------------------------------------------

@@ -234,6 +234,7 @@ class FusedDeepFM:
         return [l for l in self.spec.dnn.layers if isinstance(l, Dense)]
 
     def build(self, batch_size: int, optimizer) -> None:
+        from .clip import clip_args
         from .engine import DeepFMEngine
         from .keras_lite import Adagrad, Adam, Ftrl, SGD
 
@@ -250,7 +251,8 @@ class FusedDeepFM:
                    optimizer.l2_shrinkage, optimizer.beta)
         else:
             raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD, keras_lite.Adagrad or keras_lite.Ftrl")
-        key = key or (opt, lr)
+        clip = clip_args(optimizer)
+        key = (key or (opt, lr), clip)
         if self.engine is not None and self.engine.B >= batch_size and self._opt_key == key:
             self.engine.metrics = getattr(self.model, "_metric_set", None)
             return
@@ -271,7 +273,8 @@ class FusedDeepFM:
             eng = self._build_sharded(comm, dev, fields, small, common)
         else:
             tabs = [t.embeddings.data.to(dev) for t in self.tables]
-            eng = DeepFMEngine(tabs, fields, self.n_dense, dense_table_max_rows=small, **common)
+            clip_kw = dict(zip(("clipvalue", "clipnorm", "global_clipnorm"), clip)) if clip is not None else {}
+            eng = DeepFMEngine(tabs, fields, self.n_dense, dense_table_max_rows=small, **common, **clip_kw)
         if opt == "adam":
             eng.beta1, eng.beta2, eng.eps = optimizer.b1, optimizer.b2, optimizer.eps
         elif opt == "adagrad":

@@ -443,6 +443,47 @@ int hrb_ftrl_step_multi(int32_t count, float* const* param_host, const float* co
                         float lr_power, float l2_shrinkage, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Gradient clipping: Keras 2.6 OptimizerV2 `clipvalue`, `clipnorm`, `global_clipnorm` (optimizer_v2.py
+ * `_transform_gradients`: clipvalue first, then clipnorm, then global_clipnorm).  In-place passes that run after every
+ * gradient of a step is known and before the optimiser steps above (which are unchanged); the caller then steps with l2 = 0
+ * wherever the prepare pass folded a regulariser in.  Squared norms are summed in float64 in a fixed order (the same bits on
+ * every run) and added to sumsq[var] (fp32, caller-zeroed per step) with one rounding per call.
+ *   workspace: hrb_clip_workspace_bytes(n_tables of the plan, or 0), zeroed by the caller once.  It holds one completion
+ *   counter per entry point (each call leaves its counter zeroed) and the partial sums, so hrb_clip_prepare_multi and
+ *   hrb_plan_clip_grads may share one workspace sized for the plan (calls sharing it must be stream-ordered).
+ *   clipvalue = +INFINITY: no clamp.
+ *
+ * hrb_clip_prepare_multi   tf.clip_by_value on dense gradients with the regulariser folded in, and their squared norms:
+ *     per segment i (host arrays as in hrb_*_step_multi, any count; w_host / l2_scale_host nullable, w_host[i] NULL needs l2 0):
+ *     g[j] = clamp(fmaf(l2_scale[i], w[j], g[j]), -clipvalue, clipvalue);  sumsq[var[i]] += sum_j g[j]^2 (sumsq nullable).
+ *     NaN passes the clamp unchanged.
+ * hrb_plan_clip_grads      the same for the IndexedSlices gradient of the plan's tables (tf.clip_by_value and the norm of
+ *     clip_by_norm over the un-deduplicated values), where the DNN part of a field's gradient is in dx and the FM part in fm
+ *     (DeepFM looks every table up twice; Keras concatenates the two lookups' values, backprop_util.AggregateIndexedSlicesGradients).
+ *     Per sample b, field f, element: p = part * inv with inv = 1/n_valid (mean pooling) or 1, clamped per part; dx receives the
+ *     sum of the two parts in the form the backward reads (a part whose clamp does not bind is kept unchanged, a bound one
+ *     becomes +-clipvalue * n_valid for mean pooling, +-clipvalue otherwise), and sumsq[table] += n_valid * (p_dnn'^2 + p_fm'^2).
+ *     n_valid counts the positions the backward reads: in-range ids, and ids != 0 for pooled fields.  fm (nullable; needs
+ *     contiguous field columns) holds field f at column out_col_f - out_col_0; sumsq (n_tables floats) nullable.  No max pooling.
+ * hrb_clip_scales          tf.clip_by_norm / tf.clip_by_global_norm as a scale: scale[k] = c / max(sqrt(sumsq[k]), c) per
+ *     variable, or (global != 0) every scale[k] = c / max(sqrt(sum_k sumsq[k]), c), NaN when that norm is not finite (TF's
+ *     `scale + (norm - norm)`).  A norm <= c gives exactly 1; norm 0 with c = 0 gives NaN, as in TF.  One launch, no host sync.
+ * hrb_clip_apply_multi     g[j] *= scale[var[i]] over segments.
+ * hrb_plan_clip_apply      dx[b, columns of field f] *= scale[table of f] (the plan's layout as in hrb_lookup_bwd_update).
+ * ------------------------------------------------------------------------------------------ */
+int hrb_clip_workspace_bytes(int32_t n_tables, size_t* bytes);
+int hrb_clip_prepare_multi(int32_t count, float* const* g_host, const float* const* w_host, const int64_t* n_host,
+                           const float* l2_scale_host, const int32_t* var_host, float clipvalue, float* sumsq, void* workspace,
+                           size_t workspace_bytes, void* stream);
+int hrb_plan_clip_grads(const hrb_plan* plan, const int32_t* ids, int64_t ids_ld, int64_t batch, float* dx, int64_t dx_ld,
+                        const float* fm, int64_t fm_ld, float clipvalue, float* sumsq, void* workspace, size_t workspace_bytes,
+                        void* stream);
+int hrb_clip_scales(const float* sumsq, int32_t n_vars, float clipnorm, int32_t global, float* scale, void* stream);
+int hrb_clip_apply_multi(int32_t count, float* const* g_host, const int64_t* n_host, const int32_t* var_host, const float* scale,
+                         void* stream);
+int hrb_plan_clip_apply(const hrb_plan* plan, float* dx, int64_t dx_ld, int64_t batch, const float* scale, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * (e) row-sharded tables: owner(r) = r % n_ranks, local row r / n_ranks  (SURVEY §8e).
  * ------------------------------------------------------------------------------------------ */
 
