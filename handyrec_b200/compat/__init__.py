@@ -5,7 +5,8 @@
 `tensorflow` / `tensorflow.keras` and call a dozen TF names (`Model`, `Activation`, `tf.matmul`, `tf.nn.l2_normalize`,
 `tf.nn.embedding_lookup`, `tf.squeeze`, `tf.int32`).  `install(reference_root)` registers
 
-    tensorflow, tensorflow.keras[.layers|.models|.initializers|.regularizers|.losses|.optimizers|.metrics] -> thin modules over keras_lite
+    tensorflow, tensorflow.keras[.layers|.models|.initializers|.regularizers|.losses|.optimizers[.schedules]|.metrics|.experimental]
+                                                                                                    -> thin modules over keras_lite
     handyrec, handyrec.features, handyrec.layers, handyrec.layers.utils, handyrec.features.*        -> this package's drop-in face
     handyrec.models (+ .ranking, .retrieval, ...)                                                   -> the reference's files, loaded
                                                                                                        from `reference_root` UNMODIFIED
@@ -94,14 +95,23 @@ def _tf_module() -> types.ModuleType:
     losses.binary_crossentropy = KL.binary_crossentropy
     opts = types.ModuleType("tensorflow.keras.optimizers")
     opts.Adam, opts.SGD, opts.Adagrad, opts.Ftrl = KL.Adam, KL.SGD, KL.Adagrad, KL.Ftrl
+    from .. import schedules as S
+
+    scheds = types.ModuleType("tensorflow.keras.optimizers.schedules")
+    for n in ("LearningRateSchedule", "ExponentialDecay", "InverseTimeDecay", "PiecewiseConstantDecay", "PolynomialDecay"):
+        setattr(scheds, n, getattr(S, n))
+    opts.schedules = scheds
+    experimental = types.ModuleType("tensorflow.keras.experimental")  # Keras 2.6 keeps the cosine schedules here
+    experimental.CosineDecay, experimental.CosineDecayRestarts = S.CosineDecay, S.CosineDecayRestarts
     mets = types.ModuleType("tensorflow.keras.metrics")
     mets.AUC, mets.BinaryAccuracy, mets.Precision, mets.Recall = KL.AUC, KL.BinaryAccuracy, KL.Precision, KL.Recall
     keras.layers, keras.models, keras.initializers, keras.regularizers, keras.losses, keras.optimizers = layers, models, inits, regs, losses, opts
-    keras.metrics = mets
+    keras.metrics, keras.experimental = mets, experimental
     tf.keras = keras
     tf._submodules = {"tensorflow.nn": nn, "tensorflow.keras": keras, "tensorflow.keras.layers": layers, "tensorflow.keras.models": models,
                       "tensorflow.keras.initializers": inits, "tensorflow.keras.regularizers": regs, "tensorflow.keras.losses": losses,
-                      "tensorflow.keras.optimizers": opts, "tensorflow.keras.metrics": mets}
+                      "tensorflow.keras.optimizers": opts, "tensorflow.keras.optimizers.schedules": scheds, "tensorflow.keras.metrics": mets,
+                      "tensorflow.keras.experimental": experimental}
     return tf
 
 

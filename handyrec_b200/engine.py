@@ -58,6 +58,8 @@ class DeepFMEngine:
     Adagrad and Ftrl the touched-rows-only update is exactly Keras' step whenever l2_embd = 0 (DESIGN.md 3).  Under Ftrl a
     zero-gradient step is not a no-op, so with l2_embd = 0 the dense-updated tables step only the rows the batch gathers
     (padding id 0 of pooled fields included): `plan.mark_rows` flags them in the tail of the flat gradient buffer.
+
+    lr: the learning rate of every step, or None when `lr_step` gives each step its own (a Keras schedule).
     """
 
     def __init__(
@@ -69,7 +71,7 @@ class DeepFMEngine:
         dnn_activation: str = "relu",
         batch_size: int = 4096,
         optimizer: str = "adam",
-        lr: float = 1e-3,
+        lr: Optional[float] = 1e-3,
         l2_embd: float = 0.0,
         l2_dnn: float = 0.0,
         embedding_optimizer: Optional[str] = None,
@@ -111,11 +113,12 @@ class DeepFMEngine:
         self.act = dnn_activation or "linear"
         self.optimizer = optimizer
         self.emb_opt = embedding_optimizer or {"adam": "adam_lazy", "adagrad": "adagrad", "ftrl": "ftrl"}.get(optimizer, "sgd")
-        self.lr, self.l2_embd, self.l2_dnn = float(lr), float(l2_embd), float(l2_dnn)
+        self.l2_embd, self.l2_dnn = float(l2_embd), float(l2_dnn)
         self.beta1, self.beta2, self.eps = 0.9, 0.999, 1e-7  # Keras Adam defaults (eps: also Keras Adagrad's)
         self.initial_accumulator_value = float(initial_accumulator_value)
         self.lr_power, self.l1, self.l2_shrinkage, self.beta = float(learning_rate_power), float(l1), float(l2_shrinkage), float(beta)
-        self.ftrl_l2 = float(l2) + self.beta / (2.0 * self.lr)  # the l2 Keras hands its Ftrl kernel
+        self.ftrl_l2_reg = float(l2)
+        self.set_lr(lr)
         self.gemm_mode = gemm_mode
         self.step_count = 0
 
@@ -281,6 +284,19 @@ class DeepFMEngine:
         if self.l2_embd == 0.0 and c.scales:
             self.plan.clip_apply(self.dX0[:B], B, c.scale[nd:])
         self._mark("clip")
+
+    # When set, a callable giving the learning rate of every training step, called once per step by train_step_on_device before
+    # anything launches (lowering.FusedDeepFM: a Keras schedule / decay, counted in the optimizer's `iterations`).  The rate reaches
+    # the kernels as a launch argument: no extra launch, no host sync, no rebuild.
+    lr_step = None
+
+    def set_lr(self, lr: Optional[float]) -> None:
+        """The learning rate of the following steps, with the l2 Keras hands its Ftrl kernel at that rate (l2 + beta / (2*lr)).
+        None: no rate until `lr_step` gives the first step its own."""
+        from .schedules import ftrl_kernel_l2
+
+        self.lr = None if lr is None else float(lr)
+        self.ftrl_l2 = None if lr is None else ftrl_kernel_l2(self.ftrl_l2_reg, self.beta, self.lr)
 
     _n_pad_flags = 0  # floats the sharded engine keeps behind the touched flags
     metrics = None  # handyrec_b200.metrics.MetricSet: counted from every training step's probabilities (one launch), None: nothing
@@ -479,6 +495,8 @@ class DeepFMEngine:
         B = ids.shape[0]
         st = K._stream()
         self.step_count += 1
+        if self.lr_step is not None:
+            self.set_lr(self.lr_step())
         self.forward(ids, dense, training=True)
         self.loss_sum.zero_()
         dlogit = self.dZ[-1]  # (B, 1): the logit layer has one unit (DeepFM.py:59-60)

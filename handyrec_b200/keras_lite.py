@@ -19,6 +19,7 @@ import numpy as np
 import torch
 
 from .clip import init_clip
+from .schedules import decayed_lr, ftrl_kernel_l2, init_lr
 
 _uid = itertools.count()
 
@@ -329,13 +330,15 @@ class Activation(Layer):
 
 # ---------------------------------------------------------------------------------------------
 # optimisers / losses (Keras formulas, kernels from libhrb200).  Every optimiser takes Keras' clipnorm / clipvalue /
-# global_clipnorm (handyrec_b200.clip); the model clips the gradients before it calls `step`.
+# global_clipnorm (handyrec_b200.clip); the model clips the gradients before it calls `step`.  `learning_rate` is a float or a
+# handyrec_b200.schedules schedule, `decay` Keras' time-based decay; `step` takes the rate of `iterations` (decayed_lr, kept in
+# `lr_t` for the large tables' row updates that follow it) and then counts itself there.
 # ---------------------------------------------------------------------------------------------
 class Adam:
     def __init__(self, learning_rate=1e-3, lr=None, beta_1=0.9, beta_2=0.999, epsilon=1e-7, clipnorm=None, clipvalue=None,
-                 global_clipnorm=None):
+                 global_clipnorm=None, decay=0.0):
         init_clip(self, clipnorm, clipvalue, global_clipnorm)
-        self.lr = float(lr if lr is not None else learning_rate)
+        init_lr(self, lr if lr is not None else learning_rate, decay)
         self.b1, self.b2, self.eps, self.t = beta_1, beta_2, epsilon, 0
         self.state: Dict[int, Tuple[torch.Tensor, torch.Tensor]] = {}
 
@@ -343,6 +346,7 @@ class Adam:
         from . import kernels as K
 
         self.t += 1
+        lr = self.lr_t = decayed_lr(self)
         ps, gs, ms, vs, l2s = [], [], [], [], []
         for p, l2 in params_l2:
             if p.grad is None or not p.requires_grad:
@@ -355,7 +359,8 @@ class Adam:
             ms.append(m)
             vs.append(v)
             l2s.append(2.0 * l2)
-        K.adam_step_multi(ps, gs, ms, vs, l2s, self.lr, self.b1, self.b2, self.eps, self.t)  # all variables in one launch
+        K.adam_step_multi(ps, gs, ms, vs, l2s, lr, self.b1, self.b2, self.eps, self.t)  # all variables in one launch
+        self.iterations += 1
 
 
 class Adagrad:
@@ -363,23 +368,25 @@ class Adagrad:
     initial_accumulator_value.  Large tables take the same step on the rows a batch touches (CustomEmbedding.apply_sparse)."""
 
     def __init__(self, learning_rate=0.001, initial_accumulator_value=0.1, epsilon=1e-7, lr=None, clipnorm=None, clipvalue=None,
-                 global_clipnorm=None):
+                 global_clipnorm=None, decay=0.0):
         init_clip(self, clipnorm, clipvalue, global_clipnorm)
         if initial_accumulator_value < 0.0:
             raise ValueError(f"initial_accumulator_value must be non-negative: {initial_accumulator_value}")
-        self.lr = float(lr if lr is not None else learning_rate)
+        init_lr(self, lr if lr is not None else learning_rate, decay)
         self.initial_accumulator_value, self.eps = float(initial_accumulator_value), float(epsilon)
         self.state: Dict[int, torch.Tensor] = {}
 
     def step(self, params_l2: Sequence[Tuple[torch.nn.Parameter, float]]):
         from . import kernels as K
 
+        lr = self.lr_t = decayed_lr(self)
         live = [(p, l2) for p, l2 in params_l2 if p.grad is not None and p.requires_grad]
         for p, _ in live:
             if id(p) not in self.state:
                 self.state[id(p)] = torch.full_like(p.data, self.initial_accumulator_value)
         K.adagrad_step_multi([p.data for p, _ in live], [p.grad.contiguous() for p, _ in live], [self.state[id(p)] for p, _ in live],
-                             [2.0 * l2 for _, l2 in live], self.lr, self.eps)  # all variables in one launch
+                             [2.0 * l2 for _, l2 in live], lr, self.eps)  # all variables in one launch
+        self.iterations += 1
 
 
 class Ftrl:
@@ -395,7 +402,7 @@ class Ftrl:
 
     def __init__(self, learning_rate=0.001, learning_rate_power=-0.5, initial_accumulator_value=0.1, l1_regularization_strength=0.0,
                  l2_regularization_strength=0.0, name="Ftrl", l2_shrinkage_regularization_strength=0.0, beta=0.0, lr=None,
-                 clipnorm=None, clipvalue=None, global_clipnorm=None):
+                 clipnorm=None, clipvalue=None, global_clipnorm=None, decay=0.0):
         init_clip(self, clipnorm, clipvalue, global_clipnorm)
         if initial_accumulator_value < 0.0:
             raise ValueError(f"initial_accumulator_value {initial_accumulator_value} needs to be positive or zero")
@@ -407,7 +414,6 @@ class Ftrl:
             raise ValueError(f"l2_regularization_strength {l2_regularization_strength} needs to be positive or zero")
         if l2_shrinkage_regularization_strength < 0.0:
             raise ValueError(f"l2_shrinkage_regularization_strength {l2_shrinkage_regularization_strength} needs to be positive or zero")
-        self.lr = float(lr if lr is not None else learning_rate)
         self.name = name
         self.learning_rate_power = float(learning_rate_power)
         self.initial_accumulator_value = float(initial_accumulator_value)
@@ -415,12 +421,13 @@ class Ftrl:
         self.l2 = float(l2_regularization_strength)
         self.l2_shrinkage = float(l2_shrinkage_regularization_strength)
         self.beta = float(beta)
+        init_lr(self, lr if lr is not None else learning_rate, decay)
         self.state: Dict[int, Tuple[torch.Tensor, torch.Tensor]] = {}
 
     @property
     def kernel_l2(self) -> float:
-        """The l2 the TF kernel takes: l2_regularization_strength + beta / (2 * learning_rate)."""
-        return self.l2 + self.beta / (2.0 * self.lr)
+        """The l2 the TF kernel takes: l2_regularization_strength + beta / (2 * learning_rate), at the rate of the current step."""
+        return ftrl_kernel_l2(self.l2, self.beta, self.lr_t)
 
     def hyper(self) -> Dict[str, float]:
         """Keyword arguments of the library's Ftrl entry points."""
@@ -429,24 +436,28 @@ class Ftrl:
     def step(self, params_l2: Sequence[Tuple[torch.nn.Parameter, float]]):
         from . import kernels as K
 
+        lr = self.lr_t = decayed_lr(self)
         live = [(p, l2) for p, l2 in params_l2 if p.grad is not None and p.requires_grad]
         for p, _ in live:
             if id(p) not in self.state:
                 self.state[id(p)] = (torch.full_like(p.data, self.initial_accumulator_value), torch.zeros_like(p.data))
         K.ftrl_step_multi([p.data for p, _ in live], [p.grad.contiguous() for p, _ in live], [self.state[id(p)][0] for p, _ in live],
-                          [self.state[id(p)][1] for p, _ in live], [2.0 * l2 for _, l2 in live], self.lr, **self.hyper())
+                          [self.state[id(p)][1] for p, _ in live], [2.0 * l2 for _, l2 in live], lr, **self.hyper())
+        self.iterations += 1
 
 
 class SGD:
-    def __init__(self, learning_rate=0.01, lr=None, clipnorm=None, clipvalue=None, global_clipnorm=None):
+    def __init__(self, learning_rate=0.01, lr=None, clipnorm=None, clipvalue=None, global_clipnorm=None, decay=0.0):
         init_clip(self, clipnorm, clipvalue, global_clipnorm)
-        self.lr = float(lr if lr is not None else learning_rate)
+        init_lr(self, lr if lr is not None else learning_rate, decay)
 
     def step(self, params_l2):
         from . import kernels as K
 
+        lr = self.lr_t = decayed_lr(self)
         live = [(p, l2) for p, l2 in params_l2 if p.grad is not None and p.requires_grad]
-        K.sgd_step_multi([p.data for p, _ in live], [p.grad.contiguous() for p, _ in live], [2.0 * l2 for _, l2 in live], self.lr)
+        K.sgd_step_multi([p.data for p, _ in live], [p.grad.contiguous() for p, _ in live], [2.0 * l2 for _, l2 in live], lr)
+        self.iterations += 1
 
 
 def binary_crossentropy(y_true, y_pred):

@@ -121,15 +121,16 @@ class CustomEmbedding(Layer):
             self._linear = torch.zeros_like(w) if ftrl else None
             self._plan = K.LookupPlan([w], [(0, 1, "none", 0, 0)], [self._m] if adam else None, [self._v] if adam else None,
                                       accum=[self._accum] if (adagrad or ftrl) else None, linear=[self._linear] if ftrl else None)
+        # lr_t: the rate of the step `optimizer.step` just applied (a schedule is evaluated once per step, there)
         if adam:
-            self._plan.backward_update(ids, rows, opt="adam", lr=optimizer.lr, l2_scale=2.0 * self.l2, beta1=optimizer.b1, beta2=optimizer.b2,
+            self._plan.backward_update(ids, rows, opt="adam", lr=optimizer.lr_t, l2_scale=2.0 * self.l2, beta1=optimizer.b1, beta2=optimizer.b2,
                                        eps=optimizer.eps, step=max(optimizer.t, 1), autotune=True)
         elif adagrad:
-            self._plan.backward_update(ids, rows, opt="adagrad", lr=optimizer.lr, l2_scale=2.0 * self.l2, eps=optimizer.eps, autotune=True)
+            self._plan.backward_update(ids, rows, opt="adagrad", lr=optimizer.lr_t, l2_scale=2.0 * self.l2, eps=optimizer.eps, autotune=True)
         elif ftrl:  # every gathered id is a plain-field position here: row 0 of mask_zero padding steps like any other row
-            self._plan.backward_update(ids, rows, opt="ftrl", lr=optimizer.lr, l2_scale=2.0 * self.l2, autotune=True, **optimizer.hyper())
+            self._plan.backward_update(ids, rows, opt="ftrl", lr=optimizer.lr_t, l2_scale=2.0 * self.l2, autotune=True, **optimizer.hyper())
         else:
-            self._plan.backward_update(ids, rows, opt="sgd", lr=optimizer.lr, l2_scale=2.0 * self.l2, autotune=True)
+            self._plan.backward_update(ids, rows, opt="sgd", lr=optimizer.lr_t, l2_scale=2.0 * self.l2, autotune=True)
 
     def compute_mask(self, inputs, mask=None):
         if not self.mask_zero:  # tools.py:94-95

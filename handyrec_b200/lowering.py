@@ -237,6 +237,7 @@ class FusedDeepFM:
         from .clip import clip_args
         from .engine import DeepFMEngine
         from .keras_lite import Adagrad, Adam, Ftrl, SGD
+        from .schedules import LearningRateSchedule, decayed_lr
 
         key = None
         if isinstance(optimizer, Adam):
@@ -252,9 +253,13 @@ class FusedDeepFM:
         else:
             raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD, keras_lite.Adagrad or keras_lite.Ftrl")
         clip = clip_args(optimizer)
-        key = (key or (opt, lr), clip)
+        # a schedule is keyed by the object, not a value: the engine takes the rate per step and is not rebuilt as it changes
+        key = (key or (opt, lr), clip, optimizer.decay)
+        # every step the engine issues sets its own rate (_lr_step); a schedule is evaluated there only, once per step
+        lr = None if isinstance(lr, LearningRateSchedule) else decayed_lr(optimizer)
         if self.engine is not None and self.engine.B >= batch_size and self._opt_key == key:
             self.engine.metrics = getattr(self.model, "_metric_set", None)
+            self.engine.lr_step = _lr_step(optimizer)
             return
         self.sync_to_layers()
         dev = torch.device("cuda", torch.cuda.current_device())
@@ -284,6 +289,7 @@ class FusedDeepFM:
         eng.fm_w.copy_(self.spec.fm.linear.data.reshape(-1).to(dev))
         eng.fm_w0.copy_(self.spec.fm.w_0.data.reshape(-1).to(dev))
         eng.step_count = getattr(optimizer, "t", 0)
+        eng.lr_step = _lr_step(optimizer)
         for t, lay in enumerate(self.tables):  # the layer and the engine share ONE copy of every table
             lay.embeddings.data = eng.tables[t]
         eng.metrics = getattr(self.model, "_metric_set", None)  # counted by train_step_on_device right after the loss
@@ -447,6 +453,20 @@ class FusedDeepFM:
         if eng.l2_embd and eng.dense_tables:
             tot += eng.l2_embd * float(sum((eng.tables[t] ** 2).sum() for t in eng.dense_tables))
         return tot
+
+
+def _lr_step(optimizer):
+    """The engine's per-step rate: Keras' _decayed_lr at the optimizer's `iterations`, which then counts the step.  Called once per
+    step the engine issues, so a later fit, rebuild or layer-path step continues the schedule; every rank of a multi-GPU model
+    issues the same steps and counts alike."""
+    from .schedules import decayed_lr
+
+    def step() -> float:
+        lr = optimizer.lr_t = decayed_lr(optimizer)
+        optimizer.iterations += 1
+        return lr
+
+    return step
 
 
 def lower(model) -> Optional[FusedDeepFM]:
