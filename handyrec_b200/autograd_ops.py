@@ -258,37 +258,44 @@ class AttPoolFn(torch.autograd.Function):
 
 
 class SigmoidBCEFn(torch.autograd.Function):
-    """mean sigmoid cross-entropy with logits (Keras binary_crossentropy on a sigmoid output uses the cached logits)."""
+    """mean sigmoid cross-entropy with logits (Keras binary_crossentropy on a sigmoid output uses the cached logits).  With
+    `weight` (one float32 per sample, on the device): Keras' weighted loss, sum(w * l) / B."""
 
     @staticmethod
-    def forward(ctx, logit, label):
+    def forward(ctx, logit, label, weight=None):
         logit = logit.contiguous().reshape(-1)
         label = label.contiguous().reshape(-1).to(torch.float32)
         B = logit.numel()
         dl = torch.empty_like(logit)
         ls = torch.zeros(1, device=logit.device, dtype=torch.float32)
-        K.sigmoid_bce(logit, None, label, 1.0 / B, None, dl, ls)
+        K.sigmoid_bce(logit, None, label, 1.0 / B, None, dl, ls, weight=weight)
         ctx.save_for_backward(dl)
         return (ls / B).reshape(())
 
     @staticmethod
     def backward(ctx, g):
         (dl,) = ctx.saved_tensors
-        return (dl * g).reshape(-1, 1), None
+        return (dl * g).reshape(-1, 1), None, None
 
 
 class ClippedBCEFn(torch.autograd.Function):
-    """mean binary cross-entropy on probabilities clipped to [1e-7, 1-1e-7] (Keras' path without cached logits)."""
+    """mean binary cross-entropy on probabilities clipped to [1e-7, 1-1e-7] (Keras' path without cached logits).  With `weight`:
+    sum(w * l) / n, as SigmoidBCEFn."""
 
     @staticmethod
-    def forward(ctx, prob, label):
+    def forward(ctx, prob, label, weight=None):
         shape = prob.shape
         prob = prob.contiguous().reshape(-1)
         label = label.contiguous().reshape(-1).to(torch.float32)
         n = prob.numel()
         dp = torch.empty_like(prob)
         ls = torch.zeros(1, device=prob.device, dtype=torch.float32)
-        call("hrb_clipped_bce", K._p(prob), K._p(label), n, 1e-7, 1.0 / n, K._p(dp), K._p(ls), K._stream())
+        if weight is None:
+            call("hrb_clipped_bce", K._p(prob), K._p(label), n, 1e-7, 1.0 / n, K._p(dp), K._p(ls), K._stream())
+        else:
+            if K._chk(weight, torch.float32, "weight").numel() != n:
+                raise ValueError(f"binary_crossentropy: {weight.numel()} sample weights for {n} predictions")
+            call("hrb_clipped_bce_weighted", K._p(prob), K._p(label), K._p(weight), n, 1e-7, 1.0 / n, K._p(dp), K._p(ls), K._stream())
         ctx.save_for_backward(dp)
         ctx.shape = shape
         return (ls / n).reshape(())
@@ -296,7 +303,7 @@ class ClippedBCEFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         (dp,) = ctx.saved_tensors
-        return (dp * g).reshape(ctx.shape), None
+        return (dp * g).reshape(ctx.shape), None, None
 
 
 class ActivationFn(torch.autograd.Function):

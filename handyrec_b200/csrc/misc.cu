@@ -7,9 +7,12 @@
 
 namespace hrb {
 
+// WEIGHTED: Keras' sample weights enter at the loss, loss_sum += w*l and dlogit = (p-y)*w*grad_scale; w = 1 leaves every bit of
+// prob and dlogit as the unweighted instantiation computes them
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(256) sigmoid_bce_kernel(const float* __restrict__ dnn, const float* __restrict__ fmv,
-                                                         const float* __restrict__ label, int64_t batch,
-                                                         float grad_scale, float* __restrict__ prob,
+                                                         const float* __restrict__ label, const float* __restrict__ weight,
+                                                         int64_t batch, float grad_scale, float* __restrict__ prob,
                                                          float* __restrict__ dlogit, float* __restrict__ loss_sum) {
   __shared__ float red[8];
   float local = 0.f;
@@ -18,9 +21,16 @@ __global__ void __launch_bounds__(256) sigmoid_bce_kernel(const float* __restric
     const float p = sigmoidf_(z);
     const float y = label[i];
     // max(z,0) - z*y + log1p(exp(-|z|))  (tf.nn.sigmoid_cross_entropy_with_logits)
-    local += fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
+    const float l = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
     if (prob != nullptr) prob[i] = p;
-    if (dlogit != nullptr) dlogit[i] = (p - y) * grad_scale;
+    if constexpr (WEIGHTED) {
+      const float w = weight[i];
+      local += w * l;
+      if (dlogit != nullptr) dlogit[i] = (p - y) * w * grad_scale;
+    } else {
+      local += l;
+      if (dlogit != nullptr) dlogit[i] = (p - y) * grad_scale;
+    }
   }
   local = warp_sum(local);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = local;
@@ -34,16 +44,23 @@ __global__ void __launch_bounds__(256) sigmoid_bce_kernel(const float* __restric
 }
 
 // Keras binary_crossentropy on PROBABILITIES (no cached logits): p is clipped to [eps, 1-eps]; the gradient of the clip is 0 outside
-__global__ void __launch_bounds__(256) clipped_bce_kernel(const float* __restrict__ prob, const float* __restrict__ label, int64_t n,
-                                                         float eps, float grad_scale, float* __restrict__ dprob,
-                                                         float* __restrict__ loss_sum) {
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(256) clipped_bce_kernel(const float* __restrict__ prob, const float* __restrict__ label,
+                                                         const float* __restrict__ weight, int64_t n, float eps, float grad_scale,
+                                                         float* __restrict__ dprob, float* __restrict__ loss_sum) {
   __shared__ float red[8];
   float local = 0.f;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const float p0 = prob[i], y = label[i];
     const float p = fminf(fmaxf(p0, eps), 1.0f - eps);
-    local -= y * logf(p) + (1.0f - y) * logf(1.0f - p);
-    if (dprob != nullptr) dprob[i] = (p0 >= eps && p0 <= 1.0f - eps) ? ((1.0f - y) / (1.0f - p) - y / p) * grad_scale : 0.f;
+    if constexpr (WEIGHTED) {
+      const float w = weight[i];
+      local -= w * (y * logf(p) + (1.0f - y) * logf(1.0f - p));
+      if (dprob != nullptr) dprob[i] = (p0 >= eps && p0 <= 1.0f - eps) ? ((1.0f - y) / (1.0f - p) - y / p) * w * grad_scale : 0.f;
+    } else {
+      local -= y * logf(p) + (1.0f - y) * logf(1.0f - p);
+      if (dprob != nullptr) dprob[i] = (p0 >= eps && p0 <= 1.0f - eps) ? ((1.0f - y) / (1.0f - p) - y / p) * grad_scale : 0.f;
+    }
   }
   local = warp_sum(local);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = local;
@@ -299,8 +316,18 @@ HRB_API int hrb_sigmoid_bce(const float* dnn_logit, const float* fm_logit, const
                             float grad_scale, float* prob, float* dlogit, float* loss_sum, void* stream) {
   HRB_REQUIRE(dnn_logit && label && batch >= 0, "hrb_sigmoid_bce: null/negative argument");
   if (batch == 0) return HRB_OK;
-  sigmoid_bce_kernel<<<ew_grid(batch), 256, 0, (cudaStream_t)stream>>>(dnn_logit, fm_logit, label, batch, grad_scale, prob,
-                                                                      dlogit, loss_sum);
+  sigmoid_bce_kernel<false><<<ew_grid(batch), 256, 0, (cudaStream_t)stream>>>(dnn_logit, fm_logit, label, nullptr, batch, grad_scale,
+                                                                             prob, dlogit, loss_sum);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+HRB_API int hrb_sigmoid_bce_weighted(const float* dnn_logit, const float* fm_logit, const float* label, const float* weight,
+                                     int64_t batch, float grad_scale, float* prob, float* dlogit, float* loss_sum, void* stream) {
+  HRB_REQUIRE(dnn_logit && label && weight && batch >= 0, "hrb_sigmoid_bce_weighted: null/negative argument");
+  if (batch == 0) return HRB_OK;
+  sigmoid_bce_kernel<true><<<ew_grid(batch), 256, 0, (cudaStream_t)stream>>>(dnn_logit, fm_logit, label, weight, batch, grad_scale,
+                                                                            prob, dlogit, loss_sum);
   HRB_LAUNCH_CHECK();
   return HRB_OK;
 }
@@ -309,7 +336,16 @@ HRB_API int hrb_clipped_bce(const float* prob, const float* label, int64_t n, fl
                             float* loss_sum, void* stream) {
   HRB_REQUIRE(prob && label && n >= 0, "hrb_clipped_bce: null/negative argument");
   if (n == 0) return HRB_OK;
-  clipped_bce_kernel<<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(prob, label, n, eps, grad_scale, dprob, loss_sum);
+  clipped_bce_kernel<false><<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(prob, label, nullptr, n, eps, grad_scale, dprob, loss_sum);
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+HRB_API int hrb_clipped_bce_weighted(const float* prob, const float* label, const float* weight, int64_t n, float eps, float grad_scale,
+                                     float* dprob, float* loss_sum, void* stream) {
+  HRB_REQUIRE(prob && label && weight && n >= 0, "hrb_clipped_bce_weighted: null/negative argument");
+  if (n == 0) return HRB_OK;
+  clipped_bce_kernel<true><<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(prob, label, weight, n, eps, grad_scale, dprob, loss_sum);
   HRB_LAUNCH_CHECK();
   return HRB_OK;
 }

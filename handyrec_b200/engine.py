@@ -490,8 +490,11 @@ class DeepFMEngine:
         call("hrb_sigmoid_bce", K._p(self.A[-1]), K._p(self.fm_out), K._p(self.label_dev), B, 0.0, K._p(self.prob), None, None, K._stream())
         return self.prob[:B]
 
-    def train_step_on_device(self, ids: torch.Tensor, dense: Optional[torch.Tensor], label: torch.Tensor) -> None:
-        """One full step: forward, BCE, backward, embedding row updates, dense optimiser.  Loss sum -> self.loss_sum."""
+    def train_step_on_device(self, ids: torch.Tensor, dense: Optional[torch.Tensor], label: torch.Tensor,
+                             weight: Optional[torch.Tensor] = None) -> None:
+        """One full step: forward, BCE, backward, embedding row updates, dense optimiser.  Loss sum -> self.loss_sum.  `weight`
+        (B float32, Keras' sample weights): the loss sum becomes sum(w * l) and dlogit w * (p - y) / (B * ranks), and the weighted
+        metrics sum the weights; everything after dlogit runs unchanged."""
         B = ids.shape[0]
         st = K._stream()
         self.step_count += 1
@@ -500,10 +503,14 @@ class DeepFMEngine:
         self.forward(ids, dense, training=True)
         self.loss_sum.zero_()
         dlogit = self.dZ[-1]  # (B, 1): the logit layer has one unit (DeepFM.py:59-60)
-        call("hrb_sigmoid_bce", K._p(self.A[-1]), K._p(self.fm_out), K._p(label), B, 1.0 / (B * self.grad_scale_div), K._p(self.prob), K._p(dlogit), K._p(self.loss_sum), st)
+        if weight is None:
+            call("hrb_sigmoid_bce", K._p(self.A[-1]), K._p(self.fm_out), K._p(label), B, 1.0 / (B * self.grad_scale_div), K._p(self.prob), K._p(dlogit), K._p(self.loss_sum), st)
+        else:
+            call("hrb_sigmoid_bce_weighted", K._p(self.A[-1]), K._p(self.fm_out), K._p(label), K._p(weight), B, 1.0 / (B * self.grad_scale_div),
+                 K._p(self.prob), K._p(dlogit), K._p(self.loss_sum), st)
         self._mark("sigmoid_bce")
         if self.metrics is not None:  # Keras counts its metrics from the training forward, before the weight update
-            self.metrics.update(self.prob[:B], label)
+            self.metrics.update(self.prob[:B], label, weight)
             self._mark("metric_update")
         self._backward(ids, B, st)
 
@@ -663,22 +670,36 @@ class DeepFMEngine:
     # ------------------------------------------------------------------------------------------
     # public, host-facing API (what Model.train_on_batch / predict call)
     # ------------------------------------------------------------------------------------------
-    def train_on_batch(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor], label_host: torch.Tensor) -> float:
-        """Host (pinned) tensors in, mean BCE loss out.  Includes the H2D copies and a D2H read of the loss."""
+    _weight_dev: Optional[torch.Tensor] = None  # the sample weights of train_on_batch / predict, allocated at the first weighted call
+
+    def _weights_to_device(self, weight_host: Optional[torch.Tensor], B: int) -> Optional[torch.Tensor]:
+        if weight_host is None:
+            return None
+        if self._weight_dev is None:
+            self._weight_dev = torch.zeros(self.B, device=self.dev, dtype=torch.float32)
+        self._weight_dev[:B].copy_(weight_host, non_blocking=True)
+        return self._weight_dev[:B]
+
+    def train_on_batch(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor], label_host: torch.Tensor,
+                       weight_host: Optional[torch.Tensor] = None) -> float:
+        """Host (pinned) tensors in, mean BCE loss out (with `weight_host`: sum(w * l) / B).  Includes the H2D copies and a D2H
+        read of the loss."""
         B = ids_host.shape[0]
         self.ids_dev[:B].copy_(ids_host, non_blocking=True)
         if self.n_dense:
             self.dense_dev[:B].copy_(dense_host, non_blocking=True)
         self.label_dev[:B].copy_(label_host, non_blocking=True)
-        self.train_step_on_device(self.ids_dev[:B], self.dense_dev[:B] if self.n_dense else None, self.label_dev[:B])
+        weight = self._weights_to_device(weight_host, B)
+        self.train_step_on_device(self.ids_dev[:B], self.dense_dev[:B] if self.n_dense else None, self.label_dev[:B], weight)
         self.loss_host.copy_(self.loss_sum, non_blocking=True)
         torch.cuda.current_stream().synchronize()
         return float(self.loss_host[0]) / B
 
     def fit_batches(self, batches) -> List[float]:
-        """Keras-`fit`-like loop over host batches `(ids, dense, label)` (pinned tensors) with input prefetch:
-        the H2D copies of batch t+1 run on a copy stream while batch t computes, and every step's loss is copied
-        back asynchronously; the host waits once, at the end.  Returns the per-step mean losses."""
+        """Keras-`fit`-like loop over host batches `(ids, dense, label)` or `(ids, dense, label, weight)` (pinned tensors; weight
+        None or Keras' sample weights) with input prefetch: the H2D copies of batch t+1 run on a copy stream while batch t
+        computes, and every step's loss is copied back asynchronously; the host waits once, at the end.  Returns the per-step
+        mean losses."""
         main = torch.cuda.current_stream()
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream()
@@ -696,8 +717,12 @@ class DeepFMEngine:
 
         def upload(slot, batch):
             packed = batch if hasattr(batch, "views") else None  # lowering.HostBatch: a reusable pinned slot
-            ids_h, dense_h, label_h = packed.views() if packed is not None else batch
+            ids_h, dense_h, label_h, *weight_h = packed.views() if packed is not None else batch
+            weight_h = weight_h[0] if weight_h else None
             B = ids_h.shape[0]
+            if weight_h is not None and getattr(self, "_stage_w", None) is None:  # staged next to the label, from the first weighted batch
+                self._stage_w = [torch.zeros(self.B, device=self.dev, dtype=torch.float32) for _ in range(2)]
+            weighted[slot] = weight_h is not None
             with torch.cuda.stream(self._copy_stream):
                 self._copy_stream.wait_event(self._stage_free[slot])  # the previous user of this slot has finished
                 ids_d, dense_d, label_d = self._stage[slot]
@@ -705,12 +730,15 @@ class DeepFMEngine:
                 if self.n_dense:
                     dense_d[:B].copy_(dense_h[:, : self.n_dense], non_blocking=True)
                 label_d[:B].copy_(label_h, non_blocking=True)
+                if weight_h is not None:
+                    self._stage_w[slot][:B].copy_(weight_h, non_blocking=True)
                 self._stage_ready[slot].record(self._copy_stream)
                 if packed is not None:  # the producer may refill the pinned slot once these copies have left it
                     packed.copied = torch.cuda.Event()
                     packed.copied.record(self._copy_stream)
             return B
 
+        weighted = [False, False]
         for e in self._stage_free:
             e.record(main)
         nxt = next(it, None)
@@ -721,7 +749,8 @@ class DeepFMEngine:
             cur_slot, B = slot, nB
             main.wait_event(self._stage_ready[cur_slot])
             ids_d, dense_d, label_d = self._stage[cur_slot]
-            self.train_step_on_device(ids_d[:B], dense_d[:B] if self.n_dense else None, label_d[:B])
+            self.train_step_on_device(ids_d[:B], dense_d[:B] if self.n_dense else None, label_d[:B],
+                                      self._stage_w[cur_slot][:B] if weighted[cur_slot] else None)
             self._stage_free[cur_slot].record(main)
             k = len(losses_host) % 256
             if k == 0:
@@ -743,17 +772,20 @@ class DeepFMEngine:
         return [float(l[0]) / b for l, b in zip(losses_host, sizes)]
 
     def predict(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor], label_host: Optional[torch.Tensor] = None,
-                metrics=None) -> torch.Tensor:
-        """Probabilities of one host batch; with `metrics` (a MetricSet) and the batch's labels, also counts them (one launch)."""
+                metrics=None, weight_host: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Probabilities of one host batch; with `metrics` (a MetricSet) and the batch's labels, also counts them (one launch; with
+        the batch's sample weights `weight_host`, the weighted update)."""
         B = ids_host.shape[0]
         self.ids_dev[:B].copy_(ids_host, non_blocking=True)
         if self.n_dense:
             self.dense_dev[:B].copy_(dense_host, non_blocking=True)
+        weight = None
         if metrics is not None:
             self.label_dev[:B].copy_(label_host, non_blocking=True)
+            weight = self._weights_to_device(weight_host, B)
         prob = self.predict_on_device(self.ids_dev[:B], self.dense_dev[:B] if self.n_dense else None)
         if metrics is not None:
-            metrics.update(prob, self.label_dev[:B])
+            metrics.update(prob, self.label_dev[:B], weight)
         return prob.cpu().reshape(B, 1)
 
     def h2d_bytes_per_step(self, B: int) -> int:

@@ -460,7 +460,12 @@ class SGD:
         self.iterations += 1
 
 
+_step_weight: Optional[torch.Tensor] = None  # the sample weights of the batch a Model step is computing (device float32), or None
+
+
 def binary_crossentropy(y_true, y_pred):
+    """Keras binary_crossentropy, the mean over the batch.  Inside a Model step with sample weights it is Keras' weighted loss
+    sum(w * l) / B: the model hands the batch's weights over in `_step_weight`, as Keras' compiled loss adds them to the call."""
     from .autograd_ops import SigmoidBCEFn
 
     logits = getattr(y_pred, "_keras_logits", None)
@@ -469,8 +474,45 @@ def binary_crossentropy(y_true, y_pred):
         # output activation, layers/core.py:66-73): probabilities clipped to [eps, 1-eps], eps = 1e-7
         from .autograd_ops import ClippedBCEFn
 
-        return ClippedBCEFn.apply(y_pred, y_true)
-    return SigmoidBCEFn.apply(logits, y_true)
+        return ClippedBCEFn.apply(y_pred, y_true, _step_weight)
+    return SigmoidBCEFn.apply(logits, y_true, _step_weight)
+
+
+def _as_host(a) -> np.ndarray:
+    return a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+
+
+def sample_weights(y, sample_weight=None, class_weight=None) -> Optional[np.ndarray]:
+    """Keras 2.6's per-sample weights of labels `y`: `sample_weight` ((n,) or (n, 1)) times the `class_weight` entry of each label
+    (data_adapter._make_class_weight_map_fn: keys exactly 0..k-1, labels truncated to int64), the product formed in float64 and
+    rounded once to float32.  None when neither is given.  Raises ValueError on a bad shape, length, key set or label."""
+    if sample_weight is None and class_weight is None:
+        return None
+    yv = _as_host(y)
+    n = len(yv)
+    w = None
+    if sample_weight is not None:
+        sw = _as_host(sample_weight)
+        if not (sw.ndim == 1 or (sw.ndim == 2 and sw.shape[1] == 1)) or sw.shape[0] != n:
+            raise ValueError(f"sample_weight must have shape ({n},) or ({n}, 1) for {n} labels, got {sw.shape}")
+        w = sw.reshape(-1).astype(np.float64)
+    if class_weight is not None:
+        class_ids = sorted(class_weight.keys())
+        if class_ids != list(range(len(class_ids))):
+            raise ValueError("Expected `class_weight` to be a dict with keys from 0 to one less than the number of classes, "
+                             f"found {class_weight}")
+        if yv.ndim == 2 and yv.shape[1] > 1:
+            raise NotImplementedError("class_weight with one-hot targets: the models here have a single binary output")
+        table = np.array([class_weight[int(c)] for c in class_ids], dtype=np.float32).astype(np.float64)
+        yf = yv.reshape(-1).astype(np.float64)
+        bad = ~((yf > -1.0) & (yf < len(class_ids)))  # int64 truncation lands outside 0..k-1 (NaN included)
+        if bad.any():
+            i = int(np.flatnonzero(bad)[0])
+            raise ValueError(f"class_weight: label {yv.reshape(-1)[i]} of sample {i} is not one of the classes 0..{len(class_ids) - 1} "
+                             "after truncation to int64")
+        cw = table[np.trunc(yf).astype(np.int64)]
+        w = cw if w is None else w * cw
+    return w.astype(np.float32)
 
 
 class Model:
@@ -603,17 +645,21 @@ class Model:
     _metric_set = None  # handyrec_b200.metrics.MetricSet of the compiled metrics, None without
     _metric_list: Sequence = ()
 
-    def compile(self, optimizer=None, loss=None, distribute=None, metrics=None, **kwargs):
+    def compile(self, optimizer=None, loss=None, distribute=None, metrics=None, weighted_metrics=None, **kwargs):
         """keras.Model.compile.  `distribute` (extra): True under an initialised torch.distributed process group (one process per
         GPU), or a `handyrec_b200.sharded.TorchDistComm` -- a DeepFM-shaped graph then trains on the row-sharded multi-GPU engine.
         `metrics`: AUC / Precision / Recall / BinaryAccuracy objects or the strings "AUC", "Precision", "Recall", "accuracy", "acc",
-        "binary_accuracy" (handyrec_b200.metrics; counted on the GPU from each batch's forward output)."""
+        "binary_accuracy" (handyrec_b200.metrics; counted on the GPU from each batch's forward output).  `weighted_metrics`: the
+        same, counted with the sample weights of fit / train_on_batch / evaluate (a name an unweighted metric has becomes
+        `weighted_<name>`)."""
         from . import metrics as M
 
-        if kwargs.get("weighted_metrics"):
-            raise NotImplementedError("weighted_metrics: sample weights are not supported")
-        self._metric_list = M.from_compile(metrics)
-        self._metric_set = M.MetricSet(self._metric_list) if self._metric_list else None
+        if kwargs.get("sample_weight_mode") is not None:
+            raise NotImplementedError("sample_weight_mode: only per-sample weights are supported (no temporal weights)")
+        if weighted_metrics:
+            self._require_one_probability("weighted_metrics")
+        self._metric_list, weighted = M.from_compile(metrics, weighted_metrics)
+        self._metric_set = M.MetricSet(self._metric_list, weighted) if self._metric_list else None
         self.optimizer = optimizer if optimizer is not None else Adam()
         self.loss = loss if loss is not None else binary_crossentropy
         self._fused = None
@@ -681,36 +727,60 @@ class Model:
 
     def train_on_batch(self, x, y, sample_weight=None, class_weight=None, reset_metrics=True, return_dict=False):
         """keras.Model.train_on_batch: the loss, or [loss, *metric results] when metrics are compiled (a dict with return_dict).
-        reset_metrics=False accumulates the metrics over calls."""
-        from .metrics import _no_sample_weight
-
-        _no_sample_weight(sample_weight)
-        if class_weight is not None:
-            raise NotImplementedError("class_weight is not supported")
+        reset_metrics=False accumulates the metrics over calls.  sample_weight / class_weight: Keras' per-sample weights."""
+        w = self._weights(y, sample_weight, class_weight)
         if self._metric_set is None and not return_dict:
-            return self._train_step(x, y)
+            return self._train_step(x, y, w)
         if reset_metrics:
             self.reset_metrics()
-        loss = self._train_step(x, y)
+        loss = self._train_step(x, y, w)
         return self._with_metrics(loss, self._metric_values() if self._metric_set is not None else {}, return_dict)
 
-    def _train_step(self, x, y) -> float:
+    def _weights(self, y, sample_weight=None, class_weight=None) -> Optional[np.ndarray]:
+        """sample_weights(), refused for a loss other than binary_crossentropy and for an output other than one probability per
+        sample."""
+        w = sample_weights(y, sample_weight, class_weight)
+        if w is not None:
+            if self.loss is not binary_crossentropy:
+                raise NotImplementedError(f"sample_weight / class_weight are supported with binary_crossentropy only, not {self.loss!r}")
+            self._require_one_probability("sample_weight / class_weight")
+        return w
+
+    def _require_one_probability(self, what: str) -> None:
+        """Sample weights are one number per sample: the model must have a single output of shape (batch, 1), the binary models'
+        probability (a wider or multi-output model would need Keras' broadcasting of the weights over its columns)."""
+        out = self.outputs
+        if not isinstance(out, KTensor) or tuple(out.shape[1:]) != (1,):
+            shape = out.shape if isinstance(out, KTensor) else [getattr(o, "shape", None) for o in _flatten(out)]
+            raise NotImplementedError(f"{what}: supported for a model with one output of shape (batch, 1), not {shape}")
+
+    def _train_step(self, x, y, weight: Optional[np.ndarray] = None) -> float:
         if self._fused is not None and isinstance(x, dict):
             n = len(np.asarray(next(iter(x.values()))))
             self._fused.build(n, self.optimizer)
-            return self._fused.train_on_batch(x, y) + self._fused.reg_loss()
+            return self._fused.train_on_batch(x, y, weight) + self._fused.reg_loss()
         self.sync()
         from .kernels import deferred_id_checks
 
         with deferred_id_checks():  # the lookups' out-of-range flags are read once, with the loss, instead of one host sync per lookup
-            return self._train_on_batch_layers(x, y)
+            return self._train_on_batch_layers(x, y, weight)
 
-    def _train_on_batch_layers(self, x, y) -> float:
+    def _weighted_loss(self, yt: torch.Tensor, out, wt: Optional[torch.Tensor]):
+        """self.loss(yt, out), with the batch's sample weights handed to binary_crossentropy."""
+        global _step_weight
+        _step_weight = wt
+        try:
+            return self.loss(yt, out)
+        finally:
+            _step_weight = None
+
+    def _train_on_batch_layers(self, x, y, weight: Optional[np.ndarray] = None) -> float:
         out = self(x, training=True)
         yt = torch.as_tensor(np.asarray(y), dtype=torch.float32).to(device()) if not isinstance(y, torch.Tensor) else y.to(device())
-        loss = self.loss(yt, out)
+        wt = torch.from_numpy(weight).to(device()) if weight is not None else None
+        loss = self._weighted_loss(yt, out, wt)
         if self._metric_set is not None:  # Keras updates the metrics from the training forward, before the weight update
-            self._metric_set.update(out, yt)
+            self._metric_set.update(out, yt, wt)
         params = self.weights_with_l2()
         for p, _ in params:
             p.grad = None
@@ -806,14 +876,19 @@ class Model:
             if fn:
                 fn()
 
-    def fit(self, x=None, y=None, batch_size=32, epochs=1, validation_data=None, verbose=0, **kwargs):
-        from .metrics import _no_sample_weight
-
-        _no_sample_weight(kwargs.get("sample_weight"))
+    def fit(self, x=None, y=None, batch_size=32, epochs=1, validation_data=None, verbose=0, sample_weight=None, class_weight=None,
+            **kwargs):
+        """keras.Model.fit over a dict of arrays (+ y), an `(x, y)` / `(x, y, sample_weight)` tuple, or an iterable of such batches.
+        sample_weight / class_weight: Keras' per-sample weights of the training data (folded into one float32 weight per sample
+        once per fit); validation_data may be `(x, y, sample_weight)`."""
         history = {"loss": []}
-        if isinstance(x, tuple) and len(x) == 2 and isinstance(x[0], dict) and y is None:
-            x, y = x
-        batches = _batches(x, y, batch_size)
+        if isinstance(x, tuple) and len(x) in (2, 3) and isinstance(x[0], dict) and y is None:
+            x, y, *rest = x
+            sample_weight = rest[0] if rest else sample_weight
+        weight = self._weights(y, sample_weight, class_weight) if isinstance(x, dict) else None
+        if not isinstance(x, dict) and sample_weight is not None:
+            raise ValueError("sample_weight with an iterable of batches: yield (x, y, sample_weight) batches instead")
+        batches = _batches(x, y, batch_size, weight, class_weight=class_weight, model=self)
         for _ in range(epochs):
             self.reset_metrics()  # Keras resets the metrics at the start of every epoch
             if self._fused is not None and isinstance(x, dict):
@@ -821,15 +896,15 @@ class Model:
                 # runs on the fused engine with asynchronous loss read-back (lowering.FusedDeepFM.fit_epoch)
                 n = len(np.asarray(next(iter(x.values()))))
                 self._fused.build(min(batch_size, n), self.optimizer)
-                losses = self._fused.fit_epoch(x, y, batch_size)
+                losses = self._fused.fit_epoch(x, y, batch_size, weight)
                 sizes = [min(batch_size, n - s) for s in range(0, n, batch_size)]
                 history["loss"].append(float(np.average(losses, weights=sizes)) + self._fused.reg_loss())
                 self.last_losses = losses
             else:
                 tot, cnt = 0.0, 0
-                for xb, yb in batches():  # Keras reports the sample-weighted running mean of the batch losses
+                for xb, yb, wb in batches():  # Keras reports the sample-weighted running mean of the batch losses
                     nb = len(yb) if hasattr(yb, "__len__") else 1
-                    tot += self._train_step(xb, yb) * nb
+                    tot += self._train_step(xb, yb, wb) * nb
                     cnt += nb
                 history["loss"].append(tot / max(cnt, 1))
             if self._metric_set is not None:
@@ -851,26 +926,30 @@ class Model:
         return h
 
     def _evaluate_pass(self, data, batch_size: int):
-        """The validation pass of `fit` and the body of `evaluate`: (loss, metric results), the metrics reset first."""
+        """The validation pass of `fit` and the body of `evaluate`: (loss, metric results), the metrics reset first.  `data`: `(x, y)`,
+        `(x, y, sample_weight)` or an iterable of such batches."""
         ms = self._metric_set
         self.reset_metrics()
-        fused_val = (self._fused is not None and self._fused.engine is not None and isinstance(data, tuple) and len(data) == 2
+        fused_val = (self._fused is not None and self._fused.engine is not None and isinstance(data, tuple) and len(data) in (2, 3)
                      and isinstance(data[0], dict))
         if fused_val:
             # the fused engine's forward (the only reader a row-sharded table has); Keras' BCE on clipped probabilities
-            xv, yv = data
-            p = np.clip(self._fused.predict(xv, batch_size, y=yv, metrics=ms).reshape(-1).astype(np.float64), 1e-7, 1.0 - 1e-7)
+            xv, yv = data[:2]
+            w = self._weights(yv, data[2]) if len(data) == 3 else None
+            p = np.clip(self._fused.predict(xv, batch_size, y=yv, metrics=ms, weight=w).reshape(-1).astype(np.float64), 1e-7, 1.0 - 1e-7)
             yt = np.asarray(yv, dtype=np.float64).reshape(-1)
-            loss = float(-(yt * np.log(p) + (1.0 - yt) * np.log1p(-p)).mean())
+            l = -(yt * np.log(p) + (1.0 - yt) * np.log1p(-p))
+            loss = float((l if w is None else w.astype(np.float64) * l).mean())
         else:
             vl, vc = 0.0, 0
             with torch.no_grad():
-                for xb, yb in _batches(data, None, batch_size)():
+                for xb, yb, wb in _batches(data, None, batch_size, model=self)():
                     out = self(xb, training=False)
                     yt = torch.as_tensor(np.asarray(yb), dtype=torch.float32).to(device())
-                    vl += float(self.loss(yt, out))
+                    wt = torch.from_numpy(wb).to(device()) if wb is not None else None
+                    vl += float(self._weighted_loss(yt, out, wt))
                     if ms is not None:
-                        ms.update(out, yt)
+                        ms.update(out, yt, wt)
                     vc += 1
             loss = vl / max(vc, 1)
         return loss, (self._metric_values() if ms is not None else OrderedDict())
@@ -878,10 +957,13 @@ class Model:
     def evaluate(self, x=None, y=None, batch_size=None, verbose=0, sample_weight=None, steps=None, callbacks=None, return_dict=False,
                  **kwargs):
         """keras.Model.evaluate: the loss, or [loss, *metric results] when metrics are compiled (a dict with return_dict).  The
-        loss is what `fit(validation_data=(x, y), batch_size=batch_size)` records as val_loss on the same path."""
-        from .metrics import _no_sample_weight
-
-        _no_sample_weight(sample_weight)
+        loss is what `fit(validation_data=(x, y), batch_size=batch_size)` records as val_loss on the same path.  Sample weights
+        come with the data, as `validation_data` takes them: `evaluate((x, y, sample_weight))` or an iterable of
+        `(x, y, sample_weight)` batches (the same val_loss as `validation_data=(x, y, sample_weight)`); the `sample_weight`
+        keyword is not supported (NotImplementedError)."""
+        if sample_weight is not None:
+            raise NotImplementedError("evaluate(sample_weight=...): pass the weights with the data, evaluate((x, y, sample_weight)) or "
+                                      "an iterable of (x, y, sample_weight) batches")
         bs = batch_size or 32
         data = x if (y is None and not isinstance(x, dict)) else (x, y)
         if (self._fused is not None and self._fused.engine is None and isinstance(data, tuple) and isinstance(data[0], dict)
@@ -903,21 +985,26 @@ def _all_sublayers(l: Layer) -> List[Layer]:
     return out
 
 
-def _batches(x, y, batch_size):
-    """x: dict of arrays (+ y), or an iterable of (dict, label) batches (what tf.data yields in the reference tests)."""
+def _batches(x, y, batch_size, weight: Optional[np.ndarray] = None, class_weight=None, model: Optional[Model] = None):
+    """x: dict of arrays (+ y, + the float32 sample weights `weight`), an (x, y) or (x, y, sample_weight) tuple, or an iterable of
+    (dict, label) or (dict, label, sample_weight) batches (what tf.data yields in the reference tests).  Yields (x, y, weight or
+    None) batches; the weights of a tuple or of a batch are checked and class_weight folded in by model._weights."""
+    fold = (lambda yy, sw: model._weights(yy, sw, class_weight)) if model is not None else (lambda yy, sw: None)
 
     def gen():
         if isinstance(x, dict):
             n = len(next(iter(x.values())))
             for s in range(0, n, batch_size):
-                yield {k: v[s : s + batch_size] for k, v in x.items()}, y[s : s + batch_size]
-        elif isinstance(x, tuple) and len(x) == 2 and isinstance(x[0], dict):
-            xd, yd = x
+                yield {k: v[s : s + batch_size] for k, v in x.items()}, y[s : s + batch_size], (weight[s : s + batch_size] if weight is not None else None)
+        elif isinstance(x, tuple) and len(x) in (2, 3) and isinstance(x[0], dict):
+            xd, yd = x[:2]
+            wd = fold(yd, x[2]) if len(x) == 3 else None
             n = len(next(iter(xd.values())))
             for s in range(0, n, batch_size):
-                yield {k: v[s : s + batch_size] for k, v in xd.items()}, yd[s : s + batch_size]
+                yield {k: v[s : s + batch_size] for k, v in xd.items()}, yd[s : s + batch_size], (wd[s : s + batch_size] if wd is not None else None)
         else:
-            for xb, yb in x:
-                yield xb, yb
+            for batch in x:
+                xb, yb, *swb = batch
+                yield xb, yb, fold(yb, swb[0] if swb else None)
 
     return gen

@@ -18,7 +18,8 @@ __all__ = [
     "init_uniform", "embedding_fwd", "embedding_bwd_dense", "seq_pool_fwd", "seq_pool_bwd", "LookupPlan",
     "fm_fwd", "fm_bwd", "dense_fwd", "dense_bwd_x", "dense_bwd_w", "act_bwd", "dice_fwd", "dice_bwd",
     "lau_fwd", "lau_pack_params", "sigmoid_bce", "adam_step", "sgd_step", "adam_step_multi", "sgd_step_multi",
-    "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi", "metric_scratch_bytes", "metric_update",
+    "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi", "metric_scratch_bytes", "metric_weighted_scratch_bytes",
+    "metric_update",
     "clip_workspace", "clip_prepare_multi", "clip_scales", "clip_apply_multi",
 ]
 
@@ -482,9 +483,17 @@ def lau_fwd(table: torch.Tensor, query_ids: torch.Tensor, key_ids: torch.Tensor,
 # head / optimisers
 # --------------------------------------------------------------------------------------------
 def sigmoid_bce(dnn_logit: torch.Tensor, fm_logit: Optional[torch.Tensor], label: torch.Tensor, grad_scale: float,
-                prob: Optional[torch.Tensor] = None, dlogit: Optional[torch.Tensor] = None, loss_sum: Optional[torch.Tensor] = None):
+                prob: Optional[torch.Tensor] = None, dlogit: Optional[torch.Tensor] = None, loss_sum: Optional[torch.Tensor] = None,
+                weight: Optional[torch.Tensor] = None):
+    """With `weight` (one fp32 per sample): Keras' weighted loss, loss_sum += w*l and dlogit = (p-y)*w*grad_scale."""
     B = dnn_logit.numel()
-    call("hrb_sigmoid_bce", _p(dnn_logit), _p(fm_logit), _p(label), B, grad_scale, _p(prob), _p(dlogit), _p(loss_sum), _stream())
+    if weight is None:
+        call("hrb_sigmoid_bce", _p(dnn_logit), _p(fm_logit), _p(label), B, grad_scale, _p(prob), _p(dlogit), _p(loss_sum), _stream())
+    else:
+        if _chk(weight, torch.float32, "weight").numel() != B:
+            raise ValueError(f"sigmoid_bce: {weight.numel()} weights for {B} samples")
+        call("hrb_sigmoid_bce_weighted", _p(dnn_logit), _p(fm_logit), _p(label), _p(weight), B, grad_scale, _p(prob), _p(dlogit),
+             _p(loss_sum), _stream())
 
 
 def adam_step(param, grad, m, v, lr, beta1=0.9, beta2=0.999, eps=1e-7, step=1, l2_scale=0.0):
@@ -701,6 +710,7 @@ def dense1_bwd(x, w, dy, act_prev=None, want_t=False):
 # Keras metrics: confusion / accuracy variables counted on the device (one launch per update)
 # --------------------------------------------------------------------------------------------
 METRIC_TP, METRIC_FP, METRIC_TN, METRIC_FN, METRIC_CORRECT, METRIC_COUNT = 0, 1, 2, 3, 4, 5
+METRIC_WTP, METRIC_WFP, METRIC_WTN, METRIC_WFN, METRIC_WCORRECT, METRIC_WCOUNT = 6, 7, 8, 9, 10, 11
 METRIC_MAX_THRESHOLDS = 8192
 
 
@@ -710,11 +720,20 @@ def metric_scratch_bytes(n_thr: int) -> int:
     return need.value
 
 
+def metric_weighted_scratch_bytes(n_thr: int) -> int:
+    need = ctypes.c_size_t(0)
+    call("hrb_metric_weighted_scratch_bytes", int(n_thr), ctypes.byref(need))
+    return need.value
+
+
 def metric_update(prob: torch.Tensor, label: torch.Tensor, thresholds: torch.Tensor, var_kind: torch.Tensor, var_thr: torch.Tensor,
-                  vars: torch.Tensor, scratch: torch.Tensor, flags: Optional[torch.Tensor] = None) -> None:
+                  vars: torch.Tensor, scratch: torch.Tensor, flags: Optional[torch.Tensor] = None,
+                  weight: Optional[torch.Tensor] = None) -> None:
     """vars[v] += the batch's count of kind var_kind[v] at thresholds[var_thr[v]], one fp32 rounding per variable (hrb200.h:
     hrb_metric_update).  thresholds ascending and distinct; scratch from metric_scratch_bytes, zeroed once; flags (int32, one per
-    variable, nullable): set for the TP / FP / TN / FN variables when a prob is outside [0, 1] or NaN."""
+    variable, nullable): set for the TP / FP / TN / FN variables when a prob is outside [0, 1] or NaN.
+    With `weight` (fp32, one per sample): hrb_metric_update_weighted, which also takes the weighted kinds METRIC_WTP..WCOUNT;
+    scratch from metric_weighted_scratch_bytes."""
     _chk(prob, torch.float32, "prob")
     _chk(label, torch.float32, "label")
     _chk(thresholds, torch.float32, "thresholds")
@@ -728,6 +747,14 @@ def metric_update(prob: torch.Tensor, label: torch.Tensor, thresholds: torch.Ten
         raise ValueError("metric_update: var_kind, var_thr and vars must have one entry per variable")
     if flags is not None and (_chk(flags, torch.int32, "flags").numel() != vars.numel()):
         raise ValueError("metric_update: flags must have one entry per variable")
+    if weight is not None:
+        if _chk(weight, torch.float32, "weight").numel() != prob.numel():
+            raise ValueError(f"metric_update: {prob.numel()} predictions but {weight.numel()} weights")
+        if scratch.numel() < metric_weighted_scratch_bytes(thresholds.numel()):
+            raise ValueError("metric_update: scratch too small (metric_weighted_scratch_bytes)")
+        call("hrb_metric_update_weighted", _p(prob), _p(label), _p(weight), prob.numel(), _p(thresholds), thresholds.numel(), _p(var_kind),
+             _p(var_thr), vars.numel(), _p(vars), _p(scratch), _p(flags), _stream())
+        return
     if scratch.numel() < metric_scratch_bytes(thresholds.numel()):
         raise ValueError("metric_update: scratch too small (metric_scratch_bytes)")
     call("hrb_metric_update", _p(prob), _p(label), prob.numel(), _p(thresholds), thresholds.numel(), _p(var_kind), _p(var_thr),

@@ -194,18 +194,22 @@ class _ColumnSet:
 
 
 class HostBatch:
-    """One packed batch in pinned memory + the event that says its host->device copies are done (slot reusable)."""
+    """One packed batch in pinned memory + the event that says its host->device copies are done (slot reusable).  The sample
+    weight column is pinned at the first batch with weights; `weighted` says whether the batch packed now has them."""
 
     def __init__(self, B: int, ids_cols: int, n_dense: int):
         self.ids = torch.empty(B, max(ids_cols, 1), dtype=torch.int32).pin_memory()
         self.dense = torch.empty(B, max(n_dense, 1), dtype=torch.float32).pin_memory()
         self.label = torch.empty(B, dtype=torch.float32).pin_memory()
+        self.weight: Optional[torch.Tensor] = None
+        self.weighted = False
         self.copied: Optional[torch.cuda.Event] = None
         self.rows = 0
 
     def views(self):
+        """(ids, dense, label, weight or None) of the packed rows."""
         r = self.rows
-        return self.ids[:r], self.dense[:r], self.label[:r]
+        return self.ids[:r], self.dense[:r], self.label[:r], (self.weight[:r] if self.weighted else None)
 
 
 class FusedDeepFM:
@@ -358,9 +362,15 @@ class FusedDeepFM:
         n = len(id_cols.keep[0])
         return id_cols, dense_cols, n
 
-    def _pack(self, slot: HostBatch, id_cols, dense_cols, label_cols, start: int, rows: int) -> None:
+    def _pack(self, slot: HostBatch, id_cols, dense_cols, label_cols, start: int, rows: int, weight_cols=None) -> None:
         if slot.copied is not None:
             slot.copied.synchronize()  # the previous user's host->device copies have left this pinned slot
+        slot.weighted = weight_cols is not None
+        if slot.weighted:
+            if slot.weight is None:
+                slot.weight = torch.empty(slot.label.shape[0], dtype=torch.float32).pin_memory()
+            call("hrb_host_pack_f32", weight_cols.ptrs, weight_cols.dtype, weight_cols.width, weight_cols.ld, 1, start, rows,
+                 ctypes.c_void_p(slot.weight.data_ptr()), 1, 0)
         call("hrb_host_pack_i32", id_cols.ptrs, id_cols.dtype, id_cols.width, id_cols.ld, id_cols.n, start, rows,
              ctypes.c_void_p(slot.ids.data_ptr()), slot.ids.shape[1], self._pack_threads)
         if self.n_dense:
@@ -376,10 +386,12 @@ class FusedDeepFM:
             self._slots.append(HostBatch(self.engine.B, self.ids_cols, self.n_dense))
         return self._slots
 
-    def host_batches(self, x, y, batch_size: int, n_slots: int = 4):
-        """Generator of packed pinned batches; packing runs on a background thread, up to n_slots-2 batches ahead."""
+    def host_batches(self, x, y, batch_size: int, n_slots: int = 4, weight: Optional[np.ndarray] = None):
+        """Generator of packed pinned batches; packing runs on a background thread, up to n_slots-2 batches ahead.  `weight`: the
+        float32 sample weights of the rows (Keras' sample_weight with class_weight folded in), packed like the label."""
         id_cols, dense_cols, n = self._columns(x)
         label_cols = _ColumnSet([np.asarray(y).reshape(-1, 1)]) if y is not None else None
+        weight_cols = _weight_columns(weight)
         slots = self._get_slots(n_slots)
         q: "queue.Queue" = queue.Queue(maxsize=max(1, n_slots - 2))
         dev_index = torch.cuda.current_device()
@@ -390,7 +402,7 @@ class FusedDeepFM:
                 k = 1
                 for start in range(batch_size, n, batch_size):
                     slot = slots[k % n_slots]
-                    self._pack(slot, id_cols, dense_cols, label_cols, start, min(batch_size, n - start))
+                    self._pack(slot, id_cols, dense_cols, label_cols, start, min(batch_size, n - start), weight_cols)
                     q.put(slot)
                     k += 1
                 q.put(None)
@@ -401,7 +413,7 @@ class FusedDeepFM:
             return
         # The first batch is packed right here: the GPU gets its first step without waiting for a thread to start (0.3-0.8 ms);
         # the producer thread for the remaining batches starts while that step runs.
-        self._pack(slots[0], id_cols, dense_cols, label_cols, 0, min(batch_size, n))
+        self._pack(slots[0], id_cols, dense_cols, label_cols, 0, min(batch_size, n), weight_cols)
         yield slots[0]
         th = threading.Thread(target=producer, daemon=True)
         th.start()
@@ -415,30 +427,31 @@ class FusedDeepFM:
         th.join()
 
     # ---- Keras-facing calls -----------------------------------------------------------------------
-    def fit_epoch(self, x, y, batch_size: int) -> List[float]:
+    def fit_epoch(self, x, y, batch_size: int, weight: Optional[np.ndarray] = None) -> List[float]:
         self._dirty = True
-        return self.engine.fit_batches(self.host_batches(x, y, batch_size))
+        return self.engine.fit_batches(self.host_batches(x, y, batch_size, weight=weight))
 
-    def train_on_batch(self, x, y) -> float:
+    def train_on_batch(self, x, y, weight: Optional[np.ndarray] = None) -> float:
         id_cols, dense_cols, n = self._columns(x)
         slot = self._get_slots(1)[0]
-        self._pack(slot, id_cols, dense_cols, _ColumnSet([np.asarray(y).reshape(-1, 1)]), 0, n)
+        self._pack(slot, id_cols, dense_cols, _ColumnSet([np.asarray(y).reshape(-1, 1)]), 0, n, _weight_columns(weight))
         self._dirty = True
-        ids, dense, label = slot.views()
-        return self.engine.train_on_batch(ids, dense if self.n_dense else None, label)
+        ids, dense, label, w = slot.views()
+        return self.engine.train_on_batch(ids, dense if self.n_dense else None, label, w)
 
-    def predict(self, x, batch_size: Optional[int], y=None, metrics=None) -> np.ndarray:
+    def predict(self, x, batch_size: Optional[int], y=None, metrics=None, weight: Optional[np.ndarray] = None) -> np.ndarray:
         """Probabilities of `x`; with `metrics` (a MetricSet) and labels `y`, every batch is also counted on the device (the
-        validation pass of fit / evaluate: no second forward)."""
+        validation pass of fit / evaluate: no second forward), with the rows' sample weights `weight` when given."""
         id_cols, dense_cols, n = self._columns(x)
         bs = min(batch_size or n, self.engine.B)
         slot = self._get_slots(1)[0]
         label_cols = _ColumnSet([np.asarray(y).reshape(-1, 1)]) if metrics is not None else None
+        weight_cols = _weight_columns(weight) if metrics is not None else None
         outs = []
         for start in range(0, n, bs):
-            self._pack(slot, id_cols, dense_cols, label_cols, start, min(bs, n - start))
-            ids, dense, label = slot.views()
-            outs.append(self.engine.predict(ids, dense if self.n_dense else None, label, metrics).numpy().copy())
+            self._pack(slot, id_cols, dense_cols, label_cols, start, min(bs, n - start), weight_cols)
+            ids, dense, label, w = slot.views()
+            outs.append(self.engine.predict(ids, dense if self.n_dense else None, label, metrics, w).numpy().copy())
             slot.copied = None
         return np.concatenate(outs, 0)
 
@@ -453,6 +466,10 @@ class FusedDeepFM:
         if eng.l2_embd and eng.dense_tables:
             tot += eng.l2_embd * float(sum((eng.tables[t] ** 2).sum() for t in eng.dense_tables))
         return tot
+
+
+def _weight_columns(weight: Optional[np.ndarray]) -> Optional[_ColumnSet]:
+    return _ColumnSet([np.asarray(weight, dtype=np.float32).reshape(-1, 1)]) if weight is not None else None
 
 
 def _lr_step(optimizer):

@@ -8,23 +8,33 @@ their thresholds and one (kind, threshold) descriptor per variable, so that one 
 every metric at once.  `read()` copies the variables to the host (after a sum over ranks under a communicator) and each metric's
 `result()` applies Keras' formula there in float32.
 
+Sample weights (Keras' MetricsContainer): metrics compiled in `weighted_metrics` count every sample as its weight when a step has
+weights (tp += sum of w over the true positives, BinaryAccuracy's total += sum of w * correct and count += sum of w); metrics in
+`metrics` never do.  A set that holds weighted metrics keeps a second descriptor array in which their variables have the weighted
+kinds (hrb200.h: HRB_METRIC_WTP..WCOUNT): a batch with weights is counted by one `hrb_metric_update_weighted` (two launches), the
+unweighted metrics of the same set taking their integer counts in it; a batch without weights by `hrb_metric_update` as before.
+The weighted sums are accumulated in float64 in a fixed order and rounded once to float32, so they are reproducible bit for bit.
+
 Deviations from Keras (DESIGN.md 3, "Metrics"):
   * Keras asserts 0 <= y_pred <= 1 in the step that sees a bad prediction; here the kernel flags the variables of the confusion
     metrics that counted it, and the ValueError is raised when their results are read (end of epoch, `evaluate`,
     `train_on_batch`, `result()`).  `reset_state()` clears a metric's flags with its variables.
   * at most 8192 distinct thresholds over one model's metrics (ValueError at `compile`).
   * default names are de-duplicated within one `compile` (`auc`, `auc_1`, ...), not by Keras' session-wide counter.
+  * a metric's own `update_state` takes no `sample_weight` (NotImplementedError): the weights reach a metric compiled in
+    `weighted_metrics` through the model's fit / train_on_batch / evaluate.
 """
 from __future__ import annotations
 
 from collections import OrderedDict
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 
 MAX_THRESHOLDS = 8192
 TP, FP, TN, FN, CORRECT, COUNT = 0, 1, 2, 3, 4, 5  # hrb200.h: hrb_metric_kind
+WEIGHTED = 6  # kind + WEIGHTED: the same variable summing the samples' weights (HRB_METRIC_WTP..WCOUNT)
 _EPSILON = 1e-7  # keras.backend.epsilon()
 
 
@@ -36,7 +46,8 @@ def _div_no_nan(a: np.ndarray, b: np.ndarray) -> np.ndarray:
 
 def _no_sample_weight(sample_weight) -> None:
     if sample_weight is not None:
-        raise NotImplementedError("sample_weight is not supported by handyrec_b200's metrics")
+        raise NotImplementedError("sample_weight is not supported by a metric's own update_state: compile the metric in "
+                                  "weighted_metrics and pass the weights to fit / train_on_batch / evaluate")
 
 
 def _parse_thresholds(thresholds, default: float) -> List[float]:
@@ -228,8 +239,26 @@ def get(metric) -> Metric:
                      f"BinaryAccuracy objects")
 
 
-def from_compile(metrics) -> List[Metric]:
-    """`compile(metrics=...)`: objects and strings, names made unique within the list (`auc`, `auc_1`, ...)."""
+def from_compile(metrics, weighted_metrics=None) -> Tuple[List[Metric], List[Metric]]:
+    """`compile(metrics=..., weighted_metrics=...)`: objects and strings, names made unique within each list (`auc`, `auc_1`, ...);
+    then a weighted metric whose name an unweighted one has is renamed `weighted_<name>` (Keras' MetricsContainer).  Returns the
+    metrics followed by the weighted metrics, and the weighted metrics."""
+    out = _unique(metrics)
+    weighted = _unique(weighted_metrics)
+    for w in weighted:
+        if any(w is m for m in out):
+            raise ValueError(f"metric {w.name!r} is listed in both metrics and weighted_metrics")
+    names = {m.name for m in out}
+    for w in weighted:
+        if w.name in names:
+            w.name = "weighted_" + w.name
+        if w.name in names:
+            raise ValueError(f"Found two metrics with the same name: {w.name}")
+        names.add(w.name)
+    return out + weighted, weighted
+
+
+def _unique(metrics) -> List[Metric]:
     if metrics is None:
         return []
     items = list(metrics) if isinstance(metrics, (list, tuple)) else [metrics]
@@ -260,8 +289,9 @@ class MetricSet:
     contiguous slice of them), and the kernel's scratch.  Host-side construction checks everything; device buffers are allocated
     on the current CUDA device at the first update or read."""
 
-    def __init__(self, metrics: Sequence[Metric]):
+    def __init__(self, metrics: Sequence[Metric], weighted: Sequence[Metric] = ()):
         self.metrics = list(metrics)
+        self.weighted = [any(m is w for w in weighted) for m in self.metrics]
         thr = sorted({float(t) for m in self.metrics for _, t in m._descriptors() if t is not None})
         if len(thr) > MAX_THRESHOLDS:
             raise ValueError(f"the metrics use {len(thr)} distinct thresholds; at most {MAX_THRESHOLDS} are supported per model")
@@ -276,6 +306,11 @@ class MetricSet:
             self.slices.append(slice(off, len(kinds)))
             m._set, m._index = self, i
         self.kinds = np.array(kinds, dtype=np.int32)
+        # the descriptors of a batch with weights: the weighted metrics' variables take the weighted kinds
+        self.weighted_kinds = self.kinds.copy()
+        for sl, w in zip(self.slices, self.weighted):
+            if w:
+                self.weighted_kinds[sl] += WEIGHTED
         self.thr_index = np.array(tidx, dtype=np.int32)
         self.names = [m.name for m in self.metrics]
         self._dev = None
@@ -296,6 +331,17 @@ class MetricSet:
                 scratch=torch.zeros(K.metric_scratch_bytes(len(self.thresholds)), device=dev, dtype=torch.uint8))
         return self._dev
 
+    def _weighted_buffers(self):
+        """The weighted update's descriptors and scratch, allocated at the first batch with weights."""
+        b = self._buffers()
+        if "wscratch" not in b:
+            from . import kernels as K
+
+            dev = b["vars"].device
+            b["weighted_kinds"] = torch.from_numpy(self.weighted_kinds).to(dev)
+            b["wscratch"] = torch.zeros(K.metric_weighted_scratch_bytes(len(self.thresholds)), device=dev, dtype=torch.uint8)
+        return b
+
     @property
     def variables(self) -> torch.Tensor:
         """The local float32 variables, one slice per metric (`slices`)."""
@@ -306,8 +352,10 @@ class MetricSet:
             t = torch.as_tensor(np.asarray(t, dtype=np.float32))
         return t.detach().to(dev, torch.float32).reshape(-1).contiguous()
 
-    def update(self, y_pred, y_true, only: Optional[Metric] = None) -> None:
-        """Count one batch into every metric's variables (or `only` one metric's): one hrb_metric_update launch."""
+    def update(self, y_pred, y_true, weight=None, only: Optional[Metric] = None) -> None:
+        """Count one batch into every metric's variables (or `only` one metric's): one hrb_metric_update launch.  With `weight` (one
+        float32 per sample) the weighted metrics sum the weights, and the batch takes one hrb_metric_update_weighted instead (two
+        launches); when no metric of the update is weighted, the weights are not read."""
         from . import kernels as K
 
         b = self._buffers()
@@ -317,6 +365,14 @@ class MetricSet:
             raise ValueError(f"metrics: {p.numel()} predictions but {y.numel()} labels (single-output binary models)")
         sl = slice(0, len(self.kinds)) if only is None else self.slices[only._index]
         if sl.stop == sl.start:
+            return
+        if weight is not None and any(self.weighted):
+            w = self._as_device(weight, dev)
+            if w.numel() != p.numel():
+                raise ValueError(f"metrics: {p.numel()} predictions but {w.numel()} sample weights")
+            wb = self._weighted_buffers()
+            K.metric_update(p, y, b["thresholds"], wb["weighted_kinds"][sl], b["thr_index"][sl], b["vars"][sl], wb["wscratch"], b["flags"][sl],
+                            weight=w)
             return
         K.metric_update(p, y, b["thresholds"], b["kinds"][sl], b["thr_index"][sl], b["vars"][sl], b["scratch"], b["flags"][sl])
 

@@ -338,6 +338,15 @@ int hrb_sigmoid_bce(const float* dnn_logit, const float* fm_logit, const float* 
 int hrb_clipped_bce(const float* prob, const float* label, int64_t n, float eps, float grad_scale, float* dprob,
                     float* loss_sum, void* stream);
 
+/* Keras sample weights (losses_utils.compute_weighted_loss): the entries above with one fp32 weight per sample,
+ *   loss_sum += w*l;  dlogit (dprob) = d l / d logit (prob) * w * grad_scale.
+ * The caller divides loss_sum by the batch size, not by sum(w), and passes grad_scale = 1 / (batch * ranks) as above.
+ * w = 1 gives prob and dlogit (dprob) bit-equal to the unweighted entries. */
+int hrb_sigmoid_bce_weighted(const float* dnn_logit, const float* fm_logit, const float* label, const float* weight, int64_t batch,
+                             float grad_scale, float* prob, float* dlogit, float* loss_sum, void* stream);
+int hrb_clipped_bce_weighted(const float* prob, const float* label, const float* weight, int64_t n, float eps, float grad_scale,
+                             float* dprob, float* loss_sum, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * (f1) retrieval loss: SampledSoftmaxLayer.call = tf.nn.sampled_softmax_loss (layers/tools.py:56-75), TF defaults:
  *   num_true = 1, remove_accidental_hits, subtract log Q, log-uniform candidates drawn unique.
@@ -388,12 +397,33 @@ typedef enum hrb_metric_kind {
   HRB_METRIC_TN = 2,
   HRB_METRIC_FN = 3,
   HRB_METRIC_CORRECT = 4,
-  HRB_METRIC_COUNT = 5
+  HRB_METRIC_COUNT = 5,
+  HRB_METRIC_WTP = 6, /* the weighted kinds: hrb_metric_update_weighted only */
+  HRB_METRIC_WFP = 7,
+  HRB_METRIC_WTN = 8,
+  HRB_METRIC_WFN = 9,
+  HRB_METRIC_WCORRECT = 10,
+  HRB_METRIC_WCOUNT = 11
 } hrb_metric_kind;
 int hrb_metric_scratch_bytes(int32_t n_thr, size_t* bytes);
 int hrb_metric_update(const float* prob, const float* label, int64_t n, const float* thresholds, int32_t n_thr,
                       const int32_t* var_kind, const int32_t* var_thr, int32_t n_vars, float* vars, void* scratch, int32_t* flags,
                       void* stream);
+
+/* Keras metrics with sample weights (update_confusion_matrix_variables with sample_weight, the Mean of binary_accuracy): as
+ * hrb_metric_update with one fp32 weight per sample.  Kinds 0..5 add the same integer counts, bit-equal to hrb_metric_update on
+ * the same batch.  Kinds WTP..WCOUNT add the same sums with every sample counted as its weight instead of 1 (WCOUNT = sum w):
+ * each per-(class, bucket) sum is accumulated in fp64, the suffix sums are taken in fp64, and each variable adds its increment
+ * rounded once to fp32 (Keras assign_add).  Negative, zero and NaN weights are taken as given.  Flags: as hrb_metric_update, for
+ * WTP..WFN too.  The variables are bit-reproducible: every CTA sorts its samples by (class, bucket) with a block radix sort and
+ * sums the runs in sorted order into its own fp64 bins; a second launch adds the bins over the CTAs in CTA order, takes the
+ * suffix sums and updates the variables.  scratch: hrb_metric_weighted_scratch_bytes(n_thr) for the CURRENT device, zeroed by
+ * the caller once; every call leaves it zeroed (calls sharing a scratch must be stream-ordered).  Two launches; n = 0 launches
+ * nothing. */
+int hrb_metric_weighted_scratch_bytes(int32_t n_thr, size_t* bytes);
+int hrb_metric_update_weighted(const float* prob, const float* label, const float* weight, int64_t n, const float* thresholds,
+                               int32_t n_thr, const int32_t* var_kind, const int32_t* var_thr, int32_t n_vars, float* vars,
+                               void* scratch, int32_t* flags, void* stream);
 
 /* a8 concat glue (layers/utils.py:28-36,70-84): dense features (fp32, or int32 cast to fp32) go to the
  * head columns of the DNN input row; columns [n, n_pad) are zero-filled (alignment padding). */
