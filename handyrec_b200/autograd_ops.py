@@ -306,6 +306,47 @@ class ClippedBCEFn(torch.autograd.Function):
         return (dp * g).reshape(ctx.shape), None, None
 
 
+_loss_ws = {}  # (device index, raw stream) -> the layer path's hrb_regression_loss workspace
+
+
+def _regression_workspace(n: int, device: torch.device) -> torch.Tensor:
+    """The hrb_regression_loss workspace of the current stream, zeroed once when it is allocated (or grown for a larger batch); the
+    kernel leaves it zeroed, so later calls need no memset."""
+    need = ctypes.c_size_t(0)
+    call("hrb_regression_loss_workspace", n, ctypes.byref(need))
+    key = (device.index, K._stream().value)
+    ws = _loss_ws.get(key)
+    if ws is None or ws.numel() < need.value:
+        ws = _loss_ws[key] = torch.zeros(need.value, device=device, dtype=torch.uint8)
+    return ws
+
+
+class RegressionLossFn(torch.autograd.Function):
+    """Keras mean_squared_error / mean_absolute_error / huber (`loss`, kernels.REG_LOSS): the mean over the last axis per sample,
+    then the batch mean; with `weight`, sum(w * l) / B as SigmoidBCEFn.  `label` has the shape of `pred` (the caller applies Keras'
+    (B,) -> (B, 1) rule)."""
+
+    @staticmethod
+    def forward(ctx, pred, label, loss, delta, weight=None):
+        shape = pred.shape
+        B = shape[0] if pred.dim() else 1
+        cols = pred.numel() // B if B else 1
+        p = pred.contiguous().reshape(-1)
+        y = label.contiguous().reshape(-1).to(torch.float32)
+        dp = torch.empty_like(p)
+        ls = torch.empty(1, device=p.device, dtype=torch.float32)
+        K.regression_loss(loss, delta, p, None, y, B, cols, 1.0 / max(B, 1), None, dp, ls, weight=weight,
+                          workspace=_regression_workspace(p.numel(), p.device))
+        ctx.save_for_backward(dp)
+        ctx.shape = shape
+        return (ls / max(B, 1)).reshape(())
+
+    @staticmethod
+    def backward(ctx, g):
+        (dp,) = ctx.saved_tensors
+        return (dp * g).reshape(ctx.shape), None, None, None, None
+
+
 class ActivationFn(torch.autograd.Function):
     """Stand-alone Keras Activation(name) for relu / sigmoid / tanh (element-wise)."""
 

@@ -92,9 +92,13 @@ def _tf_module() -> types.ModuleType:
 
     regs.l2 = _L2
     losses = types.ModuleType("tensorflow.keras.losses")
-    losses.binary_crossentropy = KL.binary_crossentropy
     opts = types.ModuleType("tensorflow.keras.optimizers")
     opts.Adam, opts.SGD, opts.Adagrad, opts.Ftrl = KL.Adam, KL.SGD, KL.Adagrad, KL.Ftrl
+    for n in ("binary_crossentropy", "mean_squared_error", "mse", "MSE", "mean_absolute_error", "mae", "MAE", "MeanSquaredError",
+              "MeanAbsoluteError", "Huber", "BinaryCrossentropy"):
+        setattr(losses, n, getattr(KL, n))
+    losses.get = KL.get_loss
+    opts.get = KL.get_optimizer
     from .. import schedules as S
 
     scheds = types.ModuleType("tensorflow.keras.optimizers.schedules")

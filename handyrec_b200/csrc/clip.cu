@@ -38,18 +38,6 @@ __device__ __forceinline__ double block_sum(double s) {
   return t;  // valid in thread 0
 }
 
-// true in every thread of the last CTA to finish (the partials of every CTA are then visible to it).  The barrier first: every
-// thread of this CTA has stored its partials before thread 0 publishes the CTA as done.
-__device__ __forceinline__ bool last_block(unsigned int* counter) {
-  __shared__ bool last;
-  __syncthreads();
-  __threadfence();
-  if (threadIdx.x == 0) last = atomicAdd(counter, 1u) == gridDim.x - 1;
-  __syncthreads();
-  if (last) __threadfence();
-  return last;
-}
-
 struct ClipPrepArgs {
   float* g[HRB_MULTI_MAX];
   const float* w[HRB_MULTI_MAX];

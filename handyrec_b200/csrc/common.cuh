@@ -74,6 +74,18 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// true in every thread of the last CTA to finish (the partials of every CTA are then visible to it).  The barrier first: every
+// thread of this CTA has stored its partials before thread 0 publishes the CTA as done.
+__device__ __forceinline__ bool last_block(unsigned int* counter) {
+  __shared__ bool last;
+  __syncthreads();
+  __threadfence();
+  if (threadIdx.x == 0) last = atomicAdd(counter, 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (last) __threadfence();
+  return last;
+}
+
 // Keras Ftrl (TF ApplyFtrl / ApplyFtrlV2 functors) on one element; acc and lin are its accumulator and linear slots, g already
 // holds the l2 regulariser term, l2 has beta / (2*lr) added.  Returns the new weight.  The row update (plan.cuh), the dense step
 // and the multi-tensor step (misc.cu) all call this: every operation is rounded explicitly (no contraction left to the

@@ -73,6 +73,77 @@ __global__ void __launch_bounds__(256) clipped_bce_kernel(const float* __restric
   }
 }
 
+// Keras regression losses on one error e = pred - y (keras/losses.py mean_squared_error, mean_absolute_error, huber), with TF's
+// gradients: d|e|/de = 0 at e = 0, and the quadratic branch of huber takes the tie |e| == delta (tf.minimum gives it to its first
+// argument, q = min(|e|, delta)).
+enum RegLoss { REG_MSE = 0, REG_MAE = 1, REG_HUBER = 2 };
+
+template <int LOSS>
+__device__ __forceinline__ float reg_loss(float e, float delta, float& dl) {
+  const float a = fabsf(e);
+  const float s = e > 0.f ? 1.f : (e < 0.f ? -1.f : 0.f);
+  if (LOSS == REG_MSE) {
+    dl = 2.f * e;
+    return e * e;
+  } else if (LOSS == REG_MAE) {
+    dl = s;
+    return a;
+  } else {
+    const float q = fminf(a, delta);
+    dl = a <= delta ? e : delta * s;
+    return 0.5f * q * q + delta * (a - q);  // 0.5*q^2 + delta*(|e| - q)
+  }
+}
+
+constexpr int kRegThreads = 256;
+
+// pred = a (+ b); loss_sum = sum_i w_i * l(e_i) * inv_cols (w = 1 unweighted), dpred = dl * w * grad_scale.  The sum is reduced in
+// float64 in a fixed order (per-thread grid stride, block tree, then the last CTA adds the CTA partials in CTA order), so two
+// runs give the same bits.  label / dpred / loss_sum may be null for a forward alone (then no workspace is touched).
+template <int LOSS, bool WEIGHTED>
+__global__ void __launch_bounds__(kRegThreads) regression_loss_kernel(const float* __restrict__ a, const float* __restrict__ b,
+                                                                      const float* __restrict__ label, const float* __restrict__ weight,
+                                                                      int64_t n, int32_t cols, float delta, float grad_scale, double inv_cols,
+                                                                      float* __restrict__ pred, float* __restrict__ dpred,
+                                                                      float* __restrict__ loss_sum, double* __restrict__ partial,
+                                                                      unsigned int* __restrict__ counter) {
+  double local = 0.0;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const float p = b != nullptr ? a[i] + b[i] : a[i];  // the model's `deep + wide` (DeepFM.py:86)
+    if (pred != nullptr) pred[i] = p;
+    if (label == nullptr) continue;
+    float dl;
+    const float l = reg_loss<LOSS>(p - label[i], delta, dl);
+    if constexpr (WEIGHTED) {
+      const float w = weight[i / cols];
+      local += (double)w * (double)l;
+      if (dpred != nullptr) dpred[i] = dl * w * grad_scale;
+    } else {
+      local += (double)l;
+      if (dpred != nullptr) dpred[i] = dl * grad_scale;
+    }
+  }
+  if (loss_sum == nullptr) return;
+  __shared__ double red[kRegThreads / 32];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xffffffffu, local, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = local;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+#pragma unroll
+    for (int k = 0; k < kRegThreads / 32; ++k) t += red[k];
+    partial[blockIdx.x] = t;
+  }
+  if (!last_block(counter)) return;
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+    for (unsigned k = 0; k < gridDim.x; ++k) t += partial[k];
+    *loss_sum = (float)(t * inv_cols);
+    *counter = 0u;
+  }
+}
+
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                   float* __restrict__ v, int64_t n, float lr_t, float b1, float b2,
                                                   float eps, float l2_scale) {
@@ -348,6 +419,61 @@ HRB_API int hrb_clipped_bce_weighted(const float* prob, const float* label, cons
   clipped_bce_kernel<true><<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(prob, label, weight, n, eps, grad_scale, dprob, loss_sum);
   HRB_LAUNCH_CHECK();
   return HRB_OK;
+}
+
+// workspace: the completion counter (zeroed by the caller once; the last CTA re-zeroes it) in the first 16 bytes, then one float64
+// partial per CTA
+static size_t regression_loss_ws(int64_t n) { return 16 + sizeof(double) * (size_t)ew_grid(n); }
+
+HRB_API int hrb_regression_loss_workspace(int64_t n, size_t* bytes) {
+  HRB_REQUIRE(n >= 0 && bytes, "hrb_regression_loss_workspace: bad argument");
+  *bytes = regression_loss_ws(n);
+  return HRB_OK;
+}
+
+template <bool WEIGHTED>
+static int regression_loss(const char* name, int32_t loss, float delta, const float* a, const float* b, const float* label,
+                           const float* weight, int64_t batch, int32_t cols, float grad_scale, float* pred, float* dpred,
+                           float* loss_sum, void* workspace, size_t workspace_bytes, void* stream) {
+  HRB_REQUIRE(a && batch >= 0 && cols >= 1 && loss >= REG_MSE && loss <= REG_HUBER && delta >= 0.f, "%s: bad argument", name);
+  HRB_REQUIRE(label || (!dpred && !loss_sum), "%s: the loss and its gradient need the labels", name);
+  HRB_REQUIRE(!WEIGHTED || weight, "%s: null weight", name);
+  const int64_t n = batch * cols;
+  HRB_REQUIRE(!loss_sum || (workspace && workspace_bytes >= regression_loss_ws(n)), "%s: workspace of %zu bytes, %zu needed", name,
+              workspace_bytes, regression_loss_ws(n));
+  if (n == 0) {
+    if (loss_sum) HRB_CUDA(cudaMemsetAsync(loss_sum, 0, sizeof(float), (cudaStream_t)stream));
+    return HRB_OK;
+  }
+  unsigned int* counter = (unsigned int*)workspace;
+  double* partial = workspace ? (double*)((char*)workspace + 16) : nullptr;
+  const float gs = grad_scale / (float)cols;  // Keras' mean over the last axis
+  const double inv_cols = 1.0 / cols;
+  const unsigned grid = ew_grid(n);
+  cudaStream_t st = (cudaStream_t)stream;
+#define HRB_REG_LAUNCH(L)                                                                                                          \
+  regression_loss_kernel<L, WEIGHTED><<<grid, kRegThreads, 0, st>>>(a, b, label, weight, n, cols, delta, gs, inv_cols, pred, dpred, \
+                                                                    loss_sum, partial, counter)
+  if (loss == REG_MSE) HRB_REG_LAUNCH(REG_MSE);
+  else if (loss == REG_MAE) HRB_REG_LAUNCH(REG_MAE);
+  else HRB_REG_LAUNCH(REG_HUBER);
+#undef HRB_REG_LAUNCH
+  HRB_LAUNCH_CHECK();
+  return HRB_OK;
+}
+
+HRB_API int hrb_regression_loss(int32_t loss, float delta, const float* pred_a, const float* pred_b, const float* label, int64_t batch,
+                                int32_t cols, float grad_scale, float* pred, float* dpred, float* loss_sum, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+  return regression_loss<false>("hrb_regression_loss", loss, delta, pred_a, pred_b, label, nullptr, batch, cols, grad_scale, pred, dpred,
+                                loss_sum, workspace, workspace_bytes, stream);
+}
+
+HRB_API int hrb_regression_loss_weighted(int32_t loss, float delta, const float* pred_a, const float* pred_b, const float* label,
+                                         const float* weight, int64_t batch, int32_t cols, float grad_scale, float* pred, float* dpred,
+                                         float* loss_sum, void* workspace, size_t workspace_bytes, void* stream) {
+  return regression_loss<true>("hrb_regression_loss_weighted", loss, delta, pred_a, pred_b, label, weight, batch, cols, grad_scale, pred,
+                               dpred, loss_sum, workspace, workspace_bytes, stream);
 }
 
 HRB_API int hrb_adam_step(float* param, const float* grad, float* m, float* v, int64_t n, float lr, float beta1,

@@ -60,6 +60,9 @@ class DeepFMEngine:
     (padding id 0 of pooled fields included): `plan.mark_rows` flags them in the tail of the flat gradient buffer.
 
     lr: the learning rate of every step, or None when `lr_step` gives each step its own (a Keras schedule).
+
+    task: "binary" (sigmoid head, binary_crossentropy) or "regression" (the raw `dnn + fm`, DeepFM.py:86-88 without the sigmoid),
+    trained with `loss` "mean_squared_error", "mean_absolute_error" or "huber" (`huber_delta`); `prob` then holds the predictions.
     """
 
     def __init__(
@@ -89,13 +92,20 @@ class DeepFMEngine:
         clipvalue: Optional[float] = None,
         clipnorm: Optional[float] = None,
         global_clipnorm: Optional[float] = None,
+        loss: Optional[str] = None,
+        huber_delta: float = 1.0,
     ):
         if dnn_hidden_units[-1] != 1:  # DeepFM.py:59-60
             raise ValueError("Output size of dnn should be 1")
         if dnn_activation not in ("relu", "sigmoid", "tanh", "linear", None):
             raise ValueError(f"fused engine supports relu/sigmoid/tanh/linear DNN activations, got {dnn_activation!r}")
-        if task != "binary":
-            raise ValueError("fused engine implements task='binary'")
+        if task == "binary" and loss not in (None, "binary_crossentropy"):
+            raise ValueError(f"task='binary' trains binary_crossentropy, got loss={loss!r}")
+        if task == "regression" and loss not in K.REG_LOSS:
+            raise ValueError(f"task='regression' trains one of {sorted(K.REG_LOSS)}, got loss={loss!r}")
+        if task not in ("binary", "regression"):
+            raise ValueError(f"fused engine implements task='binary' and task='regression', got {task!r}")
+        self.task, self.loss, self.huber_delta = task, loss or "binary_crossentropy", float(huber_delta)
         if initial_accumulator_value < 0:
             raise ValueError(f"initial_accumulator_value must be non-negative, got {initial_accumulator_value}")
         if learning_rate_power > 0 or min(l1, l2, l2_shrinkage) < 0:
@@ -222,6 +232,7 @@ class DeepFMEngine:
         self.fm_sum = torch.empty(B, self.D, **f32)
         self.prob = torch.empty(B, **f32)
         self.loss_sum = torch.zeros(1, **f32)
+        self._loss_ws = K.regression_loss_workspace(B, self.dev) if task == "regression" else None
         # tcgen05 path: transposed copies (W^T, dZ^T) so that every GEMM operand has its reduction dim contiguous; the activations are
         # read untransposed by the weight-gradient GEMM (hrb_dense_bwd_w_xn)
         self.use_tc = gemm_mode != _lib.GEMM_FP32 and B >= 512 and B % 4 == 0
@@ -487,14 +498,17 @@ class DeepFMEngine:
     def predict_on_device(self, ids: torch.Tensor, dense: Optional[torch.Tensor]) -> torch.Tensor:
         B = ids.shape[0]
         self.forward(ids, dense)
+        if self.task == "regression":
+            K.regression_loss(self.loss, self.huber_delta, self.A[-1], self.fm_out, None, B, 1, 0.0, pred=self.prob)
+            return self.prob[:B]
         call("hrb_sigmoid_bce", K._p(self.A[-1]), K._p(self.fm_out), K._p(self.label_dev), B, 0.0, K._p(self.prob), None, None, K._stream())
         return self.prob[:B]
 
     def train_step_on_device(self, ids: torch.Tensor, dense: Optional[torch.Tensor], label: torch.Tensor,
                              weight: Optional[torch.Tensor] = None) -> None:
-        """One full step: forward, BCE, backward, embedding row updates, dense optimiser.  Loss sum -> self.loss_sum.  `weight`
-        (B float32, Keras' sample weights): the loss sum becomes sum(w * l) and dlogit w * (p - y) / (B * ranks), and the weighted
-        metrics sum the weights; everything after dlogit runs unchanged."""
+        """One full step: forward, loss (BCE, or the regression loss of task="regression"), backward, embedding row updates, dense
+        optimiser.  Loss sum -> self.loss_sum.  `weight` (B float32, Keras' sample weights): the loss sum becomes sum(w * l) and dlogit
+        w * dl/dlogit / (B * ranks), and the weighted metrics sum the weights; everything after dlogit runs unchanged."""
         B = ids.shape[0]
         st = K._stream()
         self.step_count += 1
@@ -503,12 +517,15 @@ class DeepFMEngine:
         self.forward(ids, dense, training=True)
         self.loss_sum.zero_()
         dlogit = self.dZ[-1]  # (B, 1): the logit layer has one unit (DeepFM.py:59-60)
-        if weight is None:
+        if self.task == "regression":  # prediction dnn + fm, loss sum and dlogit in one launch, as the sigmoid head
+            K.regression_loss(self.loss, self.huber_delta, self.A[-1], self.fm_out, label, B, 1, 1.0 / (B * self.grad_scale_div), self.prob,
+                              dlogit, self.loss_sum, weight=weight, workspace=self._loss_ws)
+        elif weight is None:
             call("hrb_sigmoid_bce", K._p(self.A[-1]), K._p(self.fm_out), K._p(label), B, 1.0 / (B * self.grad_scale_div), K._p(self.prob), K._p(dlogit), K._p(self.loss_sum), st)
         else:
             call("hrb_sigmoid_bce_weighted", K._p(self.A[-1]), K._p(self.fm_out), K._p(label), K._p(weight), B, 1.0 / (B * self.grad_scale_div),
                  K._p(self.prob), K._p(dlogit), K._p(self.loss_sum), st)
-        self._mark("sigmoid_bce")
+        self._mark("sigmoid_bce" if self.task == "binary" else "regression_loss")
         if self.metrics is not None:  # Keras counts its metrics from the training forward, before the weight update
             self.metrics.update(self.prob[:B], label, weight)
             self._mark("metric_update")
@@ -682,7 +699,7 @@ class DeepFMEngine:
 
     def train_on_batch(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor], label_host: torch.Tensor,
                        weight_host: Optional[torch.Tensor] = None) -> float:
-        """Host (pinned) tensors in, mean BCE loss out (with `weight_host`: sum(w * l) / B).  Includes the H2D copies and a D2H
+        """Host (pinned) tensors in, mean loss out (with `weight_host`: sum(w * l) / B).  Includes the H2D copies and a D2H
         read of the loss."""
         B = ids_host.shape[0]
         self.ids_dev[:B].copy_(ids_host, non_blocking=True)
@@ -773,8 +790,8 @@ class DeepFMEngine:
 
     def predict(self, ids_host: torch.Tensor, dense_host: Optional[torch.Tensor], label_host: Optional[torch.Tensor] = None,
                 metrics=None, weight_host: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Probabilities of one host batch; with `metrics` (a MetricSet) and the batch's labels, also counts them (one launch; with
-        the batch's sample weights `weight_host`, the weighted update)."""
+        """Probabilities (task="regression": predictions) of one host batch; with `metrics` (a MetricSet) and the batch's labels,
+        also counts them (one launch; with the batch's sample weights `weight_host`, the weighted update)."""
         B = ids_host.shape[0]
         self.ids_dev[:B].copy_(ids_host, non_blocking=True)
         if self.n_dense:

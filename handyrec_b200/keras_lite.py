@@ -478,6 +478,144 @@ def binary_crossentropy(y_true, y_pred):
     return SigmoidBCEFn.apply(logits, y_true, _step_weight)
 
 
+def _regression(loss: str, y_true, y_pred, delta: float = 1.0):
+    """Keras' compiled regression loss `loss` (kernels.REG_LOSS) of one output: the mean over the last axis per sample, then the
+    batch mean, or sum(w * l) / B with the step's sample weights.  A (B,) label meets a (B, 1) output as (B, 1), as Keras' compiled
+    loss expands it (compile_utils.match_dtype_and_rank) -- a plain broadcast would form a (B, B) matrix."""
+    from .autograd_ops import RegressionLossFn
+
+    yt = y_true if isinstance(y_true, torch.Tensor) else torch.as_tensor(np.asarray(y_true))
+    yt = yt.to(y_pred.device, torch.float32)
+    if yt.dim() == y_pred.dim() - 1 and y_pred.shape[-1] == 1:
+        yt = yt.unsqueeze(-1)
+    if tuple(yt.shape) != tuple(y_pred.shape):
+        raise ValueError(f"{loss}: labels of shape {tuple(yt.shape)} for predictions of shape {tuple(y_pred.shape)}")
+    return RegressionLossFn.apply(y_pred, yt, loss, float(delta), _step_weight)
+
+
+def mean_squared_error(y_true, y_pred):
+    """Keras mean_squared_error: mean((y_pred - y_true)^2, axis=-1), averaged over the batch (sample weights as binary_crossentropy)."""
+    return _regression("mean_squared_error", y_true, y_pred)
+
+
+def mean_absolute_error(y_true, y_pred):
+    """Keras mean_absolute_error: mean(|y_pred - y_true|, axis=-1), averaged over the batch (sample weights as binary_crossentropy)."""
+    return _regression("mean_absolute_error", y_true, y_pred)
+
+
+mse = MSE = mean_squared_error
+mae = MAE = mean_absolute_error
+
+
+class _Loss:
+    """tf.keras.losses.Loss with the default reduction (AUTO, i.e. SUM_OVER_BATCH_SIZE), the only one a compiled model here takes."""
+
+    def __init__(self, reduction="auto", name=None):
+        if reduction not in ("auto", "sum_over_batch_size"):
+            raise NotImplementedError(f"{type(self).__name__}(reduction={reduction!r}): only AUTO / SUM_OVER_BATCH_SIZE is supported")
+        self.reduction, self.name = reduction, name
+
+
+class MeanSquaredError(_Loss):
+    def __init__(self, reduction="auto", name="mean_squared_error"):
+        super().__init__(reduction, name)
+
+    def __call__(self, y_true, y_pred):
+        return mean_squared_error(y_true, y_pred)
+
+
+class MeanAbsoluteError(_Loss):
+    def __init__(self, reduction="auto", name="mean_absolute_error"):
+        super().__init__(reduction, name)
+
+    def __call__(self, y_true, y_pred):
+        return mean_absolute_error(y_true, y_pred)
+
+
+class Huber(_Loss):
+    """Keras Huber: 0.5*q^2 + delta*(|e| - q) with q = min(|e|, delta), e = y_pred - y_true, mean over the last axis."""
+
+    def __init__(self, delta=1.0, reduction="auto", name="huber_loss"):
+        super().__init__(reduction, name)
+        if delta < 0:
+            raise ValueError(f"Huber: delta must be non-negative, got {delta}")
+        self.delta = float(delta)
+
+    def __call__(self, y_true, y_pred):
+        return _regression("huber", y_true, y_pred, self.delta)
+
+
+class BinaryCrossentropy(_Loss):
+    """Keras BinaryCrossentropy with its defaults: binary_crossentropy."""
+
+    def __init__(self, from_logits=False, label_smoothing=0.0, reduction="auto", name="binary_crossentropy"):
+        if from_logits:
+            raise NotImplementedError("BinaryCrossentropy(from_logits=True): the models here end in a sigmoid; use the default")
+        if label_smoothing:
+            raise NotImplementedError(f"BinaryCrossentropy(label_smoothing={label_smoothing}): not supported")
+        super().__init__(reduction, name)
+
+    def __call__(self, y_true, y_pred):
+        return binary_crossentropy(y_true, y_pred)
+
+
+def builtin_loss(loss) -> Optional[Tuple[str, float]]:
+    """(name, huber delta) of a built-in loss function or object, None for anything else (a user callable)."""
+    if loss is binary_crossentropy or isinstance(loss, BinaryCrossentropy):
+        return ("binary_crossentropy", 0.0)
+    if loss is mean_squared_error or isinstance(loss, MeanSquaredError):
+        return ("mean_squared_error", 0.0)
+    if loss is mean_absolute_error or isinstance(loss, MeanAbsoluteError):
+        return ("mean_absolute_error", 0.0)
+    if isinstance(loss, Huber):
+        return ("huber", loss.delta)
+    return None
+
+
+def host_loss(loss: Tuple[str, float], pred: np.ndarray, y: np.ndarray) -> np.ndarray:
+    """Per-sample float64 loss of the built-in `loss` (builtin_loss) on one-column predictions; binary_crossentropy on probabilities
+    clipped to [1e-7, 1 - 1e-7], as Keras computes it from probabilities."""
+    name, delta = loss
+    p, y = np.asarray(pred, np.float64).reshape(-1), np.asarray(y, np.float64).reshape(-1)
+    if name == "binary_crossentropy":
+        p = np.clip(p, 1e-7, 1.0 - 1e-7)
+        return -(y * np.log(p) + (1.0 - y) * np.log1p(-p))
+    e = p - y
+    if name == "mean_squared_error":
+        return e * e
+    if name == "mean_absolute_error":
+        return np.abs(e)
+    q = np.minimum(np.abs(e), delta)
+    return 0.5 * q * q + delta * (np.abs(e) - q)
+
+
+_LOSS_IDS = {"mse": mean_squared_error, "MSE": mean_squared_error, "mean_squared_error": mean_squared_error, "mae": mean_absolute_error,
+             "MAE": mean_absolute_error, "mean_absolute_error": mean_absolute_error, "binary_crossentropy": binary_crossentropy}
+
+
+def get_loss(loss):
+    """keras.losses.get for the losses here: a string identifier resolves to its function (ValueError for an unknown one); a loss
+    object or function passes through unchanged."""
+    if isinstance(loss, str):
+        if loss not in _LOSS_IDS:
+            raise ValueError(f"Unknown loss function: {loss!r} (supported identifiers: {', '.join(_LOSS_IDS)})")
+        return _LOSS_IDS[loss]
+    if isinstance(loss, (list, tuple, dict)):
+        raise NotImplementedError("per-output losses: the models here have one output and take one loss")
+    return loss
+
+
+def get_optimizer(optimizer):
+    """keras.optimizers.get for the optimizers here: "adam", "sgd", "adagrad", "ftrl" in any case resolve to the class with Keras'
+    default arguments (ValueError for another name); an optimizer object passes through unchanged."""
+    if isinstance(optimizer, str):
+        cls = {"adam": Adam, "sgd": SGD, "adagrad": Adagrad, "ftrl": Ftrl}.get(optimizer.lower())
+        if cls is None:
+            raise ValueError(f"Unknown optimizer: {optimizer!r} (supported identifiers: adam, sgd, adagrad, ftrl)")
+        return cls()
+    return optimizer
+
+
 def _as_host(a) -> np.ndarray:
     return a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
 
@@ -651,17 +789,20 @@ class Model:
         `metrics`: AUC / Precision / Recall / BinaryAccuracy objects or the strings "AUC", "Precision", "Recall", "accuracy", "acc",
         "binary_accuracy" (handyrec_b200.metrics; counted on the GPU from each batch's forward output).  `weighted_metrics`: the
         same, counted with the sample weights of fit / train_on_batch / evaluate (a name an unweighted metric has becomes
-        `weighted_<name>`)."""
+        `weighted_<name>`).  `optimizer` may be "adam", "sgd", "adagrad" or "ftrl" (any case), `loss` "binary_crossentropy", "mse" /
+        "MSE" / "mean_squared_error" or "mae" / "MAE" / "mean_absolute_error" (get_optimizer / get_loss)."""
         from . import metrics as M
 
+        if kwargs.get("loss_weights") is not None:
+            raise NotImplementedError("loss_weights: the models here have one output and take one loss")
         if kwargs.get("sample_weight_mode") is not None:
             raise NotImplementedError("sample_weight_mode: only per-sample weights are supported (no temporal weights)")
         if weighted_metrics:
             self._require_one_probability("weighted_metrics")
         self._metric_list, weighted = M.from_compile(metrics, weighted_metrics)
         self._metric_set = M.MetricSet(self._metric_list, weighted) if self._metric_list else None
-        self.optimizer = optimizer if optimizer is not None else Adam()
-        self.loss = loss if loss is not None else binary_crossentropy
+        self.optimizer = get_optimizer(optimizer) if optimizer is not None else Adam()
+        self.loss = get_loss(loss) if loss is not None else binary_crossentropy
         self._fused = None
         if distribute is None and ShardedTables.active is not None:
             distribute = ShardedTables.active.comm
@@ -681,10 +822,11 @@ class Model:
         for l in self._all_layers():  # under Ftrl a dense step would move the rows a batch does not gather
             if hasattr(l, "SPARSE_UPDATE_MIN_ROWS"):
                 l._ftrl = isinstance(self.optimizer, Ftrl)
-        if self.fuse and self.loss is binary_crossentropy and isinstance(self.optimizer, (Adam, SGD, Adagrad, Ftrl)):
+        kind = builtin_loss(self.loss)
+        if self.fuse and kind is not None and isinstance(self.optimizer, (Adam, SGD, Adagrad, Ftrl)):
             from .lowering import lower  # a DeepFM-shaped graph runs on the fused engine (one lookup, tcgen05 towers)
 
-            self._fused = lower(self)
+            self._fused = lower(self, kind)
         if self._comm is not None and self._comm.N > 1 and self._fused is None:
             raise ValueError("distribute: only graphs the fused DeepFM engine covers train multi-GPU (lowering.py lists the conditions)")
         if clip is not None:
@@ -737,12 +879,12 @@ class Model:
         return self._with_metrics(loss, self._metric_values() if self._metric_set is not None else {}, return_dict)
 
     def _weights(self, y, sample_weight=None, class_weight=None) -> Optional[np.ndarray]:
-        """sample_weights(), refused for a loss other than binary_crossentropy and for an output other than one probability per
-        sample."""
+        """sample_weights(), refused for a loss other than the built-in ones and for an output other than one column per sample."""
         w = sample_weights(y, sample_weight, class_weight)
         if w is not None:
-            if self.loss is not binary_crossentropy:
-                raise NotImplementedError(f"sample_weight / class_weight are supported with binary_crossentropy only, not {self.loss!r}")
+            if builtin_loss(self.loss) is None:
+                raise NotImplementedError("sample_weight / class_weight are supported with the built-in losses only (binary_crossentropy, "
+                                          f"mean_squared_error, mean_absolute_error, Huber), not {self.loss!r}")
             self._require_one_probability("sample_weight / class_weight")
         return w
 
@@ -766,7 +908,7 @@ class Model:
             return self._train_on_batch_layers(x, y, weight)
 
     def _weighted_loss(self, yt: torch.Tensor, out, wt: Optional[torch.Tensor]):
-        """self.loss(yt, out), with the batch's sample weights handed to binary_crossentropy."""
+        """self.loss(yt, out), with the batch's sample weights handed to the built-in loss."""
         global _step_weight
         _step_weight = wt
         try:
@@ -933,12 +1075,10 @@ class Model:
         fused_val = (self._fused is not None and self._fused.engine is not None and isinstance(data, tuple) and len(data) in (2, 3)
                      and isinstance(data[0], dict))
         if fused_val:
-            # the fused engine's forward (the only reader a row-sharded table has); Keras' BCE on clipped probabilities
+            # the fused engine's forward (the only reader a row-sharded table has); the compiled loss of its output on the host
             xv, yv = data[:2]
             w = self._weights(yv, data[2]) if len(data) == 3 else None
-            p = np.clip(self._fused.predict(xv, batch_size, y=yv, metrics=ms, weight=w).reshape(-1).astype(np.float64), 1e-7, 1.0 - 1e-7)
-            yt = np.asarray(yv, dtype=np.float64).reshape(-1)
-            l = -(yt * np.log(p) + (1.0 - yt) * np.log1p(-p))
+            l = host_loss(self._fused.spec.loss, self._fused.predict(xv, batch_size, y=yv, metrics=ms, weight=w), yv)
             loss = float((l if w is None else w.astype(np.float64) * l).mean())
         else:
             vl, vc = 0.0, 0

@@ -17,7 +17,8 @@ from ._lib import ACT, POOL, FieldDesc, OptParams, TableDesc, call
 __all__ = [
     "init_uniform", "embedding_fwd", "embedding_bwd_dense", "seq_pool_fwd", "seq_pool_bwd", "LookupPlan",
     "fm_fwd", "fm_bwd", "dense_fwd", "dense_bwd_x", "dense_bwd_w", "act_bwd", "dice_fwd", "dice_bwd",
-    "lau_fwd", "lau_pack_params", "sigmoid_bce", "adam_step", "sgd_step", "adam_step_multi", "sgd_step_multi",
+    "lau_fwd", "lau_pack_params", "sigmoid_bce", "regression_loss", "regression_loss_workspace", "adam_step", "sgd_step",
+    "adam_step_multi", "sgd_step_multi",
     "adagrad_step", "adagrad_step_multi", "ftrl_step", "ftrl_step_multi", "metric_scratch_bytes", "metric_weighted_scratch_bytes",
     "metric_update",
     "clip_workspace", "clip_prepare_multi", "clip_scales", "clip_apply_multi",
@@ -494,6 +495,33 @@ def sigmoid_bce(dnn_logit: torch.Tensor, fm_logit: Optional[torch.Tensor], label
             raise ValueError(f"sigmoid_bce: {weight.numel()} weights for {B} samples")
         call("hrb_sigmoid_bce_weighted", _p(dnn_logit), _p(fm_logit), _p(label), _p(weight), B, grad_scale, _p(prob), _p(dlogit),
              _p(loss_sum), _stream())
+
+
+REG_LOSS = {"mean_squared_error": 0, "mean_absolute_error": 1, "huber": 2}  # hrb_regression_loss's `loss`
+
+
+def regression_loss_workspace(n: int, device) -> torch.Tensor:
+    """A zeroed workspace for hrb_regression_loss over n elements (it stays zeroed between calls)."""
+    nb = ctypes.c_size_t(0)
+    call("hrb_regression_loss_workspace", n, ctypes.byref(nb))
+    return torch.zeros(nb.value, device=device, dtype=torch.uint8)
+
+
+def regression_loss(loss: str, delta: float, a: torch.Tensor, b: Optional[torch.Tensor], label: Optional[torch.Tensor], batch: int,
+                    cols: int, grad_scale: float, pred: Optional[torch.Tensor] = None, dpred: Optional[torch.Tensor] = None,
+                    loss_sum: Optional[torch.Tensor] = None, weight: Optional[torch.Tensor] = None,
+                    workspace: Optional[torch.Tensor] = None):
+    """Keras MSE / MAE / Huber of pred = a (+ b) over the first batch * cols elements: loss_sum = sum(w * l) (l the mean over cols),
+    dpred = dl/dpred * w * grad_scale / cols.  `weight`: one fp32 per sample, or None."""
+    ws = (_p(workspace), workspace.numel()) if workspace is not None else (None, 0)
+    if weight is None:
+        call("hrb_regression_loss", REG_LOSS[loss], delta, _p(a), _p(b), _p(label), batch, cols, grad_scale, _p(pred), _p(dpred), _p(loss_sum),
+             *ws, _stream())
+    else:
+        if _chk(weight, torch.float32, "weight").numel() != batch:
+            raise ValueError(f"{loss}: {weight.numel()} sample weights for {batch} samples")
+        call("hrb_regression_loss_weighted", REG_LOSS[loss], delta, _p(a), _p(b), _p(label), _p(weight), batch, cols, grad_scale, _p(pred),
+             _p(dpred), _p(loss_sum), *ws, _stream())
 
 
 def adam_step(param, grad, m, v, lr, beta1=0.9, beta2=0.999, eps=1e-7, step=1, l2_scale=0.0):

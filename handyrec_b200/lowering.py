@@ -1,13 +1,15 @@
 """Lowering of a `keras_lite.Model` graph onto the fused engines.
 
 `handyrec.models.DeepFM(...)` (models/ranking/context_aware/DeepFM.py:59-94) wires
-    Input -> CustomEmbedding [-> SequencePoolingLayer] -> concat -> {DNN, FM} -> add -> sigmoid
+    Input -> CustomEmbedding [-> SequencePoolingLayer] -> concat -> {DNN, FM} -> add -> sigmoid   (task="binary")
+    ...                                                                              -> add              (task="regression")
 out of generic layers.  Executed layer by layer that is two lookups per table, a materialised (B,L,D) tensor + mask, a dense
 vocab x D gradient per table and one FFMA GEMM per Dense.  `lower(model)` recognises that graph, checks what the fused
 `DeepFMEngine` covers (FM and DNN groups over the same features, one embedding dim, mean / sum pooling, element-wise DNN
 activations, no BatchNorm / Dropout) and returns a `FusedDeepFM` binding through which `Model.fit / train_on_batch / predict`
 run: ONE plan lookup for both groups, the tcgen05 dense layers, the two-level-partition embedding backward and the flat
-optimiser step.  Graphs the engine does not cover return None and keep the layer-by-layer path -- same results, slower.
+optimiser step.  The sigmoid head lowers with binary_crossentropy, the linear head with mean_squared_error, mean_absolute_error
+or Huber.  Graphs and pairings the engine does not cover return None and keep the layer-by-layer path -- same results, slower.
 
 Host side of `fit`: the dict-of-arrays batches Keras takes are packed into one int32 id matrix + one fp32 dense matrix in pinned
 memory by `hrb_host_pack_*` (a thread pool inside the library) on a background thread, one batch ahead of the GPU.
@@ -84,13 +86,16 @@ def _field_of(t: KTensor) -> Optional[_Field]:
 
 
 class DeepFMSpec:
-    """What `lower` read off the graph."""
+    """What `lower` read off the graph.  `head`: "sigmoid" (task="binary") or "linear" (task="regression", the output is the add);
+    `loss`: the compiled loss as (name, huber delta), set by `lower`."""
 
     def __init__(self):
         self.fields: List[_Field] = []
         self.dense_inputs: List[KTensor] = []
         self.dnn = None
         self.fm = None
+        self.head = "sigmoid"
+        self.loss: Tuple[str, float] = ("binary_crossentropy", 0.0)
 
 
 def match_deepfm(model) -> Optional[DeepFMSpec]:
@@ -99,9 +104,12 @@ def match_deepfm(model) -> Optional[DeepFMSpec]:
     from .layers.utils import Cast, Flatten
 
     out = model.outputs
-    if not isinstance(out, KTensor) or not isinstance(_producer(out), Activation) or _producer(out).activation != "sigmoid":
+    if not isinstance(out, KTensor):
         return None
-    summed = out.node.inputs
+    head = "linear" if isinstance(_producer(out), Lambda) else "sigmoid"
+    if head == "sigmoid" and (not isinstance(_producer(out), Activation) or _producer(out).activation != "sigmoid"):
+        return None
+    summed = out if head == "linear" else out.node.inputs
     add = _producer(summed)
     if not isinstance(add, Lambda) or add.name != "add" and not add.name.startswith("add"):
         return None
@@ -158,7 +166,7 @@ def match_deepfm(model) -> Optional[DeepFMSpec]:
     if any(not f.emb.trainable for f in dnn_fields):
         return None
     spec = DeepFMSpec()
-    spec.fields, spec.dense_inputs, spec.dnn, spec.fm = dnn_fields, dense_inputs, dnn, fm
+    spec.fields, spec.dense_inputs, spec.dnn, spec.fm, spec.head = dnn_fields, dense_inputs, dnn, fm, head
     return spec
 
 
@@ -272,6 +280,8 @@ class FusedDeepFM:
         small = getattr(self.model, "dense_table_max_rows", 131072)
         common = dict(dnn_hidden_units=tuple(dnn.hidden_units), dnn_activation=dnn.activation or "linear", batch_size=batch_size, optimizer=opt,
                       lr=lr, l2_embd=self.spec.fields[0].emb.l2, l2_dnn=float(dnn.l2_reg or 0.0), seed=dnn.seed)
+        if self.spec.head == "linear":
+            common.update(task="regression", loss=self.spec.loss[0], huber_delta=self.spec.loss[1])
         if opt in ("adagrad", "ftrl"):  # the engine fills its accumulators when it is built
             common["initial_accumulator_value"] = optimizer.initial_accumulator_value
         if opt == "ftrl":
@@ -440,7 +450,7 @@ class FusedDeepFM:
         return self.engine.train_on_batch(ids, dense if self.n_dense else None, label, w)
 
     def predict(self, x, batch_size: Optional[int], y=None, metrics=None, weight: Optional[np.ndarray] = None) -> np.ndarray:
-        """Probabilities of `x`; with `metrics` (a MetricSet) and labels `y`, every batch is also counted on the device (the
+        """Probabilities (a linear head: predictions) of `x`; with `metrics` (a MetricSet) and labels `y`, every batch is also counted on the device (the
         validation pass of fit / evaluate: no second forward), with the rows' sample weights `weight` when given."""
         id_cols, dense_cols, n = self._columns(x)
         bs = min(batch_size or n, self.engine.B)
@@ -486,6 +496,11 @@ def _lr_step(optimizer):
     return step
 
 
-def lower(model) -> Optional[FusedDeepFM]:
+def lower(model, loss: Tuple[str, float] = ("binary_crossentropy", 0.0)) -> Optional[FusedDeepFM]:
+    """The fused binding of a DeepFM-shaped `model` compiled with `loss` ((name, huber delta) of a built-in loss), or None: a sigmoid
+    head trains binary_crossentropy only and a linear head the regression losses only; any other pairing keeps the layer path."""
     spec = match_deepfm(model)
-    return FusedDeepFM(model, spec) if spec is not None else None
+    if spec is None or (spec.head == "sigmoid") != (loss[0] == "binary_crossentropy"):
+        return None
+    spec.loss = loss
+    return FusedDeepFM(model, spec)

@@ -347,6 +347,25 @@ int hrb_sigmoid_bce_weighted(const float* dnn_logit, const float* fm_logit, cons
 int hrb_clipped_bce_weighted(const float* prob, const float* label, const float* weight, int64_t n, float eps, float grad_scale,
                              float* dprob, float* loss_sum, void* stream);
 
+/* Keras regression losses (keras/losses.py mean_squared_error, mean_absolute_error, huber; the head of DeepFM(task="regression"),
+ * DeepFM.py:86-88 without the sigmoid):
+ *   pred = pred_a (+ pred_b when not null); e = pred - label, elementwise over (batch, cols);
+ *   loss 0 (MSE): e^2, de = 2e;  1 (MAE): |e|, de = sign(e) (0 at e = 0);
+ *   2 (Huber):  0.5 q^2 + delta (|e| - q), q = min(|e|, delta), de = e for |e| <= delta (the tie takes the quadratic branch),
+ *               delta sign(e) otherwise;
+ *   per-sample loss l = mean over cols (Keras' mean over the last axis); loss_sum = sum_b w_b l_b (w = 1 unweighted), written (not
+ *   accumulated) and reduced in float64 in a fixed order, so it is the same bits from run to run;
+ *   dpred = de * w * grad_scale / cols (grad_scale = 1 / (batch * ranks): Keras' sum(w * l) / B, B the batch size, not sum(w)).
+ * pred, dpred, loss_sum may be null; label may be null when dpred and loss_sum are (a forward alone).  The workspace (size from
+ * hrb_regression_loss_workspace) is needed with loss_sum; it must be zeroed once before its first use and is left zeroed.
+ * The weighted entry takes one fp32 weight per sample (batch of them); w = 1 gives the unweighted bits. */
+int hrb_regression_loss_workspace(int64_t n, size_t* bytes);
+int hrb_regression_loss(int32_t loss, float delta, const float* pred_a, const float* pred_b, const float* label, int64_t batch, int32_t cols,
+                        float grad_scale, float* pred, float* dpred, float* loss_sum, void* workspace, size_t workspace_bytes, void* stream);
+int hrb_regression_loss_weighted(int32_t loss, float delta, const float* pred_a, const float* pred_b, const float* label, const float* weight,
+                                 int64_t batch, int32_t cols, float grad_scale, float* pred, float* dpred, float* loss_sum, void* workspace,
+                                 size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * (f1) retrieval loss: SampledSoftmaxLayer.call = tf.nn.sampled_softmax_loss (layers/tools.py:56-75), TF defaults:
  *   num_true = 1, remove_accidental_hits, subtract log Q, log-uniform candidates drawn unique.
