@@ -51,6 +51,7 @@ __all__ = [
     "bce_from_logits",
     "l2_normalize",
     "hash_uniform_table",
+    "hash_uniform_rows",
     "hash_u32",
     "embedding_grad_dense",
     "sharded_lookup_emulated",
@@ -493,7 +494,13 @@ def hash_uniform_table(V: int, D: int, seed: int, lo: float = -0.05, hi: float =
     Bit-identical to ``hrb_init_uniform`` (mul and add are separately rounded on
     both sides).  ``row_start/row_step`` give the rows of a ``row % N`` shard.
     """
-    rows = (np.arange(V, dtype=np.uint64) * np.uint64(row_step) + np.uint64(row_start))
+    return hash_uniform_rows(np.arange(V, dtype=np.uint64) * np.uint64(row_step) + np.uint64(row_start), D, seed, lo, hi)
+
+
+def hash_uniform_rows(rows, D: int, seed: int, lo: float = -0.05, hi: float = 0.05) -> np.ndarray:
+    """Rows ``rows`` (any order, repeats allowed) of ``hash_uniform_table(V, D, seed, lo, hi)`` without forming the table: the
+    initial values of the rows a step touches in a table too large to copy to the host."""
+    rows = np.asarray(rows).astype(np.uint64).reshape(-1)
     idx = rows[:, None] * np.uint64(D) + np.arange(D, dtype=np.uint64)[None, :]
     lo32 = (idx & np.uint64(0xFFFFFFFF)).astype(np.uint32)
     hi32 = (idx >> np.uint64(32)).astype(np.uint32)
