@@ -119,13 +119,8 @@ def load_weights(model, directory: str) -> None:
             raise KeyError(f"{directory}: no weight {key!r} (was the model built by the same constructor call?)")
         _load_tensor(p.data, directory, have[key]["files"])
     fused = getattr(model, "_fused", None)
-    if fused is not None and fused.engine is not None:  # dense / FM weights also live in the engine: push the loaded values there
-        eng = fused.engine
-        for i, d in enumerate(fused._dense_layers()):
-            eng.set_dense_weights(i, d.kernel.data.cpu(), d.bias.data.cpu())
-        eng.fm_w.copy_(fused.spec.fm.linear.data.reshape(-1))
-        eng.fm_w0.copy_(fused.spec.fm.w_0.data.reshape(-1))
-        fused._dirty = False
+    if fused is not None:  # dense / FM weights also live in the engine: push the loaded values there
+        fused.push_to_engine()
 
 
 def export_pre_embd(model) -> Dict[str, np.ndarray]:

@@ -5,7 +5,7 @@
 `tensorflow` / `tensorflow.keras` and call a dozen TF names (`Model`, `Activation`, `tf.matmul`, `tf.nn.l2_normalize`,
 `tf.nn.embedding_lookup`, `tf.squeeze`, `tf.int32`).  `install(reference_root)` registers
 
-    tensorflow, tensorflow.keras[.layers|.models|.initializers|.regularizers|.losses|.optimizers[.schedules]|.metrics|.experimental]
+    tensorflow, tensorflow.keras[.layers|.models|.initializers|.regularizers|.losses|.optimizers[.schedules]|.metrics|.experimental|.callbacks]
                                                                                                     -> thin modules over keras_lite
     handyrec, handyrec.features, handyrec.layers, handyrec.layers.utils, handyrec.features.*        -> this package's drop-in face
     handyrec.models (+ .ranking, .retrieval, ...)                                                   -> the reference's files, loaded
@@ -35,6 +35,17 @@ def _unsupported(name):
     class _Stub(KL.Layer):
         def __init__(self, *a, **k):
             raise NotImplementedError(f"{name} is outside the hot path handyrec_b200 implements (DESIGN.md 7)")
+
+    _Stub.__name__ = name
+    return _Stub
+
+
+def _unsupported_callback(name):
+    from ..callbacks import Callback
+
+    class _Stub(Callback):
+        def __init__(self, *a, **k):
+            raise NotImplementedError(f"{name} is not implemented by handyrec_b200 (DESIGN.md 7)")
 
     _Stub.__name__ = name
     return _Stub
@@ -110,12 +121,19 @@ def _tf_module() -> types.ModuleType:
     mets = types.ModuleType("tensorflow.keras.metrics")
     mets.AUC, mets.BinaryAccuracy, mets.Precision, mets.Recall = KL.AUC, KL.BinaryAccuracy, KL.Precision, KL.Recall
     keras.layers, keras.models, keras.initializers, keras.regularizers, keras.losses, keras.optimizers = layers, models, inits, regs, losses, opts
-    keras.metrics, keras.experimental = mets, experimental
+    from .. import callbacks as C
+
+    cbs = types.ModuleType("tensorflow.keras.callbacks")
+    for n in C.__all__:
+        setattr(cbs, n, getattr(C, n))
+    for n in ("TensorBoard", "ProgbarLogger", "BackupAndRestore", "RemoteMonitor"):
+        setattr(cbs, n, _unsupported_callback(n))
+    keras.metrics, keras.experimental, keras.callbacks = mets, experimental, cbs
     tf.keras = keras
     tf._submodules = {"tensorflow.nn": nn, "tensorflow.keras": keras, "tensorflow.keras.layers": layers, "tensorflow.keras.models": models,
                       "tensorflow.keras.initializers": inits, "tensorflow.keras.regularizers": regs, "tensorflow.keras.losses": losses,
                       "tensorflow.keras.optimizers": opts, "tensorflow.keras.optimizers.schedules": scheds, "tensorflow.keras.metrics": mets,
-                      "tensorflow.keras.experimental": experimental}
+                      "tensorflow.keras.experimental": experimental, "tensorflow.keras.callbacks": cbs}
     return tf
 
 

@@ -712,11 +712,16 @@ class DeepFMEngine:
         torch.cuda.current_stream().synchronize()
         return float(self.loss_host[0]) / B
 
-    def fit_batches(self, batches) -> List[float]:
+    def fit_batches(self, batches, on_step=None) -> List[float]:
         """Keras-`fit`-like loop over host batches `(ids, dense, label)` or `(ids, dense, label, weight)` (pinned tensors; weight
         None or Keras' sample weights) with input prefetch: the H2D copies of batch t+1 run on a copy stream while batch t
         computes, and every step's loss is copied back asynchronously; the host waits once, at the end.  Returns the per-step
-        mean losses."""
+        mean losses.
+
+        `on_step(t, loss)` (Keras callbacks with batch hooks): called with loss None before step t is issued, and with step t's mean
+        loss once it is on the host -- after step t has been issued and batch t+1 fetched and its copy started, so the packing
+        thread and the prefetch run on while the hook does.  A true return stops the loop before step t+1 is issued.  This costs
+        one host sync per step; without `on_step` the loop issues exactly what it issued before."""
         main = torch.cuda.current_stream()
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream()
@@ -762,8 +767,11 @@ class DeepFMEngine:
         slot = 0
         if nxt is not None:
             nB = upload(slot, nxt)
+        step_done = torch.cuda.Event() if on_step is not None else None
         while nxt is not None:
             cur_slot, B = slot, nB
+            if on_step is not None:
+                on_step(len(losses_host), None)
             main.wait_event(self._stage_ready[cur_slot])
             ids_d, dense_d, label_d = self._stage[cur_slot]
             self.train_step_on_device(ids_d[:B], dense_d[:B] if self.n_dense else None, label_d[:B],
@@ -781,10 +789,16 @@ class DeepFMEngine:
             sizes.append(B)
             # the next batch is fetched AFTER this step has been issued: the GPU never waits for the producer of batch t+1 before it
             # may start batch t (the copy still overlaps step t: it only needs the other stage slot, free since step t-1)
+            if on_step is not None:
+                step_done.record(main)
             nxt = next(it, None)
             if nxt is not None:
                 slot ^= 1
                 nB = upload(slot, nxt)
+            if on_step is not None:
+                step_done.synchronize()
+                if on_step(len(losses_host) - 1, float(lh[0]) / B):
+                    break
         main.synchronize()
         return [float(l[0]) / b for l, b in zip(losses_host, sizes)]
 

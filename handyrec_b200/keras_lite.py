@@ -757,15 +757,32 @@ class Model:
         if self._fused is not None:
             self._fused.sync_to_layers()
 
-    def predict(self, x, batch_size=None):
+    def predict(self, x, batch_size=None, callbacks=None):
+        """keras.Model.predict.  callbacks: handyrec_b200.callbacks objects; they get the on_predict_* hooks (batch-end logs:
+        {"outputs": the batch's predictions})."""
+        from .callbacks import CallbackList
+
+        cbs = CallbackList(callbacks, model=self, verbose=0, epochs=1, steps=None)
         if (self._fused is not None and self._fused.engine is None and isinstance(x, dict) and self._comm is not None and self._comm.N > 1
                 and self.optimizer is not None):
             # a multi-GPU model before its first fit: only the engine can read row-sharded tables, so it is built here (collective:
             # every rank calls predict, as with fit)
             n = len(np.asarray(next(iter(x.values()))))
             self._fused.build(min(batch_size or n, n), self.optimizer)
+        cbs.on_predict_begin()
         if self._fused is not None and self._fused.engine is not None and isinstance(x, dict):
-            return self._fused.predict(x, batch_size)
+            on_batch = None
+            if cbs.should_call_predict_batch_hooks:
+
+                def on_batch(i: int, start: int, pred: Optional[np.ndarray]) -> None:
+                    if pred is None:
+                        cbs.on_predict_batch_begin(i)
+                    else:
+                        cbs.on_predict_batch_end(i, {"outputs": pred})
+
+            out = self._fused.predict(x, batch_size, on_batch=on_batch)
+            cbs.on_predict_end()
+            return out
         self.sync()
         n = len(next(iter(x.values()))) if isinstance(x, dict) else len(x[0] if isinstance(x, (list, tuple)) else x)
         bs = batch_size or n
@@ -773,10 +790,14 @@ class Model:
         from .kernels import deferred_id_checks
 
         with torch.no_grad():
-            for s in range(0, n, bs):
+            for i, s in enumerate(range(0, n, bs)):
+                cbs.on_predict_batch_begin(i)
                 xb = {k: v[s : s + bs] for k, v in x.items()} if isinstance(x, dict) else [v[s : s + bs] for v in x]
                 with deferred_id_checks():
                     outs.append(self(xb, training=False).detach().cpu())
+                if cbs.should_call_predict_batch_hooks:
+                    cbs.on_predict_batch_end(i, {"outputs": outs[-1].numpy()})
+        cbs.on_predict_end()
         return torch.cat(outs).numpy()
 
     _comm = None
@@ -992,6 +1013,51 @@ class Model:
         clip.apply(gs + [p.grad for p in tabs], vs + [tv[id(p)] for p in tabs])
         return [(p, 0.0) for p, _ in params]
 
+    stop_training = False  # set by a callback to end fit after the current batch or epoch (reset at on_train_begin)
+
+    def get_weights(self) -> List[np.ndarray]:
+        """keras.Model.get_weights: host copies of every weight, in the order of the checkpoint keys (checkpoint._named_weights).  A
+        row-sharded table contributes this rank's rows only, as save_weights writes them."""
+        from .checkpoint import _named_weights
+
+        return [p.detach().to("cpu", copy=True).numpy() for _, _, p in _named_weights(self)]
+
+    def set_weights(self, weights) -> None:
+        """keras.Model.set_weights, the inverse of get_weights (shape-checked).  On a fused model the values go into the live
+        engine: tables through the storage the engine shares with the layers, dense and FM weights into its flat buffer.  The
+        engine is not rebuilt and its optimizer slots are kept."""
+        from .checkpoint import _named_weights
+
+        named = list(_named_weights(self))
+        if len(weights) != len(named):
+            raise ValueError(f"set_weights: the model has {len(named)} weights, got {len(weights)} arrays")
+        vals = []
+        for (key, _, p), w in zip(named, weights):
+            a = np.asarray(w, dtype=np.float32)
+            if tuple(a.shape) != tuple(p.shape):
+                raise ValueError(f"set_weights: {key} has shape {tuple(p.shape)}, got an array of shape {a.shape}")
+            vals.append(a)
+        for (_, _, p), a in zip(named, vals):
+            p.data.copy_(torch.from_numpy(a))
+        if self._fused is not None:
+            self._fused.push_to_engine()
+
+    def _set_learning_rate(self, lr) -> None:
+        """The float rate the learning-rate callbacks set, rounded to float32 as Keras' rate variable holds it.  It takes effect at
+        the next step on either path; a fused engine keeps running (no rebuild: its optimizer slots, `optimizer.iterations` and
+        step count carry on).  Assigning `optimizer.lr` directly still rebuilds the engine at the next fit."""
+        from .schedules import LearningRateSchedule
+
+        opt = self.optimizer
+        if isinstance(opt.lr, LearningRateSchedule):
+            raise ValueError(f"the optimizer's learning rate is the schedule {type(opt.lr).__name__}; it has no float rate to set")
+        fused = self._fused
+        same = fused is not None and fused.engine is not None and fused._opt_key == fused.engine_key(opt)
+        opt.lr = float(np.float32(lr))
+        opt.lr_t = decayed_lr(opt)
+        if same:
+            fused._opt_key = fused.engine_key(opt)
+
     def save_weights(self, filepath, **kwargs):
         """keras.Model.save_weights: a directory of `.npy` files (tables row-sharded), see handyrec_b200.checkpoint."""
         from .checkpoint import save_weights
@@ -1019,11 +1085,26 @@ class Model:
                 fn()
 
     def fit(self, x=None, y=None, batch_size=32, epochs=1, validation_data=None, verbose=0, sample_weight=None, class_weight=None,
-            **kwargs):
+            callbacks=None, **kwargs):
         """keras.Model.fit over a dict of arrays (+ y), an `(x, y)` / `(x, y, sample_weight)` tuple, or an iterable of such batches.
         sample_weight / class_weight: Keras' per-sample weights of the training data (folded into one float32 weight per sample
-        once per fit); validation_data may be `(x, y, sample_weight)`."""
-        history = {"loss": []}
+        once per fit); validation_data may be `(x, y, sample_weight)`.  callbacks: handyrec_b200.callbacks objects, driven in
+        Keras' order (that module's docstring).  Returns the History callback.
+
+        On several GPUs (compile(distribute=...)), the callbacks see `loss` and `val_loss` as the sample-count-weighted means over
+        the ranks (one all-reduce per epoch), so that every rank takes the same decisions; `history` keeps this rank's values.
+        Batch-hook callbacks (TerminateOnNaN, an integer ModelCheckpoint save_freq, ...) are refused there with a ValueError."""
+        from .callbacks import CallbackList, History
+
+        multi = self._comm is not None and self._comm.N > 1
+        cbs = CallbackList(callbacks, model=self, verbose=verbose, epochs=epochs, steps=None)
+        if multi and cbs.should_call_train_batch_hooks:
+            raise ValueError(f"callbacks with batch hooks ({', '.join(cbs.train_batch_hook_names())}) are not supported on a multi-GPU "
+                             "compile: use epoch-level callbacks")
+        history = History()
+        history.set_model(self)
+        history.set_params(dict(verbose=verbose, epochs=epochs, steps=None))
+        history.history["loss"] = []
         if isinstance(x, tuple) and len(x) in (2, 3) and isinstance(x[0], dict) and y is None:
             x, y, *rest = x
             sample_weight = rest[0] if rest else sample_weight
@@ -1031,68 +1112,152 @@ class Model:
         if not isinstance(x, dict) and sample_weight is not None:
             raise ValueError("sample_weight with an iterable of batches: yield (x, y, sample_weight) batches instead")
         batches = _batches(x, y, batch_size, weight, class_weight=class_weight, model=self)
-        for _ in range(epochs):
+        batch_hooks = cbs.should_call_train_batch_hooks
+        self.stop_training = False
+        cbs.on_train_begin()
+        history.on_train_begin()
+        logs = None
+        for epoch in range(epochs):
             self.reset_metrics()  # Keras resets the metrics at the start of every epoch
+            cbs.on_epoch_begin(epoch)
+            tot, cnt = 0.0, 0  # Keras reports the sample-weighted running mean of the batch losses
+
+            def batch_logs(reg: float = 0.0) -> "OrderedDict[str, Any]":
+                out = OrderedDict(loss=tot / max(cnt, 1) + reg)
+                if self._metric_set is not None:
+                    out.update(self._metric_values())
+                return out
+
             if self._fused is not None and isinstance(x, dict):
                 # dict-of-arrays input: batches are packed into pinned memory one step ahead of the GPU and the whole epoch
                 # runs on the fused engine with asynchronous loss read-back (lowering.FusedDeepFM.fit_epoch)
                 n = len(np.asarray(next(iter(x.values()))))
                 self._fused.build(min(batch_size, n), self.optimizer)
-                losses = self._fused.fit_epoch(x, y, batch_size, weight)
-                sizes = [min(batch_size, n - s) for s in range(0, n, batch_size)]
-                history["loss"].append(float(np.average(losses, weights=sizes)) + self._fused.reg_loss())
+                on_step = None
+                if batch_hooks:  # every step's loss is read back before the next step is issued
+
+                    def on_step(t: int, loss: Optional[float]) -> bool:
+                        nonlocal tot, cnt
+                        if loss is None:
+                            cbs.on_train_batch_begin(t)
+                            return False
+                        nb = min(batch_size, n - t * batch_size)
+                        tot, cnt = tot + loss * nb, cnt + nb
+                        cbs.on_train_batch_end(t, batch_logs(self._fused.reg_loss()))
+                        return self.stop_training
+
+                losses = self._fused.fit_epoch(x, y, batch_size, weight, on_step=on_step)
+                sizes = [min(batch_size, n - s) for s in range(0, n, batch_size)][: len(losses)]
+                n_seen = sum(sizes)
+                ep_loss = float(np.average(losses, weights=sizes)) + self._fused.reg_loss()
                 self.last_losses = losses
             else:
-                tot, cnt = 0.0, 0
-                for xb, yb, wb in batches():  # Keras reports the sample-weighted running mean of the batch losses
+                for step, (xb, yb, wb) in enumerate(batches()):
+                    cbs.on_train_batch_begin(step)
                     nb = len(yb) if hasattr(yb, "__len__") else 1
                     tot += self._train_step(xb, yb, wb) * nb
                     cnt += nb
-                history["loss"].append(tot / max(cnt, 1))
+                    if batch_hooks:
+                        cbs.on_train_batch_end(step, batch_logs())
+                        if self.stop_training:
+                            break
+                n_seen = cnt
+                ep_loss = tot / max(cnt, 1)
+            logs = OrderedDict(loss=ep_loss)
             if self._metric_set is not None:
-                for k, v in self._metric_values().items():
-                    history.setdefault(k, []).append(v)
+                logs.update(self._metric_values())
             # fused training leaves the dense / FM weights in the engine; they are handed back to the layers lazily, the first time
             # anything reads the layers (`layers`, `get_layer`, `predict` on the layer path, `save_weights`, `sync()`)
+            n_val = 0
             if validation_data is not None:
-                vl, vres = self._evaluate_pass(validation_data, batch_size)
-                history.setdefault("val_loss", []).append(vl)
+                vl, vres, n_val = self._evaluate_pass(validation_data, batch_size, cbs)
+                logs["val_loss"] = vl
                 for k, v in vres.items():
-                    history.setdefault("val_" + k, []).append(v)
+                    logs["val_" + k] = v
+            cb_logs = logs
+            if multi and cbs.callbacks:
+                cb_logs = self._global_losses(logs, n_seen, n_val)
+            cbs.on_epoch_end(epoch, cb_logs)
+            for k, v in cb_logs.items():  # what the callbacks added (the rates' "lr"); loss and val_loss stay this rank's
+                logs.setdefault(k, v)
+            history.on_epoch_end(epoch, logs)
+            if self.stop_training:
+                break
+        cbs.on_train_end(logs)
+        return history
 
-        class H:
-            pass
+    def _global_losses(self, logs, n_train: int, n_val: int) -> "OrderedDict[str, Any]":
+        """`logs` with loss and val_loss replaced by their sample-count-weighted means over the ranks (one all-reduce of four numbers;
+        collective, as fit is).  The metrics in `logs` are global already."""
+        t = torch.tensor([logs["loss"] * n_train, n_train, logs.get("val_loss", 0.0) * n_val, n_val], dtype=torch.float64, device=device())
+        self._comm.all_reduce_sum(t)
+        s = t.tolist()
+        out = OrderedDict(logs)
+        out["loss"] = s[0] / max(s[1], 1.0)
+        if "val_loss" in logs:
+            out["val_loss"] = s[2] / max(s[3], 1.0)
+        return out
 
-        h = H()
-        h.history = history
-        return h
+    def _evaluate_pass(self, data, batch_size: int, callbacks=None):
+        """The validation pass of `fit` and the body of `evaluate`: (loss, metric results, samples), the metrics reset first.  `data`:
+        `(x, y)`, `(x, y, sample_weight)` or an iterable of such batches.  `callbacks` (a CallbackList) get the on_test_* hooks; the
+        batch logs hold the running loss (the mean over the rows so far on the fused path, over the batches so far on the layer
+        path, as each path computes its final loss) and the running metric results."""
+        from .callbacks import CallbackList
 
-    def _evaluate_pass(self, data, batch_size: int):
-        """The validation pass of `fit` and the body of `evaluate`: (loss, metric results), the metrics reset first.  `data`: `(x, y)`,
-        `(x, y, sample_weight)` or an iterable of such batches."""
+        cbs = callbacks if callbacks is not None else CallbackList()
         ms = self._metric_set
         self.reset_metrics()
+        cbs.on_test_begin()
+
+        def batch_logs(loss: float) -> "OrderedDict[str, Any]":
+            out = OrderedDict(loss=loss)
+            if ms is not None:
+                out.update(self._metric_values())
+            return out
+
         fused_val = (self._fused is not None and self._fused.engine is not None and isinstance(data, tuple) and len(data) in (2, 3)
                      and isinstance(data[0], dict))
         if fused_val:
             # the fused engine's forward (the only reader a row-sharded table has); the compiled loss of its output on the host
             xv, yv = data[:2]
             w = self._weights(yv, data[2]) if len(data) == 3 else None
-            l = host_loss(self._fused.spec.loss, self._fused.predict(xv, batch_size, y=yv, metrics=ms, weight=w), yv)
+            yh = np.asarray(yv).reshape(-1)
+            on_batch = None
+            if cbs.should_call_test_batch_hooks:
+                seen = [0.0]
+
+                def on_batch(i: int, start: int, pred: Optional[np.ndarray]) -> None:
+                    if pred is None:
+                        cbs.on_test_batch_begin(i)
+                        return
+                    r = slice(start, start + len(pred))
+                    lb = host_loss(self._fused.spec.loss, pred, yh[r])
+                    seen[0] += float((lb if w is None else w[r].astype(np.float64) * lb).sum())
+                    cbs.on_test_batch_end(i, batch_logs(seen[0] / r.stop))
+
+            l = host_loss(self._fused.spec.loss, self._fused.predict(xv, batch_size, y=yv, metrics=ms, weight=w, on_batch=on_batch), yv)
             loss = float((l if w is None else w.astype(np.float64) * l).mean())
+            n = len(l)
         else:
-            vl, vc = 0.0, 0
+            vl, vc, n = 0.0, 0, 0
             with torch.no_grad():
                 for xb, yb, wb in _batches(data, None, batch_size, model=self)():
+                    cbs.on_test_batch_begin(vc)
                     out = self(xb, training=False)
                     yt = torch.as_tensor(np.asarray(yb), dtype=torch.float32).to(device())
                     wt = torch.from_numpy(wb).to(device()) if wb is not None else None
                     vl += float(self._weighted_loss(yt, out, wt))
                     if ms is not None:
                         ms.update(out, yt, wt)
+                    n += int(yt.shape[0])
                     vc += 1
+                    if cbs.should_call_test_batch_hooks:
+                        cbs.on_test_batch_end(vc - 1, batch_logs(vl / vc))
             loss = vl / max(vc, 1)
-        return loss, (self._metric_values() if ms is not None else OrderedDict())
+        res = self._metric_values() if ms is not None else OrderedDict()
+        cbs.on_test_end(OrderedDict([("loss", loss)] + list(res.items())))
+        return loss, res, n
 
     def evaluate(self, x=None, y=None, batch_size=None, verbose=0, sample_weight=None, steps=None, callbacks=None, return_dict=False,
                  **kwargs):
@@ -1100,7 +1265,9 @@ class Model:
         loss is what `fit(validation_data=(x, y), batch_size=batch_size)` records as val_loss on the same path.  Sample weights
         come with the data, as `validation_data` takes them: `evaluate((x, y, sample_weight))` or an iterable of
         `(x, y, sample_weight)` batches (the same val_loss as `validation_data=(x, y, sample_weight)`); the `sample_weight`
-        keyword is not supported (NotImplementedError)."""
+        keyword is not supported (NotImplementedError).  callbacks: handyrec_b200.callbacks objects; they get the on_test_* hooks."""
+        from .callbacks import CallbackList
+
         if sample_weight is not None:
             raise NotImplementedError("evaluate(sample_weight=...): pass the weights with the data, evaluate((x, y, sample_weight)) or "
                                       "an iterable of (x, y, sample_weight) batches")
@@ -1111,11 +1278,14 @@ class Model:
             # a multi-GPU model before its first fit: only the engine reads row-sharded tables (collective, as in predict)
             n = len(np.asarray(next(iter(data[0].values()))))
             self._fused.build(min(bs, n), self.optimizer)
-        loss, res = self._evaluate_pass(data, bs)
+        loss, res, _ = self._evaluate_pass(data, bs, CallbackList(callbacks, model=self, verbose=verbose, epochs=1, steps=steps))
         return self._with_metrics(loss, res, return_dict)
 
 
 from .metrics import AUC, BinaryAccuracy, Precision, Recall  # noqa: E402  (tf.keras.metrics look-alikes, re-exported)
+from .callbacks import (  # noqa: E402  (tf.keras.callbacks look-alikes, re-exported)
+    Callback, CallbackList, CSVLogger, EarlyStopping, History, LambdaCallback, LearningRateScheduler, ModelCheckpoint, ReduceLROnPlateau,
+    TerminateOnNaN)
 
 
 def _all_sublayers(l: Layer) -> List[Layer]:

@@ -245,11 +245,12 @@ class FusedDeepFM:
 
         return [l for l in self.spec.dnn.layers if isinstance(l, Dense)]
 
-    def build(self, batch_size: int, optimizer) -> None:
+    @staticmethod
+    def engine_key(optimizer) -> tuple:
+        """What an engine is built for: a fit whose optimizer gives another key rebuilds it (fresh optimizer slots).  A schedule is
+        keyed by the object, not a value: the engine takes the rate per step and is not rebuilt as it changes."""
         from .clip import clip_args
-        from .engine import DeepFMEngine
         from .keras_lite import Adagrad, Adam, Ftrl, SGD
-        from .schedules import LearningRateSchedule, decayed_lr
 
         key = None
         if isinstance(optimizer, Adam):
@@ -264,9 +265,14 @@ class FusedDeepFM:
                    optimizer.l2_shrinkage, optimizer.beta)
         else:
             raise ValueError("the fused DeepFM path takes keras_lite.Adam, keras_lite.SGD, keras_lite.Adagrad or keras_lite.Ftrl")
-        clip = clip_args(optimizer)
-        # a schedule is keyed by the object, not a value: the engine takes the rate per step and is not rebuilt as it changes
-        key = (key or (opt, lr), clip, optimizer.decay)
+        return (key or (opt, lr), clip_args(optimizer), optimizer.decay)
+
+    def build(self, batch_size: int, optimizer) -> None:
+        from .engine import DeepFMEngine
+        from .schedules import LearningRateSchedule, decayed_lr
+
+        key = self.engine_key(optimizer)
+        opt, lr, clip = key[0][0], optimizer.lr, key[1]
         # every step the engine issues sets its own rate (_lr_step); a schedule is evaluated there only, once per step
         lr = None if isinstance(lr, LearningRateSchedule) else decayed_lr(optimizer)
         if self.engine is not None and self.engine.B >= batch_size and self._opt_key == key:
@@ -360,6 +366,19 @@ class FusedDeepFM:
         self.spec.fm.w_0.data.copy_(eng.fm_w0.reshape(-1))
         self._dirty = False
 
+    def push_to_engine(self) -> None:
+        """The inverse of sync_to_layers, after load_weights / set_weights wrote the layers: the dense / FM weights go into the live
+        engine's flat buffer (and its transposed copies).  The engine is not rebuilt and its optimizer slots are kept; the tables
+        need nothing, the layers share their storage with the engine."""
+        eng = self.engine
+        if eng is None:
+            return
+        for i, d in enumerate(self._dense_layers()):
+            eng.set_dense_weights(i, d.kernel.data.cpu(), d.bias.data.cpu())
+        eng.fm_w.copy_(self.spec.fm.linear.data.reshape(-1))
+        eng.fm_w0.copy_(self.spec.fm.w_0.data.reshape(-1))
+        self._dirty = False
+
     # ---- host input packing ---------------------------------------------------------------------
     def _columns(self, x: Dict[str, np.ndarray]) -> Tuple[_ColumnSet, _ColumnSet, int]:
         for f in self.spec.fields:
@@ -406,11 +425,15 @@ class FusedDeepFM:
         q: "queue.Queue" = queue.Queue(maxsize=max(1, n_slots - 2))
         dev_index = torch.cuda.current_device()
 
+        stop = threading.Event()
+
         def producer():
             try:
                 torch.cuda.set_device(dev_index)
                 k = 1
                 for start in range(batch_size, n, batch_size):
+                    if stop.is_set():
+                        return
                     slot = slots[k % n_slots]
                     self._pack(slot, id_cols, dense_cols, label_cols, start, min(batch_size, n - start), weight_cols)
                     q.put(slot)
@@ -427,19 +450,45 @@ class FusedDeepFM:
         yield slots[0]
         th = threading.Thread(target=producer, daemon=True)
         th.start()
-        while True:
-            item = q.get()
-            if item is None:
-                break
-            if isinstance(item, BaseException):
-                raise item
-            yield item
-        th.join()
+        try:
+            while True:
+                item = q.get()
+                if item is None:
+                    break
+                if isinstance(item, BaseException):
+                    raise item
+                yield item
+        finally:
+            # a consumer that stops early (a callback ended training) closes the generator: the producer stops at its next batch,
+            # and whatever it still queues is drained so that it never blocks on the full queue
+            stop.set()
+            while th.is_alive():
+                try:
+                    q.get(timeout=0.01)
+                except queue.Empty:
+                    pass
+            th.join()
 
     # ---- Keras-facing calls -----------------------------------------------------------------------
-    def fit_epoch(self, x, y, batch_size: int, weight: Optional[np.ndarray] = None) -> List[float]:
+    def fit_epoch(self, x, y, batch_size: int, weight: Optional[np.ndarray] = None, on_step=None) -> List[float]:
+        """One epoch over `x` on the engine; `on_step`: DeepFMEngine.fit_batches' per-step hook (callbacks with batch hooks)."""
         self._dirty = True
-        return self.engine.fit_batches(self.host_batches(x, y, batch_size, weight=weight))
+        hook = None
+        if on_step is not None:
+
+            def hook(t: int, loss: Optional[float]) -> bool:
+                stop = on_step(t, loss)
+                if loss is None:
+                    # step t is issued next: a batch hook may have synced the layers (save_weights, get_weights, layers) or
+                    # pushed weights into the engine, and whatever it left in the layers is stale once the step runs
+                    self._dirty = True
+                return stop
+
+        batches = self.host_batches(x, y, batch_size, weight=weight)
+        try:
+            return self.engine.fit_batches(batches, on_step=hook)
+        finally:
+            batches.close()
 
     def train_on_batch(self, x, y, weight: Optional[np.ndarray] = None) -> float:
         id_cols, dense_cols, n = self._columns(x)
@@ -449,20 +498,25 @@ class FusedDeepFM:
         ids, dense, label, w = slot.views()
         return self.engine.train_on_batch(ids, dense if self.n_dense else None, label, w)
 
-    def predict(self, x, batch_size: Optional[int], y=None, metrics=None, weight: Optional[np.ndarray] = None) -> np.ndarray:
+    def predict(self, x, batch_size: Optional[int], y=None, metrics=None, weight: Optional[np.ndarray] = None, on_batch=None) -> np.ndarray:
         """Probabilities (a linear head: predictions) of `x`; with `metrics` (a MetricSet) and labels `y`, every batch is also counted on the device (the
-        validation pass of fit / evaluate: no second forward), with the rows' sample weights `weight` when given."""
+        validation pass of fit / evaluate: no second forward), with the rows' sample weights `weight` when given.  `on_batch(i,
+        start, pred)`: called with pred None before batch i runs and with its (rows, 1) predictions after (callbacks' batch hooks)."""
         id_cols, dense_cols, n = self._columns(x)
         bs = min(batch_size or n, self.engine.B)
         slot = self._get_slots(1)[0]
         label_cols = _ColumnSet([np.asarray(y).reshape(-1, 1)]) if metrics is not None else None
         weight_cols = _weight_columns(weight) if metrics is not None else None
         outs = []
-        for start in range(0, n, bs):
+        for i, start in enumerate(range(0, n, bs)):
+            if on_batch is not None:
+                on_batch(i, start, None)
             self._pack(slot, id_cols, dense_cols, label_cols, start, min(bs, n - start), weight_cols)
             ids, dense, label, w = slot.views()
             outs.append(self.engine.predict(ids, dense if self.n_dense else None, label, metrics, w).numpy().copy())
             slot.copied = None
+            if on_batch is not None:
+                on_batch(i, start, outs[-1])
         return np.concatenate(outs, 0)
 
     def reg_loss(self) -> float:
